@@ -16,6 +16,7 @@ weak scaling, 125k homes x 96 quarter-hour steps per GPU in feeders of 1000 resi
           bounded sample of the same workload, host cores of this box, rank 0 / N=1 only
 
 `--impl reference` times that CPU port as the reference arm.
+`--dump-outputs DIR` writes the results of the last timed step of `value` as .npy files (dump_outputs).
 """
 import argparse
 import json
@@ -40,6 +41,7 @@ WORKLOADS = {
     "tiny": ("refshape", 1),
 }
 ADMM = dict(kappa=5.0, iter_max=15, vset=1.03, vlow=0.95, vhigh=1.05)   # revs_config.yaml / revs_fixture.py:255-259
+DUMP_HOMES = 8192     # homes (rows) written by --dump-outputs: 33 MB of float64 at the workloads' T = 96, kept below 64 MB
 
 
 def workload_shape(workload):
@@ -125,6 +127,22 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(len(r) >= 7 and r[3 + i].lower().startswith("active") for r in self.rows)]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm), "source": "nvml" if self.nvml is not None else "nvidia-smi"}
+
+
+def dump_outputs(path, s):
+    """Write what the caller of the timed path receives after its last step -- the schedule (Solver.results) and
+    the operator's estimate and multipliers (Solver.estimate) -- as float64 DIR/<name>.npy, so that two builds can be
+    compared output for output.  Populations above DUMP_HOMES homes are sampled: the same seeded set of homes every
+    run, listed in home_index.npy."""
+    res = s.results()
+    res["P_est"], res["Gamma"] = s.estimate()
+    H = s.H
+    rows = np.arange(H) if H <= DUMP_HOMES else np.sort(np.random.default_rng(0).choice(H, DUMP_HOMES, replace=False))
+    arrays = {k: (v[:, rows] if k == "diff" else v[rows]) for k, v in res.items()}     # diff is [iterations, homes]
+    arrays["home_index"] = rows
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def measured_peaks():
@@ -355,6 +373,8 @@ def run_gpu(args, rank, world, local_rank):
     total_homes = sum_over_ranks(H)
     value = total_homes * HOURS / (ms_step * 1e-3)
     last = s.stats()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, s)
 
     # ---- end-to-end leg: host buffers in, host results out, every step
     for _ in range(min(args.warmup, 1)):
@@ -614,7 +634,14 @@ def main():
     ap.add_argument("--tol", type=float, default=1e-3, help="stopping rule of the convergence leg (both ADMM residuals, kW)")
     ap.add_argument("--conv-iter-max", type=int, default=100)
     ap.add_argument("--no-convergence", action="store_true", help="skip the convergence leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed device-resident steps, write rank 0's results of the last step as DIR/<name>.npy "
+                         "(float64; a fixed sample of %d homes of larger populations)" % DUMP_HOMES)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl graft)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -162,6 +162,36 @@ def test_objective_sandwich_lower_bound():
     assert lb2 == lb and abs(dist2 - lb) <= 1e-9 * abs(lb)
 
 
+@pytest.mark.parametrize("H", [300, 20000])
+def test_dump_outputs_writes_a_fixed_sample(tmp_path, H):
+    """bench --dump-outputs: every result array of the solver as float64 .npy, rows (diff: columns) of the same
+    seeded sample of homes in every run, the whole population when it is small."""
+    import bench
+    T, iters = 96, 15
+    rng = np.random.default_rng(2)
+    res = dict(P_sch=rng.random((H, T)), P_ev=rng.random((H, T)), SOC=rng.random((H, T + 1)), diff=rng.random((iters, H)))
+    est = rng.random((H, T)), rng.random((H, T))
+
+    class Fake:
+        def results(self): return dict(res)
+        def estimate(self): return est
+    fake = Fake()
+    fake.H = H
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), fake)
+    n = min(H, bench.DUMP_HOMES)
+    idx = np.load(tmp_path / "a" / "home_index.npy")
+    assert idx.dtype == np.float64 and len(np.unique(idx)) == n
+    rows = idx.astype(np.int64)
+    want = dict(res, P_est=est[0], Gamma=est[1])
+    for name, a in want.items():
+        got = np.load(tmp_path / "a" / f"{name}.npy")
+        assert got.dtype == np.float64
+        assert np.array_equal(got, a[:, rows] if name == "diff" else a[rows]), name
+        assert np.array_equal(got, np.load(tmp_path / "b" / f"{name}.npy")), name
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20
+
+
 def test_pipelined_stats_combination():
     """PipelinedSolver.stats(): counters add up, total_ms is the longest pipeline, residuals recombine as RMS."""
     from revs_admm_b200.parallel import PipelinedSolver
