@@ -21,6 +21,7 @@
  *   revs_solve_individual                         lpsolver.py:430-460 solve_residence()
  *   revs_reliability                              drawing.py:29-78    compute_flows(),
  *                                                                     compute_voltage()
+ *   revs_network_check                            drawing.py:29-78    the same for every zone at once
  *   revs_get_results / revs_get_schedule(_ld)     lpsolver.py:289-290 return diff,P_sch,S,C
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
@@ -164,6 +165,48 @@ int revs_solve_individual(revs_solver* s, double* P_res, double* P_ev, double* S
  * 1/rating), may be NULL (=1). */
 int revs_reliability(revs_solver* s, int feeder, int kind, int n_rows, const int32_t* rows,
                      const double* scale, double vset, const double* P, double* out);
+
+/* Network check of the whole population (drawing.py:29-78 for every zone of the solver at once): the voltage at
+ * every node and the flow on every line, per step, and where the limits are violated.  One kernel walks every zone's
+ * tree (leaves -> root: flows F, root -> leaves: squared-voltage drops D = R P), O(nodes x T), no sensitivity
+ * matrix; every zone needs its tree (revs_set_feeder_tree(s)).
+ * source: REVS_NET_SCHEDULE / REVS_NET_ESTIMATE (schedule / operator estimate of the last ADMM run, already on the
+ * device, P ignored) or REVS_NET_HOST (P [H,T] from the host, compact home order of revs_create).
+ * "Total nodes" are the nodes of all zones concatenated in zone order (node_off of revs_set_feeder_trees); rows of
+ * voltage / loading, and scale, follow it.  voltage = sqrt(vset^2 - D) (REVS_REL_VOLTAGE), loading = scale * F
+ * (REVS_REL_FLOW, scale = signed 1/rating per edge, NULL = 1).  voltage, loading, zone_worst and summary may be NULL.
+ * Ties of every maximum go to the lowest (zone, node or residence, step); counts are exact: two calls give the same
+ * bytes, and the result of a zone does not depend on the other zones of the solver.
+ * REVS_ERR_ARG: a zone without tree (the message names it), SCHEDULE / ESTIMATE before any ADMM iteration, HOST
+ * without P, an unknown source, or not vlow <= vset < vhigh.  Synchronous on the utility stream; adds its launches to
+ * revs_stats.kernel_launches and changes no other state.  The breadth-first arrays it needs are built on its first
+ * call after the trees are set, its scratch on first use; both are kept until revs_destroy. */
+#define REVS_NET_SCHEDULE 0   /* P_sch of the last ADMM run (what revs_get_results returns)      */
+#define REVS_NET_ESTIMATE 1   /* P_est of the last ADMM run (what revs_get_estimate returns)     */
+#define REVS_NET_HOST 2       /* P [H,T] from the host, compact home order of revs_create        */
+
+typedef struct revs_network_summary {
+    double drop_max;           /* max over all nodes and steps of (R P) at the node, pu^2 (REVS_REL_DROP)          */
+    double v_min;              /* sqrt(vset^2 - drop_max), the REVS_REL_VOLTAGE formula                           */
+    int32_t drop_zone, drop_node, drop_step;   /* where (node index local to its zone, as in revs_reliability)    */
+    int32_t pad0_;
+    double row_excess_max;     /* max over RESIDENCES and steps of (R P)_res - (vhigh^2 - vset^2): the voltage row
+                                  of the operator QP (revs_admm_begin); > 0 = violated; -inf without residences  */
+    int32_t excess_zone, excess_res, excess_step, pad1_;   /* excess_res: home index local to its zone; -1: none  */
+    int64_t rows_violated;     /* (residence, step) pairs with excess > row_tol                                   */
+    int64_t nodes_below_vlow;  /* (node, step) pairs with drop > vset^2 - vlow^2                                  */
+    double loading_max;        /* max over edges and steps of |scale[e] * flow_e| (REVS_REL_FLOW)                 */
+    int32_t loading_zone, loading_node, loading_step, pad2_;
+    int64_t edges_overloaded;  /* (edge, step) pairs with |loading| > 1; 0 when scale == NULL                      */
+} revs_network_summary;
+
+int revs_network_check(revs_solver* s, int source, const double* P, double vset, double vlow, double vhigh,
+                       double row_tol,
+                       const double* scale,        /* [total nodes] signed 1/rating per edge, or NULL (= 1)     */
+                       double* voltage,            /* [total nodes, T] or NULL                                  */
+                       double* loading,            /* [total nodes, T] or NULL                                  */
+                       double* zone_worst,         /* [n_feeders, 3]: drop_max, row_excess_max, loading_max     */
+                       revs_network_summary* summary);
 
 /* The same check with the ROWS PARTITIONED over the GPUs of one box (one process per GPU, every process holds the
  * feeder's tree; BASELINE north_star: "the sensitivity contraction is row-partitioned"): every rank builds and

@@ -12,6 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("REVS_LIB") or os.path.join(HERE, "librevs_admm.so")     # REVS_LIB: a build variant (profiles/build_variants.sh)
 
 REVS_REL_VOLTAGE, REVS_REL_FLOW, REVS_REL_DROP = 0, 1, 2
+REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST = 0, 1, 2
 
 
 class RevsError(RuntimeError):
@@ -32,6 +33,21 @@ class Stats(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+class NetworkSummary(C.Structure):
+    """revs_network_summary: worst voltage drop, voltage-row excess and line loading of a population, where they
+    are (zone, node or residence local to its zone, step) and the violation counts."""
+    _fields_ = [("drop_max", C.c_double), ("v_min", C.c_double),
+                ("drop_zone", C.c_int32), ("drop_node", C.c_int32), ("drop_step", C.c_int32), ("pad0_", C.c_int32),
+                ("row_excess_max", C.c_double),
+                ("excess_zone", C.c_int32), ("excess_res", C.c_int32), ("excess_step", C.c_int32), ("pad1_", C.c_int32),
+                ("rows_violated", C.c_int64), ("nodes_below_vlow", C.c_int64), ("loading_max", C.c_double),
+                ("loading_zone", C.c_int32), ("loading_node", C.c_int32), ("loading_step", C.c_int32), ("pad2_", C.c_int32),
+                ("edges_overloaded", C.c_int64)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if not k.startswith("pad")}
 
 
 _P = C.c_void_p
@@ -73,6 +89,8 @@ SIGNATURES = {
     "revs_gather_export": ([_P, C.c_int64, C.c_void_p], C.c_int),
     "revs_gather_attach": ([_P, C.c_int, C.c_int, C.c_void_p], C.c_int),
     "revs_reliability_sharded": ([_P, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), _D, C.c_double, _D, _D], C.c_int),
+    "revs_network_check": ([_P, C.c_int, _D, C.c_double, C.c_double, C.c_double, C.c_double, _D, _D, _D, _D,
+                            C.POINTER(NetworkSummary)], C.c_int),
 }
 
 _lib = None
@@ -183,6 +201,7 @@ class Solver:
         self.sizes = [int(n) for n in feeder_sizes]
         self.off = np.concatenate([[0], np.cumsum(self.sizes)]).astype(np.int64)
         self.H, self.T, self.nf = int(self.off[-1]), int(T), len(self.sizes)
+        self.node_counts = [None] * self.nf        # nodes of every zone's tree, as given to set_feeder_tree(s)
         self._h = _P()
         _check(self.lib.revs_create(C.byref(self._h), device, self.nf,
                                     self.off.ctypes.data_as(C.POINTER(C.c_int64)), self.T))
@@ -214,6 +233,7 @@ class Solver:
         i32 = C.POINTER(C.c_int32)
         _check(self.lib.revs_set_feeder_tree(self._h, feeder, len(parent), parent.ctypes.data_as(i32),
                                              _dp(r), res_node.ctypes.data_as(i32)))
+        self.node_counts[feeder] = len(parent)
 
     def pack_trees(self, trees):
         """The concatenated arrays revs_set_feeder_trees takes, from feeder.FeederTree-like objects (parent, r, res_node)."""
@@ -231,6 +251,7 @@ class Solver:
         i32 = C.POINTER(C.c_int32)
         _check(self.lib.revs_set_feeder_trees(self._h, node_off.ctypes.data_as(C.POINTER(C.c_int64)),
                                               parent.ctypes.data_as(i32), _dp(r), res.ctypes.data_as(i32)))
+        self.node_counts = np.diff(node_off).astype(int).tolist()
 
     def set_homes(self, load, has_ev, rating, capacity, initial, start, end):
         H, T = self.H, self.T
@@ -345,6 +366,43 @@ class Solver:
                                          rows.ctypes.data_as(C.POINTER(C.c_int32)), _dp(sc), vset,
                                          _dp(Pp), _dp(out)))
         return out
+
+    @property
+    def total_nodes(self):
+        """Nodes of all zones concatenated in zone order: the rows of network_check's arrays."""
+        return int(sum(n or 0 for n in self.node_counts))
+
+    def network_check(self, source="schedule", vset=1.0, vlow=0.95, vhigh=1.05, row_tol=1e-9, scale=None, full=False,
+                      zones=False, out=None):
+        """Voltages and line loadings of every node of every zone, per step, in one call (include/revs_admm.h:
+        revs_network_check).  source: "schedule" (P_sch of the last ADMM run), "estimate" (P_est) or a host schedule
+        P [H, T].  scale: [total_nodes] signed 1/rating per edge (None = 1).  Returns dict(summary=dict,
+        voltage=[total_nodes, T], loading=[total_nodes, T], zone_worst=[zones, 3]); the arrays are None unless
+        asked for with full / zones.  out: optional dict of C-contiguous float64 [total_nodes, T] arrays voltage
+        and loading to write into."""
+        N, T = self.total_nodes, self.T
+        Pp = None
+        if isinstance(source, str):
+            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE}.get(source)
+            if src is None:
+                raise ValueError(f"source must be 'schedule', 'estimate' or an [H, T] array, not {source!r}")
+        else:
+            src, Pp = REVS_NET_HOST, _f64(source, (self.H, T))
+        sc = None if scale is None else _f64(scale, (N,))
+        V = L = None
+        if full:
+            if out is not None:
+                V, L = out["voltage"], out["loading"]
+                for a in (V, L):
+                    if a.shape != (N, T) or a.dtype != np.float64 or not a.flags.c_contiguous:
+                        raise ValueError(f"out arrays must be C-contiguous float64 of shape {(N, T)}")
+            else:
+                V, L = np.empty((N, T)), np.empty((N, T))
+        Z = np.empty((self.nf, 3)) if zones else None
+        summ = NetworkSummary()
+        _check(self.lib.revs_network_check(self._h, src, _dp(Pp), vset, vlow, vhigh, row_tol, _dp(sc), _dp(V), _dp(L),
+                                           _dp(Z), C.byref(summ)))
+        return dict(summary=summ.as_dict(), voltage=V, loading=L, zone_worst=Z)
 
     # ---- the same check with the rows partitioned over the GPUs of the box; the all-gather of the result is fused
     # into the epilogue of the contraction kernel (peer-memory stores, include/revs_admm.h: revs_gather_*)

@@ -294,4 +294,55 @@ cudaError_t launch_pack_rows(const double* src, double* dst, const int64_t* hmap
 cudaError_t launch_hour_mask(const double* p_ev, const int64_t* hmap, int64_t H, int T, unsigned long long* out, cudaStream_t s);
 cudaError_t launch_to_time_major(const double* in, int n, int T, double* out, int64_t ld, cudaStream_t s);
 
+// ---- network_check.cu
+constexpr int kNetMaxSteps = 32;                      // steps per CTA (G) at most
+constexpr size_t kNetSmemSmall = 112 * 1024;          // state of a CTA of the first class: two CTAs per SM
+constexpr size_t kNetSmemMax = 224 * 1024;            // one step of a zone above this (28,672 nodes) runs on global scratch
+struct NetNode {          // one node of a zone in breadth-first position (children of a node are contiguous in the next level)
+    double r;             // resistance of the edge above the node: cumr[i] - cumr[parent[i]]
+    int node;             // local node index (row of the outputs)
+    int parent;           // breadth-first position of the parent, -1 = substation
+    int child0, nchild;   // breadth-first positions of the children
+    int res0, nres;       // the node's residences: entries res0.. of the zone's residence list (ascending home index)
+};
+struct NetZone {
+    int64_t node0, lvl0, res0;    // first entry of the zone in the node / level / residence pools
+    int64_t home_row;             // padded row of the zone's first home in the [Hp][T] schedule
+    int64_t out_row;              // first row of the zone in the [total nodes][T] outputs
+    int n_nodes, depth, lg, pad_; // lg: log2 of the steps per CTA
+};
+struct NetCta { int zone, t0; int64_t gstate; };     // gstate: offset of the state in the global scratch, -1: shared memory
+struct NetArg { double v; int zone, pad_; int64_t loc; };   // a maximum and where: loc = index * T + step
+struct NetPartial { NetArg drop, exc, load; unsigned long long rows, low, over; };
+struct NetParams {
+    const NetZone* zones;
+    const NetNode* nodes;
+    const int* levels;            // per zone: depth + 1 breadth-first positions
+    const int* res;               // per zone: local home indices, grouped by node
+    const NetCta* ctas;
+    const double* P;              // [Hp][T]
+    const double* scale;          // [total nodes] or null (= 1)
+    double* voltage;              // [total nodes][T] or null
+    double* loading;              // [total nodes][T] or null
+    double* gstate;               // global scratch of the zones above kNetSmemMax
+    NetPartial* part;             // [CTAs]
+    int T;
+    double v2, u, low, row_tol;   // vset^2, vhigh^2 - vset^2, vset^2 - vlow^2, tolerance of the row count
+};
+struct NetHost {                  // host side of the arrays above, built once per set of trees
+    std::vector<NetZone> zones;
+    std::vector<NetNode> nodes;
+    std::vector<int> levels, res, lists, zone_cta;
+    std::vector<NetCta> ctas;
+    int class_off[4] = {0, 0, 0, 0};        // lists[class_off[c] ..] = CTAs of class c: shared <= kNetSmemSmall, shared, global
+    size_t class_smem[3] = {0, 0, 0};
+    int64_t gstate_doubles = 0, total_nodes = 0;
+};
+void net_add_zone(NetHost& h, int n_nodes, const int* parent, const double* cumr, int n_res, const int* res_node,
+                  int64_t home_row);
+void net_finish(NetHost& h, int T);
+cudaError_t launch_network_check(const NetParams& P, const int* d_list, int n_ctas, size_t smem, cudaStream_t s);
+cudaError_t launch_network_reduce(const NetPartial* part, const int* zone_cta, int n_zones, double* zone_worst,
+                                  NetPartial* out, cudaStream_t s);
+
 }  // namespace revs

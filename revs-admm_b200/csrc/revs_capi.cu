@@ -199,6 +199,19 @@ struct revs_solver {
     double* d_pool_cumr = nullptr;
     int64_t* d_pool_off = nullptr;
     size_t pool_nodes = 0;
+    // population network check (revs_network_check, network_check.cu): breadth-first zone arrays, built on its first
+    // call after the trees were set, and its scratch, kept until revs_destroy
+    bool net_valid = false;
+    NetHost net;
+    NetZone* d_net_zones = nullptr;
+    NetNode* d_net_nodes = nullptr;
+    int *d_net_levels = nullptr, *d_net_res = nullptr, *d_net_lists = nullptr, *d_net_zone_cta = nullptr;
+    NetCta* d_net_ctas = nullptr;
+    NetPartial *d_net_part = nullptr, *d_net_sum = nullptr;
+    double *d_net_zw = nullptr, *d_net_gstate = nullptr, *d_net_P = nullptr, *d_net_scale = nullptr, *d_net_volt = nullptr,
+           *d_net_load = nullptr;
+    size_t net_cap[6] = {0, 0, 0, 0, 0, 0};    // elements allocated: nodes, levels, residences, CTAs, zones, global state
+    bool net_scale_ok = false, net_out_ok = false;
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -1123,7 +1136,9 @@ void free_all(revs_solver* s) {
                     s->d_cprob, s->d_ctiles, s->d_respart, s->d_dsum, s->d_t_perm, s->d_t_iperm, s->d_t_nodeA, s->d_t_nodeB, s->d_t_cnt,
                     s->d_t_c, s->d_t_d, s->d_t_e, s->d_t_wA, s->d_t_wB, s->d_t_zoff, s->d_tree_cols[0], s->d_tree_cols[1], s->d_tree_cols[2],
                     s->d_tree_cols[3], s->d_nt_zones, s->d_nt_lvl, s->d_nt_parent, s->d_nt_home, s->d_nt_hnode, s->d_nt_wsi, s->d_nt_child, s->d_nt_homes, s->d_nt_rho,
-                    s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2};
+                    s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2, s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists,
+                    s->d_net_zone_cta, s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_P,
+                    s->d_net_scale, s->d_net_volt, s->d_net_load};
     for (int r = 0; r < kMaxPeers; ++r)
         if (s->peer_box[r] && s->peer_box[r] != s->d_mailbox) cudaIpcCloseMemHandle(s->peer_box[r]);
     for (int r = 0; r < kGatherMaxPeers; ++r)
@@ -1377,6 +1392,7 @@ int revs_set_feeder_tree(revs_solver* s, int feeder, int n_nodes, const int32_t*
     Tree& t = s->trees[feeder];
     if (t.d_parent && !t.pooled) { cudaFree(t.d_parent); cudaFree(t.d_cumr); cudaFree(t.d_res_node); }
     t = Tree();
+    s->net_valid = false;
     t.n_nodes = n_nodes;
     CU(dalloc(&t.d_parent, (size_t)n_nodes));
     CU(dalloc(&t.d_cumr, (size_t)n_nodes));
@@ -1437,6 +1453,7 @@ int revs_set_feeder_trees(revs_solver* s, const int64_t* node_off, const int32_t
             res_p[s->feeders[f].off + (j - s->off[f])] = res_node[j];
         }
     }
+    s->net_valid = false;
     if (s->pool_nodes < (size_t)total) {
         if (s->d_pool_parent) { cudaFree(s->d_pool_parent); cudaFree(s->d_pool_cumr); s->d_pool_parent = nullptr; s->d_pool_cumr = nullptr; }
         CU(dalloc(&s->d_pool_parent, (size_t)total));
@@ -2252,6 +2269,155 @@ int revs_reliability(revs_solver* s, int feeder, int kind, int n_rows, const int
 int revs_reliability_sharded(revs_solver* s, int feeder, int kind, int n_rows, const int32_t* rows, const double* scale,
                              double vset, const double* P, double* out) {
     return reliability_impl(s, feeder, kind, n_rows, rows, scale, vset, P, out, true);
+}
+
+}  // extern "C"
+
+namespace {
+// The breadth-first arrays of revs_network_check, from the trees on the device (nothing of this runs in
+// revs_set_feeder_tree(s), which the schedule path times end to end).
+int net_prepare(revs_solver* s) {
+    if (s->net_valid) return REVS_OK;
+    for (int f = 0; f < s->nf; ++f)
+        if (!s->trees[f].d_parent)
+            return fail(REVS_ERR_ARG, "zone %d has no tree (given as a sensitivity block): the network check needs "
+                        "revs_set_feeder_tree(s)", f);
+    NetHost h;
+    std::vector<int> par, res;
+    std::vector<double> cumr;
+    for (int f = 0; f < s->nf; ++f) {
+        const Tree& t = s->trees[f];
+        const FeederDev& fd = s->feeders[f];
+        par.resize(t.n_nodes);
+        cumr.resize(t.n_nodes);
+        res.resize(fd.n);
+        CU(cudaMemcpy(par.data(), t.d_parent, sizeof(int) * t.n_nodes, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(cumr.data(), t.d_cumr, sizeof(double) * t.n_nodes, cudaMemcpyDeviceToHost));
+        if (fd.n) CU(cudaMemcpy(res.data(), t.d_res_node, sizeof(int) * fd.n, cudaMemcpyDeviceToHost));
+        net_add_zone(h, t.n_nodes, par.data(), cumr.data(), fd.n, res.data(), fd.off);
+    }
+    net_finish(h, s->T);
+    // the arrays below depend on the trees; the host-input staging d_net_P does not
+    void* old[] = {s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists, s->d_net_zone_cta,
+                   s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_scale, s->d_net_volt,
+                   s->d_net_load};
+    for (void* p : old)
+        if (p) cudaFree(p);
+    s->d_net_zones = nullptr; s->d_net_nodes = nullptr; s->d_net_levels = nullptr; s->d_net_res = nullptr;
+    s->d_net_lists = nullptr; s->d_net_zone_cta = nullptr; s->d_net_ctas = nullptr; s->d_net_part = nullptr;
+    s->d_net_sum = nullptr; s->d_net_zw = nullptr; s->d_net_gstate = nullptr; s->d_net_scale = nullptr;
+    s->d_net_volt = nullptr; s->d_net_load = nullptr;
+    CU(dalloc(&s->d_net_zones, h.zones.size()));
+    CU(dalloc(&s->d_net_nodes, h.nodes.size()));
+    CU(dalloc(&s->d_net_levels, h.levels.size()));
+    CU(dalloc(&s->d_net_res, h.res.size()));
+    CU(dalloc(&s->d_net_lists, h.lists.size()));
+    CU(dalloc(&s->d_net_zone_cta, h.zone_cta.size()));
+    CU(dalloc(&s->d_net_ctas, h.ctas.size()));
+    CU(dalloc(&s->d_net_part, h.ctas.size()));
+    CU(dalloc(&s->d_net_sum, (size_t)1));
+    CU(dalloc(&s->d_net_zw, (size_t)3 * s->nf));
+    CU(dalloc(&s->d_net_gstate, (size_t)h.gstate_doubles));
+    CU(cudaMemcpy(s->d_net_zones, h.zones.data(), sizeof(NetZone) * h.zones.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_net_nodes, h.nodes.data(), sizeof(NetNode) * h.nodes.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_net_levels, h.levels.data(), sizeof(int) * h.levels.size(), cudaMemcpyHostToDevice));
+    if (!h.res.empty()) CU(cudaMemcpy(s->d_net_res, h.res.data(), sizeof(int) * h.res.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_net_lists, h.lists.data(), sizeof(int) * h.lists.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_net_zone_cta, h.zone_cta.data(), sizeof(int) * h.zone_cta.size(), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(s->d_net_ctas, h.ctas.data(), sizeof(NetCta) * h.ctas.size(), cudaMemcpyHostToDevice));
+    s->net = std::move(h);
+    s->net_valid = true;
+    return REVS_OK;
+}
+
+void net_location(const NetArg& a, int T, int32_t* zone, int32_t* index, int32_t* step) {
+    const bool none = a.loc == INT64_MAX;      // no candidate (no residence at all)
+    *zone = none ? -1 : a.zone;
+    *index = none ? -1 : (int32_t)(a.loc / T);
+    *step = none ? -1 : (int32_t)(a.loc % T);
+}
+}  // namespace
+
+extern "C" {
+
+int revs_network_check(revs_solver* s, int source, const double* P, double vset, double vlow, double vhigh, double row_tol,
+                       const double* scale, double* voltage, double* loading, double* zone_worst,
+                       revs_network_summary* summary) {
+    if (!s) return fail(REVS_ERR_ARG, "null solver");
+    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST)
+        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE or REVS_NET_HOST)", source);
+    if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
+    if (source != REVS_NET_HOST && s->k == 0)
+        return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check", source == REVS_NET_SCHEDULE ? "schedule" : "estimate");
+    const double v2 = vset * vset, u = vhigh * vhigh - v2, lo = vlow * vlow - v2;
+    if (!(u > 0.0) || !(lo <= 0.0)) return fail(REVS_ERR_ARG, "need vlow <= vset < vhigh");
+    CU(cudaSetDevice(s->device));
+    int rc = net_prepare(s);
+    if (rc) return rc;
+    const NetHost& h = s->net;
+    const int T = s->T;
+    const size_t out_elems = (size_t)h.total_nodes * T;
+    int64_t launches = 0;
+    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : s->d_pest;
+    if (source == REVS_NET_HOST) {
+        if (!s->d_net_P) CU(dalloc(&s->d_net_P, (size_t)s->Hp * T));
+        if ((rc = h2d_homes(s, s->d_net_P, P, T))) return rc;
+        launches += s->H > 0;
+        src = s->d_net_P;
+    }
+    if (scale) {
+        if (!s->d_net_scale) CU(dalloc(&s->d_net_scale, (size_t)h.total_nodes));
+        CU(cudaMemcpyAsync(s->d_net_scale, scale, sizeof(double) * h.total_nodes, cudaMemcpyHostToDevice, s->sU));
+    }
+    if (voltage && !s->d_net_volt) CU(dalloc(&s->d_net_volt, out_elems));
+    if (loading && !s->d_net_load) CU(dalloc(&s->d_net_load, out_elems));
+    NetParams prm{};
+    prm.zones = s->d_net_zones;
+    prm.nodes = s->d_net_nodes;
+    prm.levels = s->d_net_levels;
+    prm.res = s->d_net_res;
+    prm.ctas = s->d_net_ctas;
+    prm.P = src;
+    prm.scale = scale ? s->d_net_scale : nullptr;
+    prm.voltage = voltage ? s->d_net_volt : nullptr;
+    prm.loading = loading ? s->d_net_load : nullptr;
+    prm.gstate = s->d_net_gstate;
+    prm.part = s->d_net_part;
+    prm.T = T;
+    prm.v2 = v2;
+    prm.u = u;
+    prm.low = -lo;
+    prm.row_tol = row_tol;
+    for (int c = 0; c < 3; ++c) {
+        const int n = h.class_off[c + 1] - h.class_off[c];
+        if (n == 0) continue;
+        CU(launch_network_check(prm, s->d_net_lists + h.class_off[c], n, c == 2 ? 0 : h.class_smem[c], s->sU));
+        ++launches;
+    }
+    CU(launch_network_reduce(s->d_net_part, s->d_net_zone_cta, s->nf, s->d_net_zw, s->d_net_sum, s->sU));
+    ++launches;
+    NetPartial m;
+    CU(cudaMemcpyAsync(&m, s->d_net_sum, sizeof m, cudaMemcpyDeviceToHost, s->sU));
+    if (zone_worst) CU(cudaMemcpyAsync(zone_worst, s->d_net_zw, sizeof(double) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
+    if (voltage) CU(cudaMemcpyAsync(voltage, s->d_net_volt, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
+    if (loading) CU(cudaMemcpyAsync(loading, s->d_net_load, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->stats.kernel_launches += launches;
+    if (summary) {
+        revs_network_summary o{};
+        o.drop_max = m.drop.v;
+        o.v_min = std::sqrt(v2 - m.drop.v);
+        net_location(m.drop, T, &o.drop_zone, &o.drop_node, &o.drop_step);
+        o.row_excess_max = m.exc.v;
+        net_location(m.exc, T, &o.excess_zone, &o.excess_res, &o.excess_step);
+        o.rows_violated = (int64_t)m.rows;
+        o.nodes_below_vlow = (int64_t)m.low;
+        o.loading_max = m.load.v;
+        net_location(m.load, T, &o.loading_zone, &o.loading_node, &o.loading_step);
+        o.edges_overloaded = (int64_t)m.over;
+        *summary = o;
+    }
+    return REVS_OK;
 }
 
 int revs_gather_export(revs_solver* s, int64_t capacity_doubles, void* handle64) {

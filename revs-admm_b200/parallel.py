@@ -112,6 +112,37 @@ def run_admm(stepper, kappa=5.0, iter_max=15, vset=1.0, vlow=0.95, vhigh=1.05, t
     return iter_max, history
 
 
+# maxima of a network-check summary: value, zone, (index, step) and the fields that travel with the value
+_NET_MAXIMA = (("drop_max", "drop_zone", "drop_node", "drop_step", ("v_min",)),
+               ("row_excess_max", "excess_zone", "excess_res", "excess_step", ()),
+               ("loading_max", "loading_zone", "loading_node", "loading_step", ()))
+_NET_COUNTS = ("rows_violated", "nodes_below_vlow", "edges_overloaded")
+
+
+def merge_network_summaries(summaries, zone_offsets):
+    """One network-check summary (Solver.network_check()["summary"]) from those of solvers that hold consecutive
+    blocks of the zones: part k's zone z is zone zone_offsets[k] + z of the whole.  The rule of the library: every
+    maximum goes to the largest value, ties to the lowest (zone, index, step); a part without a candidate (zone -1,
+    e.g. no residence) is skipped; counts are summed."""
+    out = dict(summaries[0])
+    for key in _NET_COUNTS:
+        out[key] = int(sum(int(s[key]) for s in summaries))
+    for val, zk, ik, tk, extra in _NET_MAXIMA:
+        best, win = None, None
+        for s, z0 in zip(summaries, zone_offsets):
+            if s[zk] < 0:
+                continue
+            key = (s[val], int(z0) + s[zk], s[ik], s[tk])
+            if best is None or key[0] > best[0] or (key[0] == best[0] and key[1:] < best[1:]):
+                best, win = key, s
+        if best is None:
+            out.update({val: -np.inf, zk: -1, ik: -1, tk: -1})
+        else:
+            out.update({val: best[0], zk: best[1], ik: best[2], tk: best[3]})
+            out.update({e: win[e] for e in extra})
+    return out
+
+
 def _pinned_empty(shape):
     """Page-locked host scratch (torch is only the allocator); plain numpy if torch has no CUDA."""
     try:
@@ -328,6 +359,35 @@ class PipelinedSolver:
             pe[lo:hi], gm[lo:hi] = self.parts[k].estimate()
         self._each(f)
         return pe, gm
+
+    def network_check(self, source="schedule", scale=None, full=False, zones=False, **kw):
+        """Solver.network_check over all pipelines at once: every pipeline checks its zones concurrently and writes
+        its contiguous block of nodes into the [total nodes, T] arrays; the summaries are merged with the zones
+        numbered over the whole population (merge_network_summaries), zone_worst is concatenated in zone order.
+        The result is that of a single solver, bit for bit."""
+        node_off = np.concatenate([[0], np.cumsum([p.total_nodes for p in self.parts])]).astype(np.int64)
+        N, T = int(node_off[-1]), self.T
+        host = not isinstance(source, str)
+        if host:
+            source = np.ascontiguousarray(source, dtype=np.float64)
+            if source.shape != (self.H, T):
+                raise ValueError(f"expected shape {(self.H, T)}, got {source.shape}")
+        if scale is not None:
+            scale = np.ascontiguousarray(scale, dtype=np.float64)
+            if scale.shape != (N,):
+                raise ValueError(f"expected shape {(N,)}, got {scale.shape}")
+        out = dict(voltage=np.empty((N, T)), loading=np.empty((N, T))) if full else None
+
+        def f(k):
+            lo, hi = self.rows[k]
+            a, b = node_off[k], node_off[k + 1]
+            return self.parts[k].network_check(source=source[lo:hi] if host else source,
+                                               scale=None if scale is None else scale[a:b], full=full, zones=zones,
+                                               out=None if out is None else {n: v[a:b] for n, v in out.items()}, **kw)
+        res = self._each(f)
+        return dict(summary=merge_network_summaries([r["summary"] for r in res], [a for a, _ in self.cuts]),
+                    voltage=None if out is None else out["voltage"], loading=None if out is None else out["loading"],
+                    zone_worst=np.concatenate([r["zone_worst"] for r in res]) if zones else None)
 
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
