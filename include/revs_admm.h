@@ -26,7 +26,7 @@
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
  *                                                 drawing.py:29-78 for one feeder over several GPUs (rows partitioned)
- *   revs_comm_export / revs_comm_attach / revs_comm_detach / revs_zone_arrays
+ *   revs_comm_export / revs_comm_attach / revs_comm_detach
  *                                                 no reference counterpart (library plumbing; the reference is one process)
  */
 #ifndef REVS_ADMM_H
@@ -234,15 +234,6 @@ int revs_contract(int device, int M, int K, int T, const double* A, const double
 int revs_screen_contract(int device, int M, int K, int T, const double* A, const double* B, double* C,
                          int impl);
 
-/* Host-only helper (no GPU needed): the static per-zone arrays the tree-structured operator kernel derives from a
- * radial zone (csrc/tree_qp.cu) -- with the residences in depth-first order perm[], R[i][j] = min(c[i..j-1]) and
- * R g is three prefix sums over the Cartesian tree of c (nodes as lo | hi << 16, sorted by lo and by hi, weights w,
- * cnt = #nodes with lo <= p | (#nodes with hi < p) << 16).  Every output has n_res entries.  Exposed so that the
- * decomposition can be checked against compute_Rmat (lpsolver.py:17-26) without a device. */
-int revs_zone_arrays(int n_nodes, const int32_t* parent, const double* r, int n_res, const int32_t* res_node, int32_t* perm,
-                     double* c, double* d, double* e, int32_t* node_lo, double* w_lo, int32_t* node_hi, double* w_hi,
-                     int32_t* cnt);
-
 /* Global stopping rule over the GPUs of one box (one process per GPU, each with its own revs_solver over its
  * share of the feeders): the residual sums of revs_stats / revs_admm_step / the tol test of revs_solve_admm then
  * run over ALL ranks.  The all-reduce happens inside the fused dual-update kernel, through mailboxes in peer
@@ -256,9 +247,7 @@ int revs_comm_export(revs_solver* s, void* handle64);
 int revs_comm_attach(revs_solver* s, int world, int rank, const void* handles);
 int revs_comm_detach(revs_solver* s);
 
-/* Options: "tree" (default 0; set it BEFORE revs_set_feeder_tree(s)) = zones given as trees (up to 320 residences) are
- * solved by the tree-structured kernel, which needs no sensitivity matrix (rows and products of R from O(n) static
- * arrays); 0 = dense kernels (BF16 tensor-core screening + FP64 rows of R), the faster of the two on B200.  "graph" (default 1) = revs_solve_admm runs the whole loop from one captured CUDA graph whose loops
+/* Options: "graph" (default 1) = revs_solve_admm runs the whole loop from one captured CUDA graph whose loops
  * (ADMM iterations, working-set rounds) are decided on the device; 0 = host-driven loop with CUDA-event spans per
  * kernel family in revs_stats (profiling).  "screen" (default 1) = BF16 tensor-core screening of the voltage rows with exact
  * FP64 recheck of the candidates inside the loop; 0 = FP64 DMMA contraction of every row.

@@ -81,8 +81,6 @@ SIGNATURES = {
     "revs_set_option": ([_P, C.c_char_p, C.c_double], C.c_int),
     "revs_screen_contract": ([C.c_int, C.c_int, C.c_int, C.c_int, _D, _D, _D, C.c_int], C.c_int),
     "revs_get_stats": ([_P, C.POINTER(Stats)], C.c_int),
-    "revs_zone_arrays": ([C.c_int, C.POINTER(C.c_int32), _D, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32), _D, _D, _D,
-                          C.POINTER(C.c_int32), _D, C.POINTER(C.c_int32), _D, C.POINTER(C.c_int32)], C.c_int),
     "revs_comm_export": ([_P, C.c_void_p], C.c_int),
     "revs_comm_attach": ([_P, C.c_int, C.c_int, C.c_void_p], C.c_int),
     "revs_comm_detach": ([_P], C.c_int),
@@ -172,25 +170,6 @@ def expand_schedule(mask, T, has_ev, rating, capacity, initial):
     for k in range(T):
         soc[:, k + 1] = soc[:, k] + inc[:, k]
     return p_ev, soc
-
-
-def zone_arrays(parent, r, res_node):
-    """Static arrays of the tree-structured operator kernel for one radial zone (host only, no GPU):
-    dict(perm, c, d, e, lo, hi, w) with the Cartesian-tree nodes in lo-order, plus the hi-order copy and cnt."""
-    parent = np.ascontiguousarray(parent, dtype=np.int32)
-    r = _f64(r, (len(parent),))
-    res_node = np.ascontiguousarray(res_node, dtype=np.int32)
-    n = len(res_node)
-    i32 = C.POINTER(C.c_int32)
-    I = lambda: np.zeros(n, dtype=np.int32)
-    perm, nlo, nhi, cnt = I(), I(), I(), I()
-    c, d, e, wlo, whi = (np.zeros(n) for _ in range(5))
-    _check(load().revs_zone_arrays(len(parent), parent.ctypes.data_as(i32), _dp(r), n, res_node.ctypes.data_as(i32),
-                                   perm.ctypes.data_as(i32), _dp(c), _dp(d), _dp(e), nlo.ctypes.data_as(i32), _dp(wlo),
-                                   nhi.ctypes.data_as(i32), _dp(whi), cnt.ctypes.data_as(i32)))
-    m = max(n - 1, 0)
-    return dict(perm=perm, c=c[:m], d=d, e=e, lo=nlo[:m] & 0xffff, hi=nlo[:m] >> 16, w=wlo[:m],
-                lo_b=nhi[:m] & 0xffff, hi_b=nhi[:m] >> 16, w_b=whi[:m], cnt_lo=cnt & 0xffff, cnt_hi=cnt >> 16)
 
 
 class Solver:

@@ -180,4 +180,47 @@ cudaError_t launch_to_time_major(const double* in, int n, int T, double* out, in
     return cudaGetLastError();
 }
 
+void bfs_tree(int n_nodes, const int* parent, int n_res, const int* res_node, BfsTree& B) {
+    const int n = n_nodes;
+    // children and residences of every node, ascending
+    std::vector<int> cofs(n + 1, 0), kids(n), rofs(n + 1, 0), homes(n_res);
+    for (int i = 0; i < n; ++i)
+        if (parent[i] >= 0) ++cofs[parent[i] + 1];
+    for (int j = 0; j < n_res; ++j) ++rofs[res_node[j] + 1];
+    for (int i = 0; i < n; ++i) { cofs[i + 1] += cofs[i]; rofs[i + 1] += rofs[i]; }
+    {
+        std::vector<int> fill(cofs.begin(), cofs.end() - 1);
+        for (int i = 0; i < n; ++i)
+            if (parent[i] >= 0) kids[fill[parent[i]]++] = i;
+        std::vector<int> rf(rofs.begin(), rofs.end() - 1);
+        for (int j = 0; j < n_res; ++j) homes[rf[res_node[j]]++] = j;
+    }
+    B.order.clear();
+    B.order.reserve(n);
+    for (int i = 0; i < n; ++i)
+        if (parent[i] < 0) B.order.push_back(i);
+    B.lvl.assign(1, 0);
+    for (size_t lo = 0; lo < B.order.size();) {
+        const size_t hi = B.order.size();
+        B.lvl.push_back((int)hi);
+        for (size_t q = lo; q < hi; ++q)
+            for (int e = cofs[B.order[q]]; e < cofs[B.order[q] + 1]; ++e) B.order.push_back(kids[e]);
+        lo = hi;
+    }
+    std::vector<int> pos(n);
+    for (int q = 0; q < n; ++q) pos[B.order[q]] = q;
+    B.parent.resize(n); B.child0.resize(n); B.nchild.resize(n); B.res0.resize(n); B.nres.resize(n);
+    B.res.clear();
+    B.res.reserve(n_res);
+    for (int q = 0; q < n; ++q) {
+        const int i = B.order[q];
+        B.parent[q] = parent[i] < 0 ? -1 : pos[parent[i]];
+        B.nchild[q] = cofs[i + 1] - cofs[i];
+        B.child0[q] = B.nchild[q] ? pos[kids[cofs[i]]] : 0;
+        B.res0[q] = (int)B.res.size();
+        B.nres[q] = rofs[i + 1] - rofs[i];
+        B.res.insert(B.res.end(), homes.begin() + rofs[i], homes.begin() + rofs[i + 1]);
+    }
+}
+
 }  // namespace revs

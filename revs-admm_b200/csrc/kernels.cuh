@@ -179,26 +179,6 @@ cudaError_t launch_utility_qp_fast(const QpParams& P, cudaStream_t stream);
 // mode 1: later rounds (every running column); mode 2: sweep (columns handed over in this round)
 cudaError_t launch_order_columns(const QpParams& P, int mode, int* order, int* order_count, cudaStream_t stream);
 
-// ---- tree_qp.cu: the operator QP on the feeder tree (no sensitivity matrix)
-struct TreeParams {             // static per-zone arrays (layout: tree_qp.cu:ZonePtr)
-    const int64_t* zoff;        // [n_feeders] offset of the zone in the strided pools (32 NJ entries per zone)
-    const int* perm;            // strided: home index of every depth-first position
-    const int* iperm;           // [Hp] at FeederDev::off + home: depth-first position
-    const double* c;            // strided: c[p] = 2 cumr(lca(p, p+1))
-    const double* d;            // strided: R[p][p]
-    const double* e;            // strided: d[p] - max(c[p-1], c[p])
-    const int* nodeA;           // strided: Cartesian-tree nodes in lo-order, shared-memory slots of G[hi] | G[lo-1] << 16
-    const double* wA;
-    const int* permB;           // strided: nodes in hi-order -> slot in lo-order
-    const int* cnt;             // strided: slots of S1[#lo <= p] | S2[#hi < p] << 16
-    int* left;                  // out: columns left to the dense kernels
-};
-int tree_qp_group(int n);       // instantiation (NJ = 4, 6, 8, 10) a zone of n residences runs in, -1: too large
-cudaError_t tree_qp_prepare();
-int tree_qp_chunk();            // columns per work chunk (all of one zone)
-cudaError_t launch_tree_qp(const QpParams& P, const TreeParams& TP, int group, const int2* chunks, int nchunks, int* queue, cudaStream_t stream);
-cudaError_t launch_tree_gate(const int* left, unsigned long long cond_round, cudaStream_t stream);
-
 // ---- tree_newton.cu: the operator QP of a large radial zone, one CTA per column, all linear algebra on the tree
 struct NewtonZone {             // one zone of the Newton path
     int feeder;                 // index of the zone in the solver
@@ -293,6 +273,19 @@ cudaError_t launch_pack_rows(const double* src, double* dst, const int64_t* hmap
                              cudaStream_t s);
 cudaError_t launch_hour_mask(const double* p_ev, const int64_t* hmap, int64_t H, int T, unsigned long long* out, cudaStream_t s);
 cudaError_t launch_to_time_major(const double* in, int n, int T, double* out, int64_t ld, cudaStream_t s);
+// Host: breadth-first numbering of a zone tree (nodes topological, parent -1 = substation), the layout of the
+// tree-Newton and network-check kernels.  Roots in index order, then level by level the children of every node in
+// index order, so the children of a node are contiguous in the next level; the residences of a node are listed by
+// ascending home index.
+struct BfsTree {
+    std::vector<int> order;           // [nodes] position -> node
+    std::vector<int> lvl;             // [levels + 1] first position of every level, then the node count
+    std::vector<int> parent;          // [nodes] position of the parent, -1: root
+    std::vector<int> child0, nchild;  // [nodes] position of the first child (0 without children), number of children
+    std::vector<int> res0, nres;      // [nodes] the node's residences: entries res0.. of res
+    std::vector<int> res;             // [residences] home indices grouped by node position
+};
+void bfs_tree(int n_nodes, const int* parent, int n_res, const int* res_node, BfsTree& B);
 
 // ---- network_check.cu
 constexpr int kNetMaxSteps = 32;                      // steps per CTA (G) at most

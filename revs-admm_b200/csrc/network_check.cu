@@ -200,58 +200,32 @@ __global__ void __launch_bounds__(kNetThreads) network_reduce_kernel(const NetPa
 
 void net_add_zone(NetHost& h, int n_nodes, const int* parent, const double* cumr, int n_res, const int* res_node,
                   int64_t home_row) {
-    const int n = n_nodes;
-    // children and residences of every node, ascending
-    std::vector<int> cofs(n + 1, 0), kids(n), rofs(n + 1, 0), homes(n_res);
-    for (int i = 0; i < n; ++i)
-        if (parent[i] >= 0) ++cofs[parent[i] + 1];
-    for (int j = 0; j < n_res; ++j) ++rofs[res_node[j] + 1];
-    for (int i = 0; i < n; ++i) { cofs[i + 1] += cofs[i]; rofs[i + 1] += rofs[i]; }
-    {
-        std::vector<int> fill(cofs.begin(), cofs.end() - 1);
-        for (int i = 0; i < n; ++i)
-            if (parent[i] >= 0) kids[fill[parent[i]]++] = i;
-        std::vector<int> rf(rofs.begin(), rofs.end() - 1);
-        for (int j = 0; j < n_res; ++j) homes[rf[res_node[j]]++] = j;
-    }
-    // breadth-first order: the roots, then level by level the children of each node in turn
-    std::vector<int> order, pos(n);
-    order.reserve(n);
+    BfsTree B;
+    bfs_tree(n_nodes, parent, n_res, res_node, B);
     NetZone z{};
     z.node0 = (int64_t)h.nodes.size();
     z.lvl0 = (int64_t)h.levels.size();
     z.res0 = (int64_t)h.res.size();
     z.home_row = home_row;
     z.out_row = h.total_nodes;
-    z.n_nodes = n;
-    for (int i = 0; i < n; ++i)
-        if (parent[i] < 0) order.push_back(i);
-    h.levels.push_back(0);
-    size_t lo = 0;
-    while (lo < order.size()) {
-        const size_t hi = order.size();
-        h.levels.push_back((int)hi);
-        for (size_t q = lo; q < hi; ++q)
-            for (int e = cofs[order[q]]; e < cofs[order[q] + 1]; ++e) order.push_back(kids[e]);
-        lo = hi;
-    }
-    z.depth = (int)(h.levels.size() - z.lvl0 - 1);
-    for (int q = 0; q < n; ++q) pos[order[q]] = q;
-    for (int q = 0; q < n; ++q) {
-        const int i = order[q], pa = parent[i];
+    z.n_nodes = n_nodes;
+    z.depth = (int)B.lvl.size() - 1;
+    h.levels.insert(h.levels.end(), B.lvl.begin(), B.lvl.end());
+    h.res.insert(h.res.end(), B.res.begin(), B.res.end());
+    for (int q = 0; q < n_nodes; ++q) {
+        const int i = B.order[q], pa = parent[i];
         NetNode nd{};
         nd.r = pa < 0 ? cumr[i] : cumr[i] - cumr[pa];
         nd.node = i;
-        nd.parent = pa < 0 ? -1 : pos[pa];
-        nd.nchild = cofs[i + 1] - cofs[i];
-        nd.child0 = nd.nchild ? pos[kids[cofs[i]]] : 0;
-        nd.res0 = (int)(h.res.size() - z.res0);
-        nd.nres = rofs[i + 1] - rofs[i];
-        for (int e = rofs[i]; e < rofs[i + 1]; ++e) h.res.push_back(homes[e]);
+        nd.parent = B.parent[q];
+        nd.child0 = B.child0[q];
+        nd.nchild = B.nchild[q];
+        nd.res0 = B.res0[q];
+        nd.nres = B.nres[q];
         h.nodes.push_back(nd);
     }
     h.zones.push_back(z);
-    h.total_nodes += n;
+    h.total_nodes += n_nodes;
 }
 
 void net_finish(NetHost& h, int T) {

@@ -73,10 +73,6 @@ struct Counters {
     int iter;        // ADMM iterations done (device-side loop; selects the ping-pong side of the schedules)
     int pad_;
     unsigned long long rounds_total;   // working-set rounds since revs_admm_begin
-    int tree_left;         // columns the tree kernels left to the dense kernels in the current utility solve ...
-    int tree_queue[4];     // ... and their work-queue heads (reset together)
-    int pad2_[3];
-    unsigned long long tree_left_total;
 };
 
 struct ZoneGroups {  // static: which warp-kernel instantiations the zone sizes of this solver need
@@ -137,7 +133,6 @@ struct revs_solver {
     int trace_iter = -1, trace_round = -1;     // REVS_DEBUG_TRACE="<admm iteration>,<round>": per-column timeline of that round
     std::string trace_file = "revs_trace.bin"; // ... written here (REVS_DEBUG_TRACE_FILE), [ncols][12] int64
     bool use_graph = true;                     // revs_solve_admm: whole loop from one captured graph, loops decided on the device
-    long long tree_left_total = 0;            // columns the tree kernels left to the dense kernels (host-driven loop, debug)
     double host_sync_ms = 0.0, cat_ms[16] = {0};   // host time waiting in round syncs / span sums per category (debug_host)
     // captured ADMM loop (capture_loop): rebuilt when a parameter baked into it changes
     cudaGraph_t loop_graph = nullptr;
@@ -146,17 +141,6 @@ struct revs_solver {
     int gk_iter_max = 0, gk_flags = -1;
     double* d_respart = nullptr;               // per-CTA partial residual sums of dual_update_kernel
     double* d_dsum = nullptr;                  // [Hp] per-home sums of (P_sch[k+1] - P_sch[k])^2, home_solve_kernel -> dual_update_kernel
-    // operator QP on the feeder tree (tree_qp.cu): static per-zone arrays, pools of Hp entries
-    bool use_tree = false, tree_on = false;    // opt-in (option "tree" / REVS_TREE=1, before the trees are set): see tree_qp.cu
-    std::vector<char> tree_ok;                 // per feeder: arrays built (revs_set_feeder_tree(s)), not overridden by a dense block
-    int *d_t_perm = nullptr, *d_t_iperm = nullptr, *d_t_nodeA = nullptr, *d_t_nodeB = nullptr, *d_t_cnt = nullptr;
-    double *d_t_c = nullptr, *d_t_d = nullptr, *d_t_e = nullptr, *d_t_wA = nullptr, *d_t_wB = nullptr;
-    int64_t* d_t_zoff = nullptr;               // offset of every zone in the strided pools (32 NJ entries per zone)
-    std::vector<int64_t> tree_zoff;
-    size_t tree_pool_n = 0, tree_sig = 0;
-    int n_dense_cols = 0;                      // columns of zones without tree arrays: the dense kernels always run for them
-    int2* d_tree_cols[4] = {nullptr, nullptr, nullptr, nullptr};  // chunks of columns by instantiation (NJ = 4, 6, 8, 10)
-    int n_tree_cols[4] = {0, 0, 0, 0};
     // all-reduce of the residual sums over the GPUs of the box (revs_comm_*): peer-mapped mailboxes
     PeerSlot* d_mailbox = nullptr;             // [2][kMaxPeers] on this device, exported by IPC handle
     PeerSlot* peer_box[kMaxPeers] = {};        // mailboxes of all ranks as mapped into this process (peer_box[rank] == d_mailbox)
@@ -344,189 +328,6 @@ int check_ready(const revs_solver* s) {
     return REVS_OK;
 }
 
-// Static arrays of the tree kernel for one zone (tree_qp.cu header; numpy restatement: tests/tree_arrays_ref.py).
-// parent / cumr: the zone's nodes in topological order (local indices, -1 = substation), res: node of every home.
-struct ZoneHost {
-    std::vector<int> perm, iperm, nodeA, nodeB, cnt, ordB_in_A;   // ordB_in_A[k]: rank in lo-order of the k-th node in hi-order
-    std::vector<double> c, d, e, wA, wB;
-};
-
-void build_zone_arrays(int n_nodes, const int* parent, const double* cumr, int n, const int* res, ZoneHost& Z) {
-    std::vector<int> depth(n_nodes, 0), first_child(n_nodes, -1), next_sib(n_nodes, -1), last_child(n_nodes, -1), roots;
-    for (int i = 0; i < n_nodes; ++i) {
-        const int p = parent[i];
-        if (p < 0) { roots.push_back(i); continue; }
-        depth[i] = depth[p] + 1;
-        if (first_child[p] < 0) first_child[p] = i; else next_sib[last_child[p]] = i;
-        last_child[p] = i;
-    }
-    std::vector<int> head(n_nodes, -1), nxt(n, -1), tail(n_nodes, -1);       // homes of a node, in home order
-    for (int h = 0; h < n; ++h) {
-        const int x = res[h];
-        if (head[x] < 0) head[x] = h; else nxt[tail[x]] = h;
-        tail[x] = h;
-    }
-    Z.perm.assign(n, 0); Z.iperm.assign(n, 0);
-    std::vector<int> leaf(n, 0), stack;
-    int cntp = 0;
-    for (int ri = (int)roots.size() - 1; ri >= 0; --ri) stack.push_back(roots[ri]);
-    while (!stack.empty()) {                         // depth-first preorder, children in index order
-        const int x = stack.back();
-        stack.pop_back();
-        for (int h = head[x]; h >= 0; h = nxt[h]) { Z.perm[cntp] = h; Z.iperm[h] = cntp; leaf[cntp] = x; ++cntp; }
-        const size_t at = stack.size();
-        for (int ch = first_child[x]; ch >= 0; ch = next_sib[ch]) stack.push_back(ch);
-        std::reverse(stack.begin() + at, stack.end());
-    }
-    const int m = n > 0 ? n - 1 : 0;
-    Z.c.assign(n, 0.0); Z.d.assign(n, 0.0); Z.e.assign(n, 0.0);
-    for (int p = 0; p < n; ++p) Z.d[p] = 2.0 * cumr[leaf[p]];
-    for (int p = 0; p < m; ++p) {
-        int a = leaf[p], b = leaf[p + 1];
-        while (a != b && a >= 0 && b >= 0) {
-            if (depth[a] > depth[b]) a = parent[a];
-            else if (depth[b] > depth[a]) b = parent[b];
-            else { a = parent[a]; b = parent[b]; }
-        }
-        Z.c[p] = (a >= 0 && a == b) ? 2.0 * cumr[a] : 0.0;
-    }
-    // Cartesian tree of c: previous strictly smaller, next smaller-or-equal
-    std::vector<int> prev_s(m, -1), next_se(m, m), st;
-    for (int q = 0; q < m; ++q) {
-        while (!st.empty() && Z.c[st.back()] >= Z.c[q]) { next_se[st.back()] = q; st.pop_back(); }
-        prev_s[q] = st.empty() ? -1 : st.back();
-        st.push_back(q);
-    }
-    std::vector<int> lo(m), hi(m), ord(m);
-    std::vector<double> w(m);
-    for (int q = 0; q < m; ++q) {
-        lo[q] = prev_s[q] + 1;
-        hi[q] = next_se[q] < m ? next_se[q] : n - 1;
-        const double pv = std::max(prev_s[q] >= 0 ? Z.c[prev_s[q]] : 0.0, next_se[q] < m ? Z.c[next_se[q]] : 0.0);
-        w[q] = Z.c[q] - pv;
-        ord[q] = q;
-    }
-    for (int p = 0; p < n; ++p) Z.e[p] = Z.d[p] - std::max(p > 0 ? Z.c[p - 1] : 0.0, p < m ? Z.c[p] : 0.0);
-    Z.nodeA.assign(n, 0); Z.nodeB.assign(n, 0); Z.cnt.assign(n, 0); Z.wA.assign(n, 0.0); Z.wB.assign(n, 0.0);
-    std::stable_sort(ord.begin(), ord.end(), [&](int a, int b) { return lo[a] < lo[b]; });
-    std::vector<int> rank_lo(m, 0);
-    for (int k = 0; k < m; ++k) { Z.nodeA[k] = lo[ord[k]] | (hi[ord[k]] << 16); Z.wA[k] = w[ord[k]]; rank_lo[ord[k]] = k; }
-    std::vector<int> clo(n + 1, 0), chi(n + 1, 0);
-    for (int q = 0; q < m; ++q) { clo[lo[q]]++; chi[hi[q] + 1]++; }      // #nodes with lo == p ; #nodes with hi == p - 1
-    for (int q = 0; q < m; ++q) ord[q] = q;
-    std::stable_sort(ord.begin(), ord.end(), [&](int a, int b) { return hi[a] < hi[b]; });
-    Z.ordB_in_A.assign(m, 0);
-    for (int k = 0; k < m; ++k) { Z.nodeB[k] = lo[ord[k]] | (hi[ord[k]] << 16); Z.wB[k] = w[ord[k]]; Z.ordB_in_A[k] = rank_lo[ord[k]]; }
-    int a = 0, b = 0;
-    for (int p = 0; p < n; ++p) {
-        a += clo[p];                                 // nodes with lo <= p
-        b += chi[p];                                 // nodes with hi <  p
-        Z.cnt[p] = a | (b << 16);
-    }
-}
-
-// The kernel's layout of one zone (tree_qp.cu:ZonePtr): 32 NJ entries per array, position p at slot(p), nodes and
-// counts as shared-memory slots.
-struct ZonePacked {
-    std::vector<int> perm, nodeA, permB, cnt;
-    std::vector<double> c, d, e, wA;
-};
-
-void pack_zone(const ZoneHost& Z, int n, int nj, ZonePacked& K) {
-    const int S = 32 * nj, zero = S;
-    auto slot = [&](int p) { return (p % nj) * 32 + p / nj; };
-    K.perm.assign(S, -1); K.nodeA.assign(S, zero | (zero << 16)); K.permB.assign(S, 0); K.cnt.assign(S, zero | (zero << 16));
-    K.c.assign(S, 0.0); K.d.assign(S, 0.0); K.e.assign(S, 0.0); K.wA.assign(S, 0.0);
-    for (int p = 0; p < S; ++p) K.permB[slot(p)] = slot(p);            // padded nodes: weight 0, map to themselves
-    const int m = n > 0 ? n - 1 : 0;
-    for (int p = 0; p < n; ++p) {
-        const int sp = slot(p);
-        K.perm[sp] = Z.perm[p];
-        K.c[sp] = p < m ? Z.c[p] : 0.0;
-        K.d[sp] = Z.d[p];
-        K.e[sp] = Z.e[p];
-        const int a = Z.cnt[p] & 0xffff, b = Z.cnt[p] >> 16;            // S1[a], S2[b]: sums of the first a / b node terms
-        K.cnt[sp] = (a ? slot(a - 1) : zero) | ((b ? slot(b - 1) : zero) << 16);
-    }
-    for (int k = 0; k < m; ++k) {
-        const int lo = Z.nodeA[k] & 0xffff, hi = Z.nodeA[k] >> 16;
-        K.nodeA[slot(k)] = slot(hi) | ((lo ? slot(lo - 1) : zero) << 16);
-        K.wA[slot(k)] = Z.wA[k];
-    }
-    for (int k = 0; k < m; ++k) K.permB[slot(k)] = slot(Z.ordB_in_A[k]);
-}
-
-int alloc_tree_pools(revs_solver* s) {
-    if (s->d_t_perm) return REVS_OK;
-    std::vector<int64_t> zoff((size_t)s->nf, 0);
-    int64_t tot = 0;
-    for (int f = 0; f < s->nf; ++f) {
-        zoff[f] = tot;
-        const int g = tree_qp_group(s->feeders[f].n);
-        if (g >= 0) tot += 32 * (4 + 2 * g);
-    }
-    s->tree_zoff = zoff;
-    const size_t n = (size_t)tot, hp = (size_t)s->Hp;
-    CU(dalloc(&s->d_t_zoff, (size_t)s->nf));
-    CU(cudaMemcpy(s->d_t_zoff, zoff.data(), sizeof(int64_t) * s->nf, cudaMemcpyHostToDevice));
-    CU(dalloc(&s->d_t_perm, n)); CU(dalloc(&s->d_t_iperm, hp)); CU(dalloc(&s->d_t_nodeA, n)); CU(dalloc(&s->d_t_nodeB, n));
-    CU(dalloc(&s->d_t_cnt, n)); CU(dalloc(&s->d_t_c, n)); CU(dalloc(&s->d_t_d, n)); CU(dalloc(&s->d_t_e, n)); CU(dalloc(&s->d_t_wA, n));
-    s->tree_pool_n = n;
-    return REVS_OK;
-}
-
-// upload the arrays of feeder f
-int upload_zone_arrays(revs_solver* s, int f, const ZoneHost& Z) {
-    const FeederDev& fd = s->feeders[f];
-    int rc = alloc_tree_pools(s);
-    if (rc) return rc;
-    const int g = tree_qp_group(fd.n);
-    if (fd.n == 0 || g < 0) return REVS_OK;
-    ZonePacked K;
-    pack_zone(Z, fd.n, 4 + 2 * g, K);
-    const size_t S = K.perm.size(), o = (size_t)s->tree_zoff[f];
-    CU(cudaMemcpy(s->d_t_perm + o, K.perm.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_nodeA + o, K.nodeA.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_nodeB + o, K.permB.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_cnt + o, K.cnt.data(), sizeof(int) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_c + o, K.c.data(), sizeof(double) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_d + o, K.d.data(), sizeof(double) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_e + o, K.e.data(), sizeof(double) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_wA + o, K.wA.data(), sizeof(double) * S, cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_t_iperm + fd.off, Z.iperm.data(), sizeof(int) * fd.n, cudaMemcpyHostToDevice));
-    return REVS_OK;
-}
-
-// column lists of the tree kernels: every (zone, hour) of the zones that have tree arrays, by instantiation
-int rebuild_tree_lists(revs_solver* s) {
-    std::vector<int2> cols[4];                     // chunks of columns of one zone: {zone, first hour | count << 16}
-    const int ch = tree_qp_chunk();
-    s->n_dense_cols = s->ncols;
-    for (int f = 0; f < s->nf; ++f) {
-        if (!s->tree_ok[f] || s->feeders[f].n == 0) continue;
-        const int g = tree_qp_group(s->feeders[f].n);
-        if (g < 0) continue;
-        for (int t = 0; t < s->T; t += ch) cols[g].push_back(make_int2(f, t | (std::min(ch, s->T - t) << 16)));
-        s->n_dense_cols -= s->T;
-    }
-    s->tree_on = false;
-    for (int g = 0; g < 4; ++g) {
-        if (s->d_tree_cols[g]) { cudaFree(s->d_tree_cols[g]); s->d_tree_cols[g] = nullptr; }
-        s->n_tree_cols[g] = (int)cols[g].size();
-        if (cols[g].empty()) continue;
-        CU(dalloc(&s->d_tree_cols[g], cols[g].size()));
-        CU(cudaMemcpy(s->d_tree_cols[g], cols[g].data(), sizeof(int2) * cols[g].size(), cudaMemcpyHostToDevice));
-        s->tree_on = true;
-    }
-    // the captured loop bakes the lists in: a new capture only when they changed
-    size_t sig = 1469598103934665603ull;
-    for (int g = 0; g < 4; ++g)
-        for (const int2& c : cols[g]) { sig = (sig ^ (size_t)(unsigned)c.x) * 1099511628211ull; sig = (sig ^ (size_t)(unsigned)c.y) * 1099511628211ull; }
-    if (sig != s->tree_sig && s->loop_exec) { cudaGraphExecDestroy(s->loop_exec); s->loop_exec = nullptr; }
-    s->tree_sig = sig;
-    return REVS_OK;
-}
-
 // Zone-size groups, contraction / screening tile tables and tensor maps over the zones that have a dense block
 // (everything but the tree-Newton zones).  Called by revs_create and again when option "newton_min_n" moves zones.
 int build_tables(revs_solver* s) {
@@ -702,7 +503,7 @@ int rebuild_newton(revs_solver* s) {
 }
 
 bool newton_active(const revs_solver* s) { return s->n_newton_cols > 0; }
-int dense_cols(const revs_solver* s) { return s->n_dense_cols - s->n_newton_cols; }   // columns only the dense kernels can solve
+int dense_cols(const revs_solver* s) { return s->ncols - s->n_newton_cols; }   // columns the dense kernels solve
 
 int launch_newton_stage(revs_solver* s, bool timed) {
     if (!newton_active(s)) return REVS_OK;
@@ -773,15 +574,6 @@ int launch_newton_stage(revs_solver* s, bool timed) {
     return REVS_OK;
 }
 
-TreeParams tree_params(revs_solver* s) {
-    TreeParams TP{};
-    TP.zoff = s->d_t_zoff;
-    TP.perm = s->d_t_perm; TP.iperm = s->d_t_iperm; TP.c = s->d_t_c; TP.d = s->d_t_d; TP.e = s->d_t_e;
-    TP.nodeA = s->d_t_nodeA; TP.wA = s->d_t_wA; TP.permB = s->d_t_nodeB; TP.cnt = s->d_t_cnt;
-    TP.left = &s->d_cnt->tree_left;
-    return TP;
-}
-
 QpParams qp_params(revs_solver* s) {
     QpParams Q{};
     Q.feeders = s->d_feeders;
@@ -848,24 +640,6 @@ int launch_init(revs_solver* s, QpParams Q, bool in_loop, bool timed) {
     Q.order = nullptr;
     TimedSpan* sp = timed ? span_begin(s, 6, s->sU) : nullptr;
     CU(launch_qp_init(Q, s->use_warp_kernel ? qp_warp_max_n() : 0, s->sU));
-    if (sp) span_end(sp, s->sU);
-    return REVS_OK;
-}
-
-// The tree kernels: every column of a zone that was given as a tree is solved here, from z alone; what they
-// cannot finish (more than 16 binding rows, a failed safeguard) stays for the working-set rounds of the dense kernels.
-bool tree_active(const revs_solver* s) { return s->use_tree && s->tree_on; }
-
-int launch_tree_stage(revs_solver* s, const QpParams& Q, bool timed) {
-    if (!tree_active(s)) return REVS_OK;
-    CU(cudaMemsetAsync(&s->d_cnt->tree_left, 0, 5 * sizeof(int), s->sU));
-    TreeParams TP = tree_params(s);
-    TimedSpan* sp = timed ? span_begin(s, 8, s->sU) : nullptr;
-    for (int g = 3; g >= 0; --g) {
-        if (s->n_tree_cols[g] == 0) continue;
-        CU(launch_tree_qp(Q, TP, g, s->d_tree_cols[g], s->n_tree_cols[g], &s->d_cnt->tree_queue[g], s->sU));
-        s->stats.kernel_launches++;
-    }
     if (sp) span_end(sp, s->sU);
     return REVS_OK;
 }
@@ -1019,24 +793,11 @@ int utility_solve(revs_solver* s, bool in_loop = false) {
     s->stats.kernel_launches++;
     if (newton_active(s)) {
         if ((rc = launch_newton_stage(s, true))) return rc;
-        if (dense_cols(s) == 0 && !tree_active(s)) {
+        if (dense_cols(s) == 0) {
             CU(cudaMemcpyAsync(s->h_cnt, s->d_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, s->sU));
             CU(cudaStreamSynchronize(s->sU));
             return check_device_flags(s);
         }
-    }
-    if (tree_active(s)) {
-        if ((rc = launch_tree_stage(s, Q, true))) return rc;
-        CU(cudaMemcpyAsync(s->h_cnt, s->d_cnt, sizeof(Counters), cudaMemcpyDeviceToHost, s->sU));
-        const double t0 = now_ms();
-        CU(cudaStreamSynchronize(s->sU));
-        s->host_sync_ms += now_ms() - t0;
-        if ((rc = check_device_flags(s))) return rc;
-        s->ws_bound = std::max(s->ws_bound, s->h_cnt->max_ws);
-        s->tree_left_total += s->h_cnt->tree_left;
-        if (s->debug)
-            fprintf(stderr, "[revs] admm %d tree stage: %d columns left to the dense kernels, max_ws %d\n", s->k, s->h_cnt->tree_left, s->h_cnt->max_ws);
-        if (s->h_cnt->tree_left == 0 && dense_cols(s) == 0) return REVS_OK;
     }
     bool use[kQpClasses];
     // first round: qp_init_kernel assigns classes on the device by the size of the stored working
@@ -1133,9 +894,8 @@ void free_all(revs_solver* s) {
                     s->d_pev, s->d_soc, s->d_has_ev, s->d_rating, s->d_capacity, s->d_initial, s->d_indconst,
                     s->d_start, s->d_end, s->d_nmin, s->d_nmax, s->d_zero_i, s->d_cost, s->d_zt, s->d_lamt,
                     s->d_gt, s->d_vt, s->d_wcount, s->d_widx, s->d_status, s->d_innerok, s->d_cls, s->d_order, s->d_order4, s->d_order_count, s->d_cnt, s->d_diff,
-                    s->d_cprob, s->d_ctiles, s->d_respart, s->d_dsum, s->d_t_perm, s->d_t_iperm, s->d_t_nodeA, s->d_t_nodeB, s->d_t_cnt,
-                    s->d_t_c, s->d_t_d, s->d_t_e, s->d_t_wA, s->d_t_wB, s->d_t_zoff, s->d_tree_cols[0], s->d_tree_cols[1], s->d_tree_cols[2],
-                    s->d_tree_cols[3], s->d_nt_zones, s->d_nt_lvl, s->d_nt_parent, s->d_nt_home, s->d_nt_hnode, s->d_nt_wsi, s->d_nt_child, s->d_nt_homes, s->d_nt_rho,
+                    s->d_cprob, s->d_ctiles, s->d_respart, s->d_dsum,
+                    s->d_nt_zones, s->d_nt_lvl, s->d_nt_parent, s->d_nt_home, s->d_nt_hnode, s->d_nt_wsi, s->d_nt_child, s->d_nt_homes, s->d_nt_rho,
                     s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2, s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists,
                     s->d_net_zone_cta, s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_P,
                     s->d_net_scale, s->d_net_volt, s->d_net_load};
@@ -1210,7 +970,6 @@ int revs_create(revs_solver** out, int device, int n_feeders, const int64_t* fee
     s->H = feeder_off[n_feeders];
     s->feeders.resize(n_feeders);
     s->sens_set.assign(n_feeders, 0);
-    s->tree_ok.assign(n_feeders, 0);
     s->trees.resize(n_feeders);
     s->is_newton.assign(n_feeders, 0);
     s->nt_host.resize(n_feeders);
@@ -1323,7 +1082,6 @@ int revs_create(revs_solver** out, int device, int n_feeders, const int64_t* fee
         s->debug = getenv("REVS_DEBUG") != nullptr;
         s->debug_host = getenv("REVS_DEBUG_HOST") != nullptr;
         if ((e = getenv("REVS_NO_GRAPH")) && atoi(e)) s->use_graph = false;
-        if ((e = getenv("REVS_TREE")) && atoi(e)) s->use_tree = true;
         if ((e = getenv("REVS_DEBUG_TRACE")) && sscanf(e, "%d,%d", &s->trace_iter, &s->trace_round) == 2) s->use_graph = false;
         if ((e = getenv("REVS_DEBUG_TRACE_FILE"))) s->trace_file = e;
         if (s->debug) s->use_graph = false;      // the per-round lines need the host-driven loop
@@ -1367,11 +1125,6 @@ int revs_set_sensitivity(revs_solver* s, int feeder, const double* R_res) {
                         (size_t)fd.n * sizeof(double), fd.n, cudaMemcpyHostToDevice));
     s->sens_set[feeder] = 1;
     s->rn2_valid = false;
-    if (s->tree_ok[feeder]) {            // a dense block replaces the tree: this zone runs in the dense kernels
-        s->tree_ok[feeder] = 0;
-        int rc = rebuild_tree_lists(s);
-        if (rc) return rc;
-    }
     return REVS_OK;
 }
 
@@ -1410,24 +1163,13 @@ int revs_set_feeder_tree(revs_solver* s, int feeder, int n_nodes, const int32_t*
     if (s->is_newton[feeder]) {
         newton_build_zone(n_nodes, parent, r, fd.n, res_node, s->nt_host[feeder]);
         s->sens_set[feeder] = 1;
-        s->tree_ok[feeder] = 0;
-        int rc = rebuild_newton(s);
-        return rc ? rc : rebuild_tree_lists(s);
+        return rebuild_newton(s);
     }
     CU(launch_sens_voltage(t.d_parent, t.d_cumr, nullptr, t.d_res_node, fd.n, fd.n, s->d_Rpool + fd.roff, fd.np, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->sens_set[feeder] = 1;
     s->rn2_valid = false;
-    if (s->use_tree && tree_qp_group(fd.n) >= 0) {
-        ZoneHost Z;
-        build_zone_arrays(n_nodes, parent, cumr.data(), fd.n, res_node, Z);
-        int rc = upload_zone_arrays(s, feeder, Z);
-        if (rc) return rc;
-        s->tree_ok[feeder] = 1;
-    } else {
-        s->tree_ok[feeder] = 0;
-    }
-    return rebuild_tree_lists(s);
+    return REVS_OK;
 }
 
 int revs_set_feeder_trees(revs_solver* s, const int64_t* node_off, const int32_t* parent, const double* r,
@@ -1506,55 +1248,12 @@ int revs_set_feeder_trees(revs_solver* s, const int64_t* node_off, const int32_t
     if (max_n > 0)
     CU(launch_sens_voltage_batched(s->d_feeders, s->nf, max_n, s->d_pool_off, s->d_pool_parent, s->d_pool_cumr,
                                    s->d_pool_res, s->d_Rpool, s->sU));
-    // static arrays of the tree kernels, all zones into host pools, one upload per array
-    for (int f = 0; f < s->nf; ++f) s->tree_ok[f] = 0;
-    if (s->use_tree) {
-        int rc = alloc_tree_pools(s);
-        if (rc) return rc;
-        const size_t np_ = s->tree_pool_n, hp = (size_t)s->Hp;
-        std::vector<int> perm(np_, -1), iperm(hp, 0), nodeA(np_, 0), permB(np_, 0), cnt(np_, 0);
-        std::vector<double> c(np_, 0.0), d(np_, 0.0), e(np_, 0.0), wA(np_, 0.0);
-        ZoneHost Z;
-        ZonePacked K;
-        for (int f = 0; f < s->nf; ++f) {
-            const FeederDev& fd = s->feeders[f];
-            s->tree_ok[f] = 0;
-            const int g = tree_qp_group(fd.n);
-            if (fd.n == 0 || g < 0 || s->is_newton[f]) continue;
-            const int64_t o = node_off[f];
-            build_zone_arrays((int)(node_off[f + 1] - o), parent + o, cumr.data() + o, fd.n, res_node + s->off[f], Z);
-            pack_zone(Z, fd.n, 4 + 2 * g, K);
-            const size_t zo = (size_t)s->tree_zoff[f];
-            std::copy(K.perm.begin(), K.perm.end(), perm.begin() + zo);
-            std::copy(K.nodeA.begin(), K.nodeA.end(), nodeA.begin() + zo);
-            std::copy(K.permB.begin(), K.permB.end(), permB.begin() + zo);
-            std::copy(K.cnt.begin(), K.cnt.end(), cnt.begin() + zo);
-            std::copy(K.c.begin(), K.c.end(), c.begin() + zo);
-            std::copy(K.d.begin(), K.d.end(), d.begin() + zo);
-            std::copy(K.e.begin(), K.e.end(), e.begin() + zo);
-            std::copy(K.wA.begin(), K.wA.end(), wA.begin() + zo);
-            std::copy(Z.iperm.begin(), Z.iperm.end(), iperm.begin() + fd.off);
-            s->tree_ok[f] = 1;
-        }
-        CU(cudaMemcpyAsync(s->d_t_perm, perm.data(), sizeof(int) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_iperm, iperm.data(), sizeof(int) * hp, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_nodeA, nodeA.data(), sizeof(int) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_nodeB, permB.data(), sizeof(int) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_cnt, cnt.data(), sizeof(int) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_c, c.data(), sizeof(double) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_d, d.data(), sizeof(double) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_e, e.data(), sizeof(double) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaMemcpyAsync(s->d_t_wA, wA.data(), sizeof(double) * np_, cudaMemcpyHostToDevice, s->sU));
-        CU(cudaStreamSynchronize(s->sU));     // the host staging vectors die here
-    }
     s->stats.kernel_launches++;
     s->rn2_valid = false;
-    const double th2 = now_ms();
-    const int rc_lists = rebuild_tree_lists(s);
     if (s->debug_host)
-        fprintf(stderr, "[revs host] set_feeder_trees: checks + cumulative resistances %.3f ms, copies + zone tables + sensitivity launch %.3f ms, lists %.3f ms\n",
-                th1 - th0, th2 - th1, now_ms() - th2);
-    return rc_lists;
+        fprintf(stderr, "[revs host] set_feeder_trees: checks + cumulative resistances %.3f ms, copies + zone tables + sensitivity launch %.3f ms\n",
+                th1 - th0, now_ms() - th1);
+    return REVS_OK;
 }
 
 int revs_set_homes(revs_solver* s, const double* load, const uint8_t* has_ev, const double* rating,
@@ -1767,15 +1466,16 @@ int admm_step_impl(revs_solver* s, double sums[3], bool sync_now) {
 //   while (k < iter_max && !converged && !error)            cudaGraphCondTypeWhile, condition set by the last CTA of dual_update_kernel
 //       home_solve            (own branch: uses the previous iterates, joins before dual_update)
 //       qp_init
+//       tree_newton           (zones of the tree-Newton path, if any)
 //       while (columns running)                             cudaGraphCondTypeWhile, condition set by round_end_kernel
-//           screening pass, work lists, QP classes side by side, round end
+//           screening pass, work lists, QP classes side by side, round end      (only when some zone has a dense block)
 //       dual_update           (k += 1)
 //
 // Every kernel reads what changes from iteration to iteration (ping-pong side of the schedules, row of diff,
 // round number) from device counters, so the bodies are captured once.  Nothing returns to the host until the
 // schedule is finished: no round trip per working-set round, no launch latency per kernel.
 int capture_loop(revs_solver* s) {
-    const int flags = (s->screen ? 1 : 0) | (s->screen_impl << 1) | (s->overlap_home ? 4 : 0) | (s->use_warp_kernel ? 8 : 0) | (s->use_fast ? 16 : 0) | (s->comm_world << 8) | (s->comm_rank << 16) | (tree_active(s) ? 32 : 0) | (dense_cols(s) ? 64 : 0) | (newton_active(s) ? 128 : 0);
+    const int flags = (s->screen ? 1 : 0) | (s->screen_impl << 1) | (s->overlap_home ? 4 : 0) | (s->use_warp_kernel ? 8 : 0) | (s->use_fast ? 16 : 0) | (s->comm_world << 8) | (s->comm_rank << 16) | (dense_cols(s) ? 64 : 0) | (newton_active(s) ? 128 : 0);
     if (s->loop_exec && s->gk_kappa == s->kappa && s->gk_vset == s->vset && s->gk_vhigh == s->vhigh && s->gk_tol == s->tol &&
         s->gk_iter_max == s->iter_max && s->gk_flags == flags)
         return REVS_OK;
@@ -1784,15 +1484,17 @@ int capture_loop(revs_solver* s) {
     // function attributes are set outside the capture
     for (int cl = 1; cl < kQpClasses; ++cl) CU(launch_utility_qp(QpParams{}, 0, cl, s->sU));
     CU(qp_warp_prepare());
-    CU(tree_qp_prepare());
     CU(screen_prepare());
     CU(screen_tc5_prepare());
     CU(cudaGraphCreate(&s->loop_graph, 0));
-    cudaGraphConditionalHandle h_loop, h_round;
-    CU(cudaGraphConditionalHandleCreate(&h_loop, s->loop_graph, 1, cudaGraphCondAssignDefault));
-    CU(cudaGraphConditionalHandleCreate(&h_round, s->loop_graph, 0, cudaGraphCondAssignDefault));
+    const bool rounds = dense_cols(s) > 0;         // the working-set loop of the dense kernels
+    cudaGraphConditionalHandle h_loop, h_round = 0;
     GateCapture gc{};
-    for (int cl = 2; cl < kQpClasses; ++cl) CU(cudaGraphConditionalHandleCreate(&gc.h[cl], s->loop_graph, 0, cudaGraphCondAssignDefault));
+    CU(cudaGraphConditionalHandleCreate(&h_loop, s->loop_graph, 1, cudaGraphCondAssignDefault));
+    if (rounds) {
+        CU(cudaGraphConditionalHandleCreate(&h_round, s->loop_graph, 0, cudaGraphCondAssignDefault));
+        for (int cl = 2; cl < kQpClasses; ++cl) CU(cudaGraphConditionalHandleCreate(&gc.h[cl], s->loop_graph, 0, cudaGraphCondAssignDefault));
+    }
     cudaGraphNodeParams np_loop{};
     np_loop.type = cudaGraphNodeTypeConditional;
     np_loop.conditional.handle = h_loop;
@@ -1820,8 +1522,10 @@ int capture_loop(revs_solver* s) {
         CU(launch_home_solve(hp, sHome));
         if (s->overlap_home) CU(cudaEventRecord(s->evHomeDone, s->sH));
         QpParams Q = qp_params(s);
-        Q.cond_round = (unsigned long long)h_round;
-        Q.use_cond = 1;
+        if (rounds) {                                // qp_init_kernel opens the working-set loop
+            Q.cond_round = (unsigned long long)h_round;
+            Q.use_cond = 1;
+        }
         int r = launch_init(s, Q, true, false);
         if (r) return r;
         if (newton_active(s)) {
@@ -1830,29 +1534,23 @@ int capture_loop(revs_solver* s) {
             s->stats = keep;
             if (r) return r;
         }
-        if (tree_active(s)) {
-            const revs_stats keep = s->stats;
-            r = launch_tree_stage(s, Q, false);
-            s->stats = keep;
-            if (r) return r;
+        if (rounds) {
+            // the working-set while node goes into the graph being captured, after what the stream has enqueued so far
+            cudaStreamCaptureStatus st;
+            cudaGraph_t g_cap = nullptr;
+            const cudaGraphNode_t* deps = nullptr;
+            size_t n_deps = 0;
+            CU(cudaStreamGetCaptureInfo(s->sU, &st, nullptr, &g_cap, &deps, &n_deps));
+            cudaGraphNodeParams np_round{};
+            np_round.type = cudaGraphNodeTypeConditional;
+            np_round.conditional.handle = h_round;
+            np_round.conditional.type = cudaGraphCondTypeWhile;
+            np_round.conditional.size = 1;
+            cudaGraphNode_t n_round;
+            CU(cudaGraphAddNode(&n_round, g_cap, deps, n_deps, &np_round));
+            body_round = np_round.conditional.phGraph_out[0];
+            CU(cudaStreamUpdateCaptureDependencies(s->sU, &n_round, 1, cudaStreamSetCaptureDependencies));
         }
-        if ((tree_active(s) || newton_active(s)) && dense_cols(s) == 0)     // the rounds of the dense kernels run only for what is left
-            CU(launch_tree_gate(&s->d_cnt->tree_left, (unsigned long long)h_round, s->sU));
-        // the working-set while node goes into the graph being captured, after what the stream has enqueued so far
-        cudaStreamCaptureStatus st;
-        cudaGraph_t g_cap = nullptr;
-        const cudaGraphNode_t* deps = nullptr;
-        size_t n_deps = 0;
-        CU(cudaStreamGetCaptureInfo(s->sU, &st, nullptr, &g_cap, &deps, &n_deps));
-        cudaGraphNodeParams np_round{};
-        np_round.type = cudaGraphNodeTypeConditional;
-        np_round.conditional.handle = h_round;
-        np_round.conditional.type = cudaGraphCondTypeWhile;
-        np_round.conditional.size = 1;
-        cudaGraphNode_t n_round;
-        CU(cudaGraphAddNode(&n_round, g_cap, deps, n_deps, &np_round));
-        body_round = np_round.conditional.phGraph_out[0];
-        CU(cudaStreamUpdateCaptureDependencies(s->sU, &n_round, 1, cudaStreamSetCaptureDependencies));
         if (s->overlap_home) CU(cudaStreamWaitEvent(s->sU, s->evHomeDone, 0));
         DualParams D = dual_params(s);
         D.iter = &s->d_cnt->iter;
@@ -1866,39 +1564,40 @@ int capture_loop(revs_solver* s) {
     cudaError_t ce = cudaStreamEndCapture(s->sU, &got);
     if (rc) return rc;
     if (ce != cudaSuccess) return fail(REVS_ERR_CUDA, "capture of the ADMM loop body failed: %s", cudaGetErrorString(ce));
-
-    // ---- body of the working-set loop
-    CU(cudaStreamBeginCaptureToGraph(s->sU, body_round, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-    auto capture_round = [&]() -> int {
-        QpParams Q = qp_params(s);
-        const revs_stats keep = s->stats;             // launch accounting of a captured run comes from the device counters
-        int r = enqueue_round(s, Q, -1, nullptr, nullptr, false, &gc);
-        s->stats = keep;
-        if (r) return r;
-        RoundEndParams E{};
-        E.n_running = &s->d_cnt->n_running;
-        E.n_failed = &s->d_cnt->n_failed;
-        E.infeasible = &s->d_cnt->infeasible;
-        E.round_ctr = &s->d_cnt->round;
-        E.noconv = &s->d_cnt->noconv;
-        E.rounds_total = &s->d_cnt->rounds_total;
-        E.round_max = kQpRoundMax;
-        E.cond_round = (unsigned long long)h_round;
-        E.use_cond = 1;
-        CU(launch_round_end(E, s->sU));
-        return REVS_OK;
-    };
-    rc = capture_round();
-    ce = cudaStreamEndCapture(s->sU, &got);
-    if (rc) return rc;
-    if (ce != cudaSuccess) return fail(REVS_ERR_CUDA, "capture of the working-set loop body failed: %s", cudaGetErrorString(ce));
-    for (int cl = 2; cl < kQpClasses; ++cl) {          // bodies of the class gates: the CTA kernel of that class
-        CU(cudaStreamBeginCaptureToGraph(s->sQ[cl], gc.body[cl], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
-        QpParams Q = qp_params(s);
-        cudaError_t le = launch_utility_qp(Q, s->ncols, cl, s->sQ[cl]);
-        ce = cudaStreamEndCapture(s->sQ[cl], &got);
-        if (le != cudaSuccess || ce != cudaSuccess)
-            return fail(REVS_ERR_CUDA, "capture of QP class %d failed: %s", cl, cudaGetErrorString(le != cudaSuccess ? le : ce));
+    if (rounds) {
+        // ---- body of the working-set loop
+        CU(cudaStreamBeginCaptureToGraph(s->sU, body_round, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+        auto capture_round = [&]() -> int {
+            QpParams Q = qp_params(s);
+            const revs_stats keep = s->stats;             // launch accounting of a captured run comes from the device counters
+            int r = enqueue_round(s, Q, -1, nullptr, nullptr, false, &gc);
+            s->stats = keep;
+            if (r) return r;
+            RoundEndParams E{};
+            E.n_running = &s->d_cnt->n_running;
+            E.n_failed = &s->d_cnt->n_failed;
+            E.infeasible = &s->d_cnt->infeasible;
+            E.round_ctr = &s->d_cnt->round;
+            E.noconv = &s->d_cnt->noconv;
+            E.rounds_total = &s->d_cnt->rounds_total;
+            E.round_max = kQpRoundMax;
+            E.cond_round = (unsigned long long)h_round;
+            E.use_cond = 1;
+            CU(launch_round_end(E, s->sU));
+            return REVS_OK;
+        };
+        rc = capture_round();
+        ce = cudaStreamEndCapture(s->sU, &got);
+        if (rc) return rc;
+        if (ce != cudaSuccess) return fail(REVS_ERR_CUDA, "capture of the working-set loop body failed: %s", cudaGetErrorString(ce));
+        for (int cl = 2; cl < kQpClasses; ++cl) {          // bodies of the class gates: the CTA kernel of that class
+            CU(cudaStreamBeginCaptureToGraph(s->sQ[cl], gc.body[cl], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+            QpParams Q = qp_params(s);
+            cudaError_t le = launch_utility_qp(Q, s->ncols, cl, s->sQ[cl]);
+            ce = cudaStreamEndCapture(s->sQ[cl], &got);
+            if (le != cudaSuccess || ce != cudaSuccess)
+                return fail(REVS_ERR_CUDA, "capture of QP class %d failed: %s", cl, cudaGetErrorString(le != cudaSuccess ? le : ce));
+        }
     }
     CU(cudaGraphInstantiate(&s->loop_exec, s->loop_graph, 0));
     s->gk_kappa = s->kappa; s->gk_vset = s->vset; s->gk_vhigh = s->vhigh; s->gk_tol = s->tol;
@@ -1935,12 +1634,8 @@ int revs_solve_admm(revs_solver* s, double kappa, int iter_max, double vset, dou
         s->stats.gemm_launches = (int64_t)s->h_cnt->rounds_total;
         s->stats.gemm_full_launches = s->k;
         s->stats.qp_warp_rounds = (s->use_warp_kernel && s->zg.warp_n > 0) ? (int64_t)s->h_cnt->rounds_total : 0;
-        int tree_launches = 0;
-        if (tree_active(s))
-            for (int g = 0; g < 4; ++g) tree_launches += s->n_tree_cols[g] > 0;
-        if (newton_active(s)) ++tree_launches;
-        if (tree_launches && dense_cols(s) == 0) ++tree_launches;              // + the gate of the working-set loop
-        s->stats.kernel_launches += (int64_t)s->k * (3 + tree_launches) + (int64_t)s->h_cnt->rounds_total * round_launches(s);
+        // per iteration: home solve, qp_init, tree-Newton, dual update; per working-set round: round_launches
+        s->stats.kernel_launches += (int64_t)s->k * (newton_active(s) ? 4 : 3) + (int64_t)s->h_cnt->rounds_total * round_launches(s);
         if (rc) return rc;
     } else {
         for (int k = 0; k < iter_max; ++k) {
@@ -2569,26 +2264,6 @@ int revs_screen_contract(int device, int M, int K, int T, const double* A, const
     return REVS_OK;
 }
 
-int revs_zone_arrays(int n_nodes, const int32_t* parent, const double* r, int n_res, const int32_t* res_node, int32_t* perm,
-                     double* c, double* d, double* e, int32_t* node_lo, double* w_lo, int32_t* node_hi, double* w_hi, int32_t* cnt) {
-    if (n_nodes <= 0 || n_res <= 0 || !parent || !r || !res_node || !perm || !c || !d || !e || !node_lo || !w_lo || !node_hi || !w_hi || !cnt)
-        return fail(REVS_ERR_ARG, "bad arguments");
-    std::vector<double> cumr(n_nodes);
-    for (int i = 0; i < n_nodes; ++i) {
-        if (parent[i] >= i || parent[i] < -1) return fail(REVS_ERR_ARG, "nodes must be topologically ordered (parent[i] < i)");
-        cumr[i] = (parent[i] < 0 ? 0.0 : cumr[parent[i]]) + r[i];
-    }
-    for (int j = 0; j < n_res; ++j)
-        if (res_node[j] < 0 || res_node[j] >= n_nodes) return fail(REVS_ERR_ARG, "res_node[%d] out of range", j);
-    ZoneHost Z;
-    build_zone_arrays(n_nodes, parent, cumr.data(), n_res, res_node, Z);
-    for (int p = 0; p < n_res; ++p) {
-        perm[p] = Z.perm[p]; c[p] = Z.c[p]; d[p] = Z.d[p]; e[p] = Z.e[p];
-        node_lo[p] = Z.nodeA[p]; w_lo[p] = Z.wA[p]; node_hi[p] = Z.nodeB[p]; w_hi[p] = Z.wB[p]; cnt[p] = Z.cnt[p];
-    }
-    return REVS_OK;
-}
-
 int revs_comm_export(revs_solver* s, void* handle64) {
     if (!s || !handle64) return fail(REVS_ERR_ARG, "bad arguments");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
@@ -2648,16 +2323,6 @@ int revs_set_option(revs_solver* s, const char* name, double value) {
         if (value != 0.0 && s->zg.max_n > 16384) return fail(REVS_ERR_ARG, "screening is limited to zones of at most 16384 residences");
         if (mid_run) return fail(REVS_ERR_ARG, "'screen' cannot change between revs_admm_step calls of one run");
         s->screen = value != 0.0;
-        return REVS_OK;
-    }
-    if (!strcmp(name, "tree")) {
-        // 1: zones given as trees (<= 320 residences) are solved by the tree-structured kernel, which needs no sensitivity
-        // matrix (tree_qp.cu); the static arrays are built by revs_set_feeder_tree(s), so set the option before them
-        if (mid_run) return fail(REVS_ERR_ARG, "'tree' cannot change between revs_admm_step calls of one run");
-        if (value != 0.0 && !s->use_tree)
-            for (int f = 0; f < s->nf; ++f)
-                if (s->sens_set[f]) return fail(REVS_ERR_ARG, "set option 'tree' before revs_set_feeder_tree(s): the tree arrays are built there");
-        s->use_tree = value != 0.0;
         return REVS_OK;
     }
     if (!strcmp(name, "newton_min_n")) {

@@ -648,37 +648,22 @@ void newton_build_zone(int n_nodes, const int* parent, const double* r, int n_re
         if (!tiny) { nw0[k] = (int)par.size(); par.push_back(parent[k] >= 0 ? nw0[rep[parent[k]]] : -1); rr.push_back(r[k]); }
     }
     const int n = (int)par.size();
-    std::vector<int> depth(n, 0);
-    int maxd = 0;
-    for (int k = 0; k < n; ++k) { depth[k] = par[k] >= 0 ? depth[par[k]] + 1 : 0; maxd = std::max(maxd, depth[k]); }
-    // level by level, each level ordered by the new index of the parent (children of a node contiguous)
-    std::vector<std::vector<int>> lv(maxd + 1);
-    for (int k = 0; k < n; ++k) lv[depth[k]].push_back(k);
-    std::vector<int> nw(n, -1), order;
-    order.reserve(n);
-    Z.lvl.assign(1, 0);
-    for (int d = 0; d <= maxd; ++d) {
-        if (d > 0) std::stable_sort(lv[d].begin(), lv[d].end(), [&](int a, int b) { return nw[par[a]] < nw[par[b]]; });
-        for (int k : lv[d]) { nw[k] = (int)order.size(); order.push_back(k); }
-        Z.lvl.push_back((int)order.size());
-    }
-    Z.parent.assign(n, -1); Z.rho.assign(n, 0.0);
-    Z.child0.assign(n, 0); Z.nchild.assign(n, 0); Z.home0.assign(n, 0); Z.nhome.assign(n, 0);
-    for (int i = 0; i < n; ++i) {
-        const int k = order[i];
-        Z.parent[i] = par[k] >= 0 ? nw[par[k]] : -1;
-        Z.rho[i] = 2.0 * rr[k];
-    }
-    for (int i = n - 1; i >= 0; --i)
-        if (Z.parent[i] >= 0) { Z.child0[Z.parent[i]] = i; Z.nchild[Z.parent[i]]++; }
-    std::vector<int> node_of(n_res);
-    for (int h = 0; h < n_res; ++h) { node_of[h] = nw[nw0[rep[res_node[h]]]]; Z.nhome[node_of[h]]++; }
-    int run = 0;
-    for (int i = 0; i < n; ++i) { Z.home0[i] = run; run += Z.nhome[i]; }
-    Z.hlist.assign(n_res, 0);
-    Z.hnode.assign(n_res, 0);
-    std::vector<int> fill(n, 0);
-    for (int h = 0; h < n_res; ++h) { const int k = node_of[h]; const int j = Z.home0[k] + fill[k]++; Z.hlist[j] = h; Z.hnode[j] = k; }
+    std::vector<int> cres(n_res);
+    for (int h = 0; h < n_res; ++h) cres[h] = nw0[rep[res_node[h]]];
+    BfsTree B;
+    bfs_tree(n, par.data(), n_res, cres.data(), B);
+    Z.lvl = std::move(B.lvl);
+    Z.parent = std::move(B.parent);
+    Z.child0 = std::move(B.child0);
+    Z.nchild = std::move(B.nchild);
+    Z.home0 = std::move(B.res0);
+    Z.nhome = std::move(B.nres);
+    Z.hlist = std::move(B.res);
+    Z.rho.resize(n);
+    for (int i = 0; i < n; ++i) Z.rho[i] = 2.0 * rr[B.order[i]];
+    Z.hnode.resize(n_res);
+    for (int i = 0; i < n; ++i)
+        for (int j = Z.home0[i]; j < Z.home0[i] + Z.nhome[i]; ++j) Z.hnode[j] = i;
     // scale of the shifts: mean over the residences of (row sum of R)^2 / n (a lower bound of the squared row norm)
     std::vector<double> acc(n, 0.0), mu(n, 0.0);
     for (int i = 0; i < n; ++i) acc[i] = (double)Z.nhome[i];

@@ -234,9 +234,8 @@ def test_pipelined_solver_equals_single_solver(gpu_lib, pipelines):
         assert np.array_equal(base[k], out[k]), k
 
 
-@pytest.mark.parametrize("tree", [1, 0])
 @pytest.mark.parametrize("sizes,T,vhigh", [([140, 60, 33], 48, 1.015), ([300, 210], 24, 1.02), ([600, 90], 24, 1.05), ([120, 96], 12, 1.02)])
-def test_captured_loop_equals_host_driven_loop(gpu_lib, sizes, T, vhigh, tree):
+def test_captured_loop_equals_host_driven_loop(gpu_lib, sizes, T, vhigh):
     """revs_solve_admm from ONE captured graph (ADMM iterations and working-set rounds decided on the
     device, CTA classes behind IF nodes) against the host-driven loop (one host sync per round):
     bit-identical results, same number of working-set rounds -- including zones that need several rounds
@@ -251,7 +250,6 @@ def test_captured_loop_equals_host_driven_loop(gpu_lib, sizes, T, vhigh, tree):
     for graph in (1, 0):
         with gpu_lib.Solver(sizes, T) as s:
             s.set_option("graph", graph)
-            s.set_option("tree", tree)
             s.set_option("newton_min_n", 4096)            # zones above 512 on the dense kernels (tree-Newton: test_gpu_newton.py)
             s.set_feeder_trees(trees)
             s.set_homes(**hm)
@@ -267,8 +265,7 @@ def test_captured_loop_equals_host_driven_loop(gpu_lib, sizes, T, vhigh, tree):
     for k in ("P_sch", "P_ev", "SOC", "diff", "P_est", "Gamma"):
         assert np.array_equal(outs[0][k], outs[1][k]), k
     assert rounds[0] == rounds[1]
-    if tree == 0 or max(sizes) > 320:                # the dense kernels run at least one working-set round per iteration
-        assert rounds[0] >= kw["iter_max"]
+    assert rounds[0] >= kw["iter_max"]               # the dense kernels run at least one working-set round per iteration
 
 
 @pytest.mark.parametrize("sizes,T", [([70, 45, 33], 96), ([40, 21], 24), ([30], 100), ([12], 256)])
@@ -405,37 +402,22 @@ def test_compact_schedule_download_equals_full_results(gpu_lib):
 
 
 @pytest.mark.parametrize("sizes,T,vhigh", [([140, 60, 33], 48, 1.015), ([297, 157, 257, 320, 129], 24, 1.02), ([120, 96], 12, 1.02), ([1, 2, 31, 33], 24, 1.01)])
-def test_tree_kernel_equals_dense_kernels(gpu_lib, sizes, T, vhigh):
-    """The tree-structured operator kernel (no sensitivity matrix: rows and products from the feeder tree) against
-    the dense kernels (BF16 screening + FP64 rows of R) and the oracle: identical charging hours, estimates within
-    1e-7 kW of each other, the tree path never launching a screening contraction unless it leaves columns behind."""
+def test_warp_zone_sizes_match_oracle(gpu_lib, sizes, T, vhigh):
+    """The dense kernels (BF16 screening + FP64 rows of R) on zones on both sides of every size-class boundary of the
+    warp kernels (128 / 129, 256 / 257, 320) against the oracle: identical charging hours, estimates within 1e-6 kW,
+    binding working sets of two rows or more."""
     trees, hm, cost = _problem(sizes, T, seed=13 + sum(sizes), r_secondary=2e-3 if T == 12 else 1e-3,
                                **(dict(adoption=1.0) if T == 12 else {}))
     if T == 12:
         hm["start"][:] = 0
         hm["end"][:] = T
     kw = dict(kappa=5.0, iter_max=6, vset=1.0, vlow=0.95, vhigh=vhigh)
-    outs = []
-    for tree in (1, 0):
-        with gpu_lib.Solver(sizes, T) as s:
-            s.set_option("tree", tree)               # before the trees: the tree arrays are built by set_feeder_trees
-            s.set_feeder_trees(trees)
-            s.set_homes(**hm)
-            s.set_tariff(cost)
-            done = s.solve_admm(**kw)
-            out = s.results(done)
-            out["P_est"], out["Gamma"] = s.estimate()
-            out["stats"] = s.stats()
-            outs.append(out)
+    out = _gpu(gpu_lib, sizes, T, trees, hm, cost, kw)
     ref = _oracle(trees, hm, cost, kw)
-    for out in outs:
-        assert np.array_equal(out["P_ev"], ref["P_ev"])
-        assert np.abs(out["P_est"] - ref["P_est"]).max() <= 1e-6
-        assert np.abs(out["diff"] - ref["diff"]).max() <= 1e-7
-    assert np.abs(outs[0]["P_est"] - outs[1]["P_est"]).max() <= 1e-7
-    assert outs[0]["stats"]["max_working_set"] >= 2
-    if T != 12:                                      # (T = 12: working sets beyond 16 rows go on to the dense kernels)
-        assert outs[0]["stats"]["gemm_launches"] < outs[1]["stats"]["gemm_launches"]
+    assert np.array_equal(out["P_ev"], ref["P_ev"])
+    assert np.abs(out["P_est"] - ref["P_est"]).max() <= 1e-6
+    assert np.abs(out["diff"] - ref["diff"]).max() <= 1e-7
+    assert out["stats"]["max_working_set"] >= 2
 
 
 def test_sharded_reliability_on_one_rank_equals_plain_check(gpu_lib):

@@ -212,50 +212,6 @@ def test_pipelined_stats_combination():
     ps.pool = None
 
 
-@pytest.mark.parametrize("kind", ["refshape", "laterals", "unsplit", "chain", "star"])
-def test_zone_tree_arrays_reproduce_the_dense_block(kind):
-    """The tree-structured operator kernel replaces the dense block R_res of lpsolver.py:183-189 by O(n) arrays
-    (revs_zone_arrays, host code of the library).  Checked here against the dense matrix without any GPU:
-    rows (min of c between the positions), the three-prefix-sum product, and the numpy restatement."""
-    import tree_arrays_ref as TA
-    from revs_admm_b200._cabi import zone_arrays
-    from revs_admm_b200.feeder import FeederTree, reference_shaped_feeder, split_zones, synthetic_feeder
-    rng = np.random.default_rng(5)
-    if kind == "refshape":
-        zones = [z for z, _ in split_zones(reference_shaped_feeder(700, seed=3))]
-    elif kind == "laterals":
-        zones = [z for z, _ in split_zones(synthetic_feeder(300, seed=1))]
-    elif kind == "unsplit":
-        zones = [synthetic_feeder(150, seed=2)]                      # several roots: blocks of zeros in R
-    elif kind == "chain":                                            # every residence hangs behind the previous one
-        n = 40
-        zones = [FeederTree(parent=np.arange(-1, n - 1, dtype=np.int32), r=rng.uniform(1e-4, 1e-3, n), res_node=np.arange(n, dtype=np.int32))]
-    else:                                                            # star with equal resistances: ties in c, two homes on one node
-        n = 30
-        res = np.r_[np.arange(1, n + 1), [3, 3]].astype(np.int32)
-        zones = [FeederTree(parent=np.r_[-1, np.zeros(n, dtype=np.int32)].astype(np.int32), r=np.full(n + 1, 2e-4), res_node=res)]
-    for z in zones:
-        R = z.rmat()[np.ix_(z.res_node, z.res_node)]
-        za = zone_arrays(z.parent, z.r, z.res_node)
-        ref = TA.zone_arrays(z.parent, z.r, z.res_node)
-        P = za["perm"]
-        assert sorted(P.tolist()) == list(range(z.n_res))
-        Rd = R[np.ix_(P, P)]
-        n = z.n_res
-        for i in rng.integers(0, n, 6):                              # rows
-            row = np.array([za["d"][i] if j == i else za["c"][min(i, j):max(i, j)].min() for j in range(n)])
-            assert np.array_equal(row, Rd[i])
-        assert (za["w"] >= 0).all() and (za["e"] >= -1e-18).all()
-        g = rng.uniform(0, 5, n)
-        G = np.concatenate([[0.0], np.cumsum(g)])
-        S1 = np.concatenate([[0.0], np.cumsum(za["w"] * (G[za["hi"] + 1] - G[za["lo"]]))])
-        S2 = np.concatenate([[0.0], np.cumsum(za["w_b"] * (G[za["hi_b"] + 1] - G[za["lo_b"]]))])
-        v = za["e"] * g + S1[za["cnt_lo"]] - S2[za["cnt_hi"]]
-        assert np.abs(v - Rd @ g).max() <= 1e-13 * max(1.0, np.abs(Rd @ g).max())
-        assert np.array_equal(ref["perm"], P) and np.array_equal(ref["c"], za["c"]) and np.array_equal(ref["d"], za["d"])
-        assert np.abs(TA.product(ref, g) - v).max() <= 1e-14
-
-
 def test_pack_trees_concatenates_the_zone_arrays():
     """Solver.pack_trees (the interpreter-side half of revs_set_feeder_trees, done pipeline by pipeline in
     PipelinedSolver.schedule): node offsets, parents, resistances and residence nodes of all zones back to back, in the
