@@ -22,6 +22,7 @@
  *   revs_reliability                              drawing.py:29-78    compute_flows(),
  *                                                                     compute_voltage()
  *   revs_network_check                            drawing.py:29-78    the same for every zone at once
+ *   revs_repair_schedule                          no reference counterpart (a voltage-feasible binary schedule)
  *   revs_get_results / revs_get_schedule(_ld)     lpsolver.py:289-290 return diff,P_sch,S,C
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
@@ -171,14 +172,15 @@ int revs_reliability(revs_solver* s, int feeder, int kind, int n_rows, const int
  * tree (leaves -> root: flows F, root -> leaves: squared-voltage drops D = R P), O(nodes x T), no sensitivity
  * matrix; every zone needs its tree (revs_set_feeder_tree(s)).
  * source: REVS_NET_SCHEDULE / REVS_NET_ESTIMATE (schedule / operator estimate of the last ADMM run, already on the
- * device, P ignored) or REVS_NET_HOST (P [H,T] from the host, compact home order of revs_create).
+ * device, P ignored), REVS_NET_HOST (P [H,T] from the host, compact home order of revs_create) or REVS_NET_REPAIRED
+ * (the repaired schedule of revs_repair_schedule, below).
  * "Total nodes" are the nodes of all zones concatenated in zone order (node_off of revs_set_feeder_trees); rows of
  * voltage / loading, and scale, follow it.  voltage = sqrt(vset^2 - D) (REVS_REL_VOLTAGE), loading = scale * F
  * (REVS_REL_FLOW, scale = signed 1/rating per edge, NULL = 1).  voltage, loading, zone_worst and summary may be NULL.
  * Ties of every maximum go to the lowest (zone, node or residence, step); counts are exact: two calls give the same
  * bytes, and the result of a zone does not depend on the other zones of the solver.
  * REVS_ERR_ARG: a zone without tree (the message names it), SCHEDULE / ESTIMATE before any ADMM iteration, HOST
- * without P, an unknown source, or not vlow <= vset < vhigh.  Synchronous on the utility stream; adds its launches to
+ * without P, REPAIRED before a repair of the current ADMM run, an unknown source, or not vlow <= vset < vhigh.  Synchronous on the utility stream; adds its launches to
  * revs_stats.kernel_launches and changes no other state.  The breadth-first arrays it needs are built on its first
  * call after the trees are set, its scratch on first use; both are kept until revs_destroy. */
 #define REVS_NET_SCHEDULE 0   /* P_sch of the last ADMM run (what revs_get_results returns)      */
@@ -207,6 +209,33 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
                        double* loading,            /* [total nodes, T] or NULL                                  */
                        double* zone_worst,         /* [n_feeders, 3]: drop_max, row_excess_max, loading_max     */
                        revs_network_summary* summary);
+
+/* Greedy voltage repair of the last ADMM run's charging decisions (see the header comment for the rule).
+ * P_out [H,T] (compact home order) and hour_mask [H, mask_words] may be NULL; zone_info [n_feeders, 3] int32 =
+ * {status 0/1/2, hours moved, hours dropped}, may be NULL.  The repaired schedule stays on the device for
+ * revs_network_check(REVS_NET_REPAIRED) until the next ADMM run.
+ *
+ * The rule, zone by zone (R is block-diagonal over zones), with D = R P at the residences, u = vhigh^2 - vset^2 and a
+ * row (i, t) violated when D[i,t] - u > row_tol:
+ *   1. take the worst violated row (i*, t*) of the steps not marked stuck: largest excess, then lowest residence, then
+ *      lowest step (the order of revs_network_check); stop when there is none;
+ *   2. the candidates are the homes charging at t*, by relief rating_h R[i*,h] descending, ties to the lowest home;
+ *   3. the first candidate charging more than n_min hours (the SOC target) drops hour t*; one at n_min moves it to the
+ *      cheapest hour of its plug-in window it does not charge at and that stays feasible (ties: earliest hour);
+ *   4. when no candidate can drop or move, t* is marked stuck.
+ * Charges only leave violated steps and only enter steps that stay feasible: no feasible step becomes violated, no
+ * row's excess grows past max(its input excess, row_tol), every home keeps its SOC window and plug-in window, and the
+ * loop ends after at most as many drops and moves as there were charges at violated steps.  Homes whose hours did not
+ * change keep their P_sch bytes; changed ones get P = load + (charging ? rating : 0).
+ * The rule is a heuristic: it does not look for the cheapest feasible schedule.  Zone status: 0 = no violated row,
+ * untouched; 1 = repaired, no violated row left; 2 = violated rows left (e.g. the base load alone violates a row).
+ * Needs the tree of every zone (revs_set_feeder_tree(s)).  REVS_ERR_ARG: a zone without tree (named), no ADMM
+ * iteration, mask_words != ceil(T/64) with hour_mask, not vset < vhigh, row_tol < 0 or NaN.  Synchronous on the
+ * utility stream; adds its launches to revs_stats.kernel_launches and changes no other state (P_sch, P_ev, P_est,
+ * Gamma, diff stay as they are). */
+int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_tol,
+                         double* P_out, uint64_t* hour_mask, int mask_words, int32_t* zone_info);
+#define REVS_NET_REPAIRED 3   /* the schedule of the last revs_repair_schedule of the current ADMM run  */
 
 /* The same check with the ROWS PARTITIONED over the GPUs of one box (one process per GPU, every process holds the
  * feeder's tree; BASELINE north_star: "the sensitivity contraction is row-partitioned"): every rank builds and

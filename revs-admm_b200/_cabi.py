@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("REVS_LIB") or os.path.join(HERE, "librevs_admm.so")     # REVS_LIB: a build variant (profiles/build_variants.sh)
 
 REVS_REL_VOLTAGE, REVS_REL_FLOW, REVS_REL_DROP = 0, 1, 2
-REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST = 0, 1, 2
+REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED = 0, 1, 2, 3
 
 
 class RevsError(RuntimeError):
@@ -89,6 +89,8 @@ SIGNATURES = {
     "revs_reliability_sharded": ([_P, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32), _D, C.c_double, _D, _D], C.c_int),
     "revs_network_check": ([_P, C.c_int, _D, C.c_double, C.c_double, C.c_double, C.c_double, _D, _D, _D, _D,
                             C.POINTER(NetworkSummary)], C.c_int),
+    "revs_repair_schedule": ([_P, C.c_double, C.c_double, C.c_double, _D, C.POINTER(C.c_uint64), C.c_int,
+                              C.POINTER(C.c_int32)], C.c_int),
 }
 
 _lib = None
@@ -170,6 +172,14 @@ def expand_schedule(mask, T, has_ev, rating, capacity, initial):
     for k in range(T):
         soc[:, k + 1] = soc[:, k] + inc[:, k]
     return p_ev, soc
+
+
+def repair_totals(r):
+    """Add the totals of zone_info to a repair_schedule result."""
+    z = r["zone_info"]
+    r.update(moves=int(z[:, 1].sum()), drops=int(z[:, 2].sum()), zones_violated=int((z[:, 0] > 0).sum()),
+             zones_repaired=int((z[:, 0] == 1).sum()), zones_left=int((z[:, 0] == 2).sum()))
+    return r
 
 
 class Solver:
@@ -354,17 +364,17 @@ class Solver:
     def network_check(self, source="schedule", vset=1.0, vlow=0.95, vhigh=1.05, row_tol=1e-9, scale=None, full=False,
                       zones=False, out=None):
         """Voltages and line loadings of every node of every zone, per step, in one call (include/revs_admm.h:
-        revs_network_check).  source: "schedule" (P_sch of the last ADMM run), "estimate" (P_est) or a host schedule
-        P [H, T].  scale: [total_nodes] signed 1/rating per edge (None = 1).  Returns dict(summary=dict,
+        revs_network_check).  source: "schedule" (P_sch of the last ADMM run), "estimate" (P_est), "repaired" (the
+        schedule of the last repair_schedule of that run) or a host schedule P [H, T].  scale: [total_nodes] signed 1/rating per edge (None = 1).  Returns dict(summary=dict,
         voltage=[total_nodes, T], loading=[total_nodes, T], zone_worst=[zones, 3]); the arrays are None unless
         asked for with full / zones.  out: optional dict of C-contiguous float64 [total_nodes, T] arrays voltage
         and loading to write into."""
         N, T = self.total_nodes, self.T
         Pp = None
         if isinstance(source, str):
-            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE}.get(source)
+            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE, "repaired": REVS_NET_REPAIRED}.get(source)
             if src is None:
-                raise ValueError(f"source must be 'schedule', 'estimate' or an [H, T] array, not {source!r}")
+                raise ValueError(f"source must be 'schedule', 'estimate', 'repaired' or an [H, T] array, not {source!r}")
         else:
             src, Pp = REVS_NET_HOST, _f64(source, (self.H, T))
         sc = None if scale is None else _f64(scale, (N,))
@@ -382,6 +392,23 @@ class Solver:
         _check(self.lib.revs_network_check(self._h, src, _dp(Pp), vset, vlow, vhigh, row_tol, _dp(sc), _dp(V), _dp(L),
                                            _dp(Z), C.byref(summ)))
         return dict(summary=summ.as_dict(), voltage=V, loading=L, zone_worst=Z)
+
+    def repair_schedule(self, vset=1.0, vhigh=1.05, row_tol=1e-9, schedule=True, mask=False):
+        """Greedy voltage repair of the last ADMM run's charging decisions, zone by zone on the device
+        (include/revs_admm.h: revs_repair_schedule; a heuristic, a zone may be left with violated rows).  Returns
+        dict(P_sch=[H, T] repaired schedule or None, mask=[H, ceil(T/64)] uint64 charging bits or None,
+        zone_info=[zones, 3] int32 {status 0 untouched / 1 repaired / 2 violations left, hours moved, hours dropped},
+        moves, drops, zones_violated, zones_repaired, zones_left).  P_sch, P_est and the results of the run stay as
+        they are; expand_schedule(mask, ...) gives the repaired P_ev and SOC."""
+        H, T = self.H, self.T
+        W = (T + 63) // 64
+        P = np.empty((H, T)) if schedule else None
+        M = np.empty((H, W), dtype=np.uint64) if mask else None
+        Z = np.zeros((self.nf, 3), dtype=np.int32)
+        _check(self.lib.revs_repair_schedule(self._h, vset, vhigh, row_tol, _dp(P),
+                                             None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W,
+                                             Z.ctypes.data_as(C.POINTER(C.c_int32))))
+        return repair_totals(dict(P_sch=P, mask=M, zone_info=Z))
 
     # ---- the same check with the rows partitioned over the GPUs of the box; the all-gather of the result is fused
     # into the epilogue of the contraction kernel (peer-memory stores, include/revs_admm.h: revs_gather_*)

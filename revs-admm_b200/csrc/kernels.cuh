@@ -302,7 +302,8 @@ struct NetZone {
     int64_t node0, lvl0, res0;    // first entry of the zone in the node / level / residence pools
     int64_t home_row;             // padded row of the zone's first home in the [Hp][T] schedule
     int64_t out_row;              // first row of the zone in the [total nodes][T] outputs
-    int n_nodes, depth, lg, pad_; // lg: log2 of the steps per CTA
+    int n_nodes, depth, lg;       // lg: log2 of the steps per CTA
+    int n_res;                    // residences
 };
 struct NetCta { int zone, t0; int64_t gstate; };     // gstate: offset of the state in the global scratch, -1: shared memory
 struct NetArg { double v; int zone, pad_; int64_t loc; };   // a maximum and where: loc = index * T + step
@@ -317,6 +318,7 @@ struct NetParams {
     const double* scale;          // [total nodes] or null (= 1)
     double* voltage;              // [total nodes][T] or null
     double* loading;              // [total nodes][T] or null
+    double* drop;                 // [Hp * T] or null: D at every residence, the zone's block [T][n_res] at home_row * T
     double* gstate;               // global scratch of the zones above kNetSmemMax
     NetPartial* part;             // [CTAs]
     int T;
@@ -337,5 +339,30 @@ void net_finish(NetHost& h, int T);
 cudaError_t launch_network_check(const NetParams& P, const int* d_list, int n_ctas, size_t smem, cudaStream_t s);
 cudaError_t launch_network_reduce(const NetPartial* part, const int* zone_cta, int n_zones, double* zone_worst,
                                   NetPartial* out, cudaStream_t s);
+
+// ---- repair.cu: greedy voltage repair of the schedule, one CTA per zone
+constexpr int kRepairSmemMaxN = 2048;   // zones above this many residences keep their state in the global scratch
+constexpr int kRepairMaxT = 256;        // longest horizon (home_solve.cu)
+struct RepairParams {
+    const NetZone* zones;         // the network check's breadth-first arrays
+    const NetNode* nodes;
+    const int* res;
+    const double* cumr;           // [total nodes] cumulative resistance of every node, zone z at zones[z].out_row
+    const double* zone_worst;     // [zones][3] of the network check of the schedule: zones with excess > row_tol run
+    const double* load;           // [Hp][T]
+    const double* rating;         // [Hp]
+    const double* cost;           // [T]
+    const int *start, *end, *n_min;   // [Hp]
+    double* D;                    // [Hp * T] drops of the schedule at the residences (NetParams::drop), updated
+    double* P;                    // [Hp][T] in: the schedule, out: the repaired schedule
+    double* p_ev;                 // [Hp][T] in: the charger power, out: the repaired one
+    char* gws;                    // global scratch of the zones above kRepairSmemMaxN ...
+    const int64_t* ws_off;        // ... [zones] byte offset of the zone's state in it, -1: shared memory
+    int32_t* info;                // [zones][3] status, moves, drops
+    int T;
+    double u, row_tol;
+};
+size_t repair_ws_bytes(int n_res, int T);     // bytes of a zone's state
+cudaError_t launch_repair(const RepairParams& P, int n_zones, size_t smem, cudaStream_t s);
 
 }  // namespace revs

@@ -156,6 +156,10 @@ __global__ void __launch_bounds__(kNetThreads) network_check_kernel(NetParams p,
             net_take(m.drop, d, c.zone, (int64_t)n.node * T + t);
             if (d > p.low) ++m.low;
             if (n.nres > 0) {
+                if (p.drop) {
+                    double* dt = p.drop + z.home_row * T + (int64_t)t * z.n_res;
+                    for (int e = 0; e < n.nres; ++e) dt[rl[n.res0 + e]] = d;
+                }
                 const double x = d - p.u;
                 net_take(m.exc, x, c.zone, (int64_t)rl[n.res0] * T + t);     // first (lowest) residence of the node
                 if (x > p.row_tol) m.rows += (unsigned long long)n.nres;
@@ -209,6 +213,7 @@ void net_add_zone(NetHost& h, int n_nodes, const int* parent, const double* cumr
     z.home_row = home_row;
     z.out_row = h.total_nodes;
     z.n_nodes = n_nodes;
+    z.n_res = n_res;
     z.depth = (int)B.lvl.size() - 1;
     h.levels.insert(h.levels.end(), B.lvl.begin(), B.lvl.end());
     h.res.insert(h.res.end(), B.res.begin(), B.res.end());

@@ -196,6 +196,14 @@ struct revs_solver {
            *d_net_load = nullptr;
     size_t net_cap[6] = {0, 0, 0, 0, 0, 0};    // elements allocated: nodes, levels, residences, CTAs, zones, global state
     bool net_scale_ok = false, net_out_ok = false;
+    double* d_net_cumr = nullptr;              // [total nodes] cumulative resistances in the network check's zone order
+    // greedy voltage repair (revs_repair_schedule, repair.cu): the repaired schedule of the current ADMM run and scratch
+    bool rep_valid = false;
+    double *d_rep_P = nullptr, *d_rep_pev = nullptr, *d_rep_D = nullptr;
+    char* d_rep_gws = nullptr;
+    int64_t* d_rep_wsoff = nullptr;
+    int32_t* d_rep_info = nullptr;
+    size_t rep_smem = 0;
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -898,7 +906,8 @@ void free_all(revs_solver* s) {
                     s->d_nt_zones, s->d_nt_lvl, s->d_nt_parent, s->d_nt_home, s->d_nt_hnode, s->d_nt_wsi, s->d_nt_child, s->d_nt_homes, s->d_nt_rho,
                     s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2, s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists,
                     s->d_net_zone_cta, s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_P,
-                    s->d_net_scale, s->d_net_volt, s->d_net_load};
+                    s->d_net_scale, s->d_net_volt, s->d_net_load, s->d_net_cumr, s->d_rep_P, s->d_rep_pev, s->d_rep_D,
+                    s->d_rep_gws, s->d_rep_wsoff, s->d_rep_info};
     for (int r = 0; r < kMaxPeers; ++r)
         if (s->peer_box[r] && s->peer_box[r] != s->d_mailbox) cudaIpcCloseMemHandle(s->peer_box[r]);
     for (int r = 0; r < kGatherMaxPeers; ++r)
@@ -1331,6 +1340,7 @@ int revs_admm_begin(revs_solver* s, double kappa, int iter_max, double vset, dou
     CU(cudaSetDevice(s->device));
     s->kappa = kappa; s->iter_max = iter_max; s->vset = vset; s->vlow = vlow; s->vhigh = vhigh;
     s->k = 0; s->cur = 0; s->running = true;
+    s->rep_valid = false;            // the repaired schedule belongs to the previous run
     s->warm_cls = 0;                 // multipliers start at zero
     s->ws_bound = 0;
     memset(&s->stats, 0, sizeof s->stats);
@@ -1979,7 +1989,7 @@ int net_prepare(revs_solver* s) {
                         "revs_set_feeder_tree(s)", f);
     NetHost h;
     std::vector<int> par, res;
-    std::vector<double> cumr;
+    std::vector<double> cumr, all_cumr;
     for (int f = 0; f < s->nf; ++f) {
         const Tree& t = s->trees[f];
         const FeederDev& fd = s->feeders[f];
@@ -1990,19 +2000,23 @@ int net_prepare(revs_solver* s) {
         CU(cudaMemcpy(cumr.data(), t.d_cumr, sizeof(double) * t.n_nodes, cudaMemcpyDeviceToHost));
         if (fd.n) CU(cudaMemcpy(res.data(), t.d_res_node, sizeof(int) * fd.n, cudaMemcpyDeviceToHost));
         net_add_zone(h, t.n_nodes, par.data(), cumr.data(), fd.n, res.data(), fd.off);
+        all_cumr.insert(all_cumr.end(), cumr.begin(), cumr.end());
     }
     net_finish(h, s->T);
     // the arrays below depend on the trees; the host-input staging d_net_P does not
     void* old[] = {s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists, s->d_net_zone_cta,
                    s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_scale, s->d_net_volt,
-                   s->d_net_load};
+                   s->d_net_load, s->d_net_cumr};
     for (void* p : old)
         if (p) cudaFree(p);
     s->d_net_zones = nullptr; s->d_net_nodes = nullptr; s->d_net_levels = nullptr; s->d_net_res = nullptr;
     s->d_net_lists = nullptr; s->d_net_zone_cta = nullptr; s->d_net_ctas = nullptr; s->d_net_part = nullptr;
     s->d_net_sum = nullptr; s->d_net_zw = nullptr; s->d_net_gstate = nullptr; s->d_net_scale = nullptr;
-    s->d_net_volt = nullptr; s->d_net_load = nullptr;
+    s->d_net_volt = nullptr; s->d_net_load = nullptr; s->d_net_cumr = nullptr;
     CU(dalloc(&s->d_net_zones, h.zones.size()));
+    CU(dalloc(&s->d_net_cumr, all_cumr.size()));
+    if (!all_cumr.empty())
+        CU(cudaMemcpy(s->d_net_cumr, all_cumr.data(), sizeof(double) * all_cumr.size(), cudaMemcpyHostToDevice));
     CU(dalloc(&s->d_net_nodes, h.nodes.size()));
     CU(dalloc(&s->d_net_levels, h.levels.size()));
     CU(dalloc(&s->d_net_res, h.res.size()));
@@ -2025,6 +2039,40 @@ int net_prepare(revs_solver* s) {
     return REVS_OK;
 }
 
+// The network check kernels on the schedule P (device, [Hp][T]): per-CTA partials, d_net_zw and d_net_sum, and
+// optionally the voltages, loadings and residence drops.
+int net_run(revs_solver* s, const double* P, double v2, double u, double low, double row_tol, const double* scale,
+            double* voltage, double* loading, double* drop, int64_t* launches) {
+    const NetHost& h = s->net;
+    NetParams prm{};
+    prm.zones = s->d_net_zones;
+    prm.nodes = s->d_net_nodes;
+    prm.levels = s->d_net_levels;
+    prm.res = s->d_net_res;
+    prm.ctas = s->d_net_ctas;
+    prm.P = P;
+    prm.scale = scale;
+    prm.voltage = voltage;
+    prm.loading = loading;
+    prm.drop = drop;
+    prm.gstate = s->d_net_gstate;
+    prm.part = s->d_net_part;
+    prm.T = s->T;
+    prm.v2 = v2;
+    prm.u = u;
+    prm.low = low;
+    prm.row_tol = row_tol;
+    for (int c = 0; c < 3; ++c) {
+        const int n = h.class_off[c + 1] - h.class_off[c];
+        if (n == 0) continue;
+        CU(launch_network_check(prm, s->d_net_lists + h.class_off[c], n, c == 2 ? 0 : h.class_smem[c], s->sU));
+        ++*launches;
+    }
+    CU(launch_network_reduce(s->d_net_part, s->d_net_zone_cta, s->nf, s->d_net_zw, s->d_net_sum, s->sU));
+    ++*launches;
+    return REVS_OK;
+}
+
 void net_location(const NetArg& a, int T, int32_t* zone, int32_t* index, int32_t* step) {
     const bool none = a.loc == INT64_MAX;      // no candidate (no residence at all)
     *zone = none ? -1 : a.zone;
@@ -2039,11 +2087,15 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
                        const double* scale, double* voltage, double* loading, double* zone_worst,
                        revs_network_summary* summary) {
     if (!s) return fail(REVS_ERR_ARG, "null solver");
-    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST)
-        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE or REVS_NET_HOST)", source);
+    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST && source != REVS_NET_REPAIRED)
+        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST or REVS_NET_REPAIRED)",
+                    source);
     if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
     if (source != REVS_NET_HOST && s->k == 0)
-        return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check", source == REVS_NET_SCHEDULE ? "schedule" : "estimate");
+        return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check",
+                    source == REVS_NET_SCHEDULE ? "schedule" : source == REVS_NET_ESTIMATE ? "estimate" : "repaired schedule");
+    if (source == REVS_NET_REPAIRED && !s->rep_valid)
+        return fail(REVS_ERR_ARG, "REVS_NET_REPAIRED: revs_repair_schedule has not run since the last ADMM run began");
     const double v2 = vset * vset, u = vhigh * vhigh - v2, lo = vlow * vlow - v2;
     if (!(u > 0.0) || !(lo <= 0.0)) return fail(REVS_ERR_ARG, "need vlow <= vset < vhigh");
     CU(cudaSetDevice(s->device));
@@ -2053,7 +2105,7 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
     const int T = s->T;
     const size_t out_elems = (size_t)h.total_nodes * T;
     int64_t launches = 0;
-    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : s->d_pest;
+    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->d_rep_P : s->d_pest;
     if (source == REVS_NET_HOST) {
         if (!s->d_net_P) CU(dalloc(&s->d_net_P, (size_t)s->Hp * T));
         if ((rc = h2d_homes(s, s->d_net_P, P, T))) return rc;
@@ -2066,31 +2118,9 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
     }
     if (voltage && !s->d_net_volt) CU(dalloc(&s->d_net_volt, out_elems));
     if (loading && !s->d_net_load) CU(dalloc(&s->d_net_load, out_elems));
-    NetParams prm{};
-    prm.zones = s->d_net_zones;
-    prm.nodes = s->d_net_nodes;
-    prm.levels = s->d_net_levels;
-    prm.res = s->d_net_res;
-    prm.ctas = s->d_net_ctas;
-    prm.P = src;
-    prm.scale = scale ? s->d_net_scale : nullptr;
-    prm.voltage = voltage ? s->d_net_volt : nullptr;
-    prm.loading = loading ? s->d_net_load : nullptr;
-    prm.gstate = s->d_net_gstate;
-    prm.part = s->d_net_part;
-    prm.T = T;
-    prm.v2 = v2;
-    prm.u = u;
-    prm.low = -lo;
-    prm.row_tol = row_tol;
-    for (int c = 0; c < 3; ++c) {
-        const int n = h.class_off[c + 1] - h.class_off[c];
-        if (n == 0) continue;
-        CU(launch_network_check(prm, s->d_net_lists + h.class_off[c], n, c == 2 ? 0 : h.class_smem[c], s->sU));
-        ++launches;
-    }
-    CU(launch_network_reduce(s->d_net_part, s->d_net_zone_cta, s->nf, s->d_net_zw, s->d_net_sum, s->sU));
-    ++launches;
+    if ((rc = net_run(s, src, v2, u, -lo, row_tol, scale ? s->d_net_scale : nullptr, voltage ? s->d_net_volt : nullptr,
+                      loading ? s->d_net_load : nullptr, nullptr, &launches)))
+        return rc;
     NetPartial m;
     CU(cudaMemcpyAsync(&m, s->d_net_sum, sizeof m, cudaMemcpyDeviceToHost, s->sU));
     if (zone_worst) CU(cudaMemcpyAsync(zone_worst, s->d_net_zw, sizeof(double) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
@@ -2112,6 +2142,89 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
         o.edges_overloaded = (int64_t)m.over;
         *summary = o;
     }
+    return REVS_OK;
+}
+
+int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_tol, double* P_out, uint64_t* hour_mask,
+                         int mask_words, int32_t* zone_info) {
+    if (!s) return fail(REVS_ERR_ARG, "null solver");
+    if (s->k == 0) return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no schedule to repair");
+    if (hour_mask && mask_words != (s->T + 63) / 64) return fail(REVS_ERR_ARG, "mask_words must be ceil(T / 64) = %d", (s->T + 63) / 64);
+    const double v2 = vset * vset, u = vhigh * vhigh - v2;
+    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
+    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
+    CU(cudaSetDevice(s->device));
+    int rc = net_prepare(s);
+    if (rc) return rc;
+    const int T = s->T;
+    const size_t HT = (size_t)s->Hp * T;
+    if (!s->d_rep_P) {
+        // the zones' state: shared memory up to kRepairSmemMaxN residences, else a block of the global scratch
+        std::vector<int64_t> off(s->nf);
+        int64_t g = 0;
+        for (int f = 0; f < s->nf; ++f) {
+            const size_t b = repair_ws_bytes(s->feeders[f].n, T);
+            if (s->feeders[f].n > kRepairSmemMaxN) {
+                off[f] = g;
+                g += (int64_t)b;
+            } else {
+                off[f] = -1;
+                s->rep_smem = std::max(s->rep_smem, b);
+            }
+        }
+        CU(dalloc(&s->d_rep_wsoff, (size_t)s->nf));
+        CU(cudaMemcpy(s->d_rep_wsoff, off.data(), sizeof(int64_t) * s->nf, cudaMemcpyHostToDevice));
+        CU(dalloc(&s->d_rep_gws, (size_t)g));
+        CU(dalloc(&s->d_rep_info, (size_t)3 * s->nf));
+        CU(dalloc(&s->d_rep_D, HT));
+        CU(dalloc(&s->d_rep_pev, HT));
+        CU(dalloc(&s->d_rep_P, HT));
+        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
+    }
+    s->rep_valid = false;
+    int64_t launches = 0;
+    CU(cudaMemcpyAsync(s->d_rep_P, s->d_psch[s->cur], HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(s->d_rep_pev, s->d_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    // the drops of the schedule at every residence, and which zones violate a row
+    if ((rc = net_run(s, s->d_psch[s->cur], v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_rep_D, &launches))) return rc;
+    RepairParams rp{};
+    rp.zones = s->d_net_zones;
+    rp.nodes = s->d_net_nodes;
+    rp.res = s->d_net_res;
+    rp.cumr = s->d_net_cumr;
+    rp.zone_worst = s->d_net_zw;
+    rp.load = s->d_load;
+    rp.rating = s->d_rating;
+    rp.cost = s->d_cost;
+    rp.start = s->d_start;
+    rp.end = s->d_end;
+    rp.n_min = s->d_nmin;
+    rp.D = s->d_rep_D;
+    rp.P = s->d_rep_P;
+    rp.p_ev = s->d_rep_pev;
+    rp.gws = s->d_rep_gws;
+    rp.ws_off = s->d_rep_wsoff;
+    rp.info = s->d_rep_info;
+    rp.T = T;
+    rp.u = u;
+    rp.row_tol = row_tol;
+    CU(launch_repair(rp, s->nf, s->rep_smem, s->sU));
+    launches += s->nf > 0;
+    if (hour_mask && s->H > 0) {
+        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
+        CU(launch_hour_mask(s->d_rep_pev, s->d_hmap, s->H, T, d_mask, s->sU));
+        ++launches;
+        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
+    }
+    if (P_out && s->H > 0) {
+        if ((rc = d2h_homes(s, P_out, s->d_rep_P, T))) return rc;
+        ++launches;
+    }
+    if (zone_info && s->nf > 0)
+        CU(cudaMemcpyAsync(zone_info, s->d_rep_info, sizeof(int32_t) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->stats.kernel_launches += launches;
+    s->rep_valid = true;
     return REVS_OK;
 }
 

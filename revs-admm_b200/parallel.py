@@ -389,6 +389,15 @@ class PipelinedSolver:
                     voltage=None if out is None else out["voltage"], loading=None if out is None else out["loading"],
                     zone_worst=np.concatenate([r["zone_worst"] for r in res]) if zones else None)
 
+    def repair_schedule(self, schedule=True, mask=False, **kw):
+        """Solver.repair_schedule over all pipelines at once: the schedules, masks and zone_info are concatenated in
+        zone order and the totals summed -- the bytes of a single solver over the same zones."""
+        from ._cabi import repair_totals
+        res = self._each(lambda k: self.parts[k].repair_schedule(schedule=schedule, mask=mask, **kw))
+        return repair_totals(dict(P_sch=np.concatenate([r["P_sch"] for r in res]) if schedule else None,
+                                  mask=np.concatenate([r["mask"] for r in res]) if mask else None,
+                                  zone_info=np.concatenate([r["zone_info"] for r in res])))
+
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
         pipeline (they run side by side), residuals are recombined from the per-pipeline norms."""
