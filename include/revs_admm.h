@@ -23,6 +23,7 @@
  *                                                                     compute_voltage()
  *   revs_network_check                            drawing.py:29-78    the same for every zone at once
  *   revs_repair_schedule                          no reference counterpart (a voltage-feasible binary schedule)
+ *   revs_central_bracket                          lpsolver.py:463-502 solve_central(), bracketed per zone
  *   revs_get_results / revs_get_schedule(_ld)     lpsolver.py:289-290 return diff,P_sch,S,C
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
@@ -172,15 +173,17 @@ int revs_reliability(revs_solver* s, int feeder, int kind, int n_rows, const int
  * tree (leaves -> root: flows F, root -> leaves: squared-voltage drops D = R P), O(nodes x T), no sensitivity
  * matrix; every zone needs its tree (revs_set_feeder_tree(s)).
  * source: REVS_NET_SCHEDULE / REVS_NET_ESTIMATE (schedule / operator estimate of the last ADMM run, already on the
- * device, P ignored), REVS_NET_HOST (P [H,T] from the host, compact home order of revs_create) or REVS_NET_REPAIRED
- * (the repaired schedule of revs_repair_schedule, below).
+ * device, P ignored), REVS_NET_HOST (P [H,T] from the host, compact home order of revs_create), REVS_NET_REPAIRED
+ * (the repaired schedule of revs_repair_schedule, below) or REVS_NET_CENTRAL (the kept schedule of
+ * revs_central_bracket, below).
  * "Total nodes" are the nodes of all zones concatenated in zone order (node_off of revs_set_feeder_trees); rows of
  * voltage / loading, and scale, follow it.  voltage = sqrt(vset^2 - D) (REVS_REL_VOLTAGE), loading = scale * F
  * (REVS_REL_FLOW, scale = signed 1/rating per edge, NULL = 1).  voltage, loading, zone_worst and summary may be NULL.
  * Ties of every maximum go to the lowest (zone, node or residence, step); counts are exact: two calls give the same
  * bytes, and the result of a zone does not depend on the other zones of the solver.
  * REVS_ERR_ARG: a zone without tree (the message names it), SCHEDULE / ESTIMATE before any ADMM iteration, HOST
- * without P, REPAIRED before a repair of the current ADMM run, an unknown source, or not vlow <= vset < vhigh.  Synchronous on the utility stream; adds its launches to
+ * without P, REPAIRED before a repair of the current ADMM run, CENTRAL before a bracket of the current homes, tariff and
+ * trees, an unknown source, or not vlow <= vset < vhigh.  Synchronous on the utility stream; adds its launches to
  * revs_stats.kernel_launches and changes no other state.  The breadth-first arrays it needs are built on its first
  * call after the trees are set, its scratch on first use; both are kept until revs_destroy. */
 #define REVS_NET_SCHEDULE 0   /* P_sch of the last ADMM run (what revs_get_results returns)      */
@@ -236,6 +239,39 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
 int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_tol,
                          double* P_out, uint64_t* hour_mask, int mask_words, int32_t* zone_info);
 #define REVS_NET_REPAIRED 3   /* the schedule of the last revs_repair_schedule of the current ADMM run  */
+
+/* Bracket of the centralized optimum (the reference's solve_central, lpsolver.py:463-502: minimise the tariff cost
+ * under the SOC and voltage rows), zone by zone on the device: UB_z, the cost of a voltage-feasible binary schedule
+ * that keeps every home's SOC window and plug-in window, and LB_z, a lower bound on the cost of every such schedule.
+ * Needs the homes, the tariff and the tree of every zone; an ADMM run is not needed, and nothing of one is read or
+ * changed.  P_out [H,T] (compact home order), hour_mask [H, mask_words], zone_bounds [n_feeders, 2] {LB, UB} and
+ * zone_info [n_feeders, 3] int32 {status, ascent steps run, hours moved + dropped by the repair of the kept start}
+ * may each be NULL.  The kept schedule stays on the device for revs_network_check(REVS_NET_CENTRAL) until the homes,
+ * tariff or trees change.
+ *
+ * The method, with u = vhigh^2 - vset^2, c the tariff, P = load + rating e (e binary inside the plug-in window,
+ * n_min <= sum e <= n_max as in the home solve), R the residences' sensitivity block and y >= 0 one price per
+ * (residence, step):
+ *   1. priced selection e*(y): every home takes the n_min window hours of smallest reduced cost rating (c_t + (R y)_t),
+ *      then further hours while the reduced cost is negative, up to n_max; ties to the earliest hour, exact values;
+ *   2. phi(y) = sum c P(y) + sum y (R P(y) - u) is a lower bound on every feasible schedule's cost, at every y;
+ *   3. start y = 0 (phi(0) = cost of every home's cheapest SOC-feasible hours); the greedy rule of
+ *      revs_repair_schedule applied to e*(0) gives UB_z (+inf when it leaves a violated row);
+ *   4. evaluations k = 0..iters of phi(y_k); LB_z = the best; theta_z (from 1) halves after 20 evaluations without a
+ *      new best; y <- max(y + theta_z (target_z - phi_z) / ||g_z||^2 (R P - u), 0), g the projected subgradient,
+ *      target_z = UB_z when a feasible schedule is known, else C_max_z + 0.01 |C_max_z|.  C_max_z is the cost of the
+ *      most expensive SOC-feasible schedule (the n_min dearest window hours, then further hours while c_t > 0, up to
+ *      n_max).  A zone stops when UB_z - LB_z <= 1e-9 |UB_z|, g_z = 0, or (without a feasible schedule) LB_z > C_max_z;
+ *   5. the greedy repair of e*(y_best) is a second start; the cheaper repaired schedule is kept, ties to the first.
+ * Status: 0 = e*(0) meets every row (optimal, LB = UB); 1 = bracketed, LB <= optimum <= UB; 2 = no feasible schedule
+ * found (UB = +inf; the kept schedule violates rows); 3 = certified infeasible, LB_z > C_max_z (UB = +inf).
+ * Sums run in a fixed order: two calls give the same bytes, and a zone's result does not depend on the other zones.
+ * REVS_ERR_INFEASIBLE: a home whose n_min exceeds its plug-in window.  REVS_ERR_ARG: homes or tariff not set, a zone
+ * without tree (named), iters < 0, mask_words != ceil(T/64) with hour_mask, not vset < vhigh, row_tol < 0 or NaN.
+ * Synchronous on the utility stream; adds its launches to revs_stats.kernel_launches. */
+int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_tol, int iters, double* P_out,
+                         uint64_t* hour_mask, int mask_words, double* zone_bounds, int32_t* zone_info);
+#define REVS_NET_CENTRAL 4    /* the kept schedule of the last revs_central_bracket                    */
 
 /* The same check with the ROWS PARTITIONED over the GPUs of one box (one process per GPU, every process holds the
  * feeder's tree; BASELINE north_star: "the sensitivity contraction is row-partitioned"): every rank builds and

@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("REVS_LIB") or os.path.join(HERE, "librevs_admm.so")     # REVS_LIB: a build variant (profiles/build_variants.sh)
 
 REVS_REL_VOLTAGE, REVS_REL_FLOW, REVS_REL_DROP = 0, 1, 2
-REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED = 0, 1, 2, 3
+REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED, REVS_NET_CENTRAL = 0, 1, 2, 3, 4
 
 
 class RevsError(RuntimeError):
@@ -90,6 +90,8 @@ SIGNATURES = {
     "revs_network_check": ([_P, C.c_int, _D, C.c_double, C.c_double, C.c_double, C.c_double, _D, _D, _D, _D,
                             C.POINTER(NetworkSummary)], C.c_int),
     "revs_repair_schedule": ([_P, C.c_double, C.c_double, C.c_double, _D, C.POINTER(C.c_uint64), C.c_int,
+                              C.POINTER(C.c_int32)], C.c_int),
+    "revs_central_bracket": ([_P, C.c_double, C.c_double, C.c_double, C.c_int, _D, C.POINTER(C.c_uint64), C.c_int, _D,
                               C.POINTER(C.c_int32)], C.c_int),
 }
 
@@ -179,6 +181,18 @@ def repair_totals(r):
     z = r["zone_info"]
     r.update(moves=int(z[:, 1].sum()), drops=int(z[:, 2].sum()), zones_violated=int((z[:, 0] > 0).sum()),
              zones_repaired=int((z[:, 0] == 1).sum()), zones_left=int((z[:, 0] == 2).sum()))
+    return r
+
+
+def central_totals(r):
+    """Add the totals of zone_bounds / zone_info to a central_bracket result: lb (sum of LB over all zones), lb_bracketed
+    and ub (sums of LB and UB over the zones of status 0 and 1), gap = (ub - lb_bracketed) / |lb_bracketed| and
+    zones_status (zones of status 0, 1, 2, 3)."""
+    b, st = r["zone_bounds"], r["zone_info"][:, 0]
+    ok = st <= 1
+    lbb, ub = float(b[ok, 0].sum()), float(b[ok, 1].sum())
+    r.update(lb=float(b[:, 0].sum()), lb_bracketed=lbb, ub=ub, gap=(ub - lbb) / abs(lbb) if lbb else 0.0,
+             zones_status=[int((st == k).sum()) for k in range(4)])
     return r
 
 
@@ -365,16 +379,19 @@ class Solver:
                       zones=False, out=None):
         """Voltages and line loadings of every node of every zone, per step, in one call (include/revs_admm.h:
         revs_network_check).  source: "schedule" (P_sch of the last ADMM run), "estimate" (P_est), "repaired" (the
-        schedule of the last repair_schedule of that run) or a host schedule P [H, T].  scale: [total_nodes] signed 1/rating per edge (None = 1).  Returns dict(summary=dict,
+        schedule of the last repair_schedule of that run), "central" (the kept schedule of the last central_bracket) or a host
+        schedule P [H, T].  scale: [total_nodes] signed 1/rating per edge (None = 1).  Returns dict(summary=dict,
         voltage=[total_nodes, T], loading=[total_nodes, T], zone_worst=[zones, 3]); the arrays are None unless
         asked for with full / zones.  out: optional dict of C-contiguous float64 [total_nodes, T] arrays voltage
         and loading to write into."""
         N, T = self.total_nodes, self.T
         Pp = None
         if isinstance(source, str):
-            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE, "repaired": REVS_NET_REPAIRED}.get(source)
+            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE, "repaired": REVS_NET_REPAIRED,
+                   "central": REVS_NET_CENTRAL}.get(source)
             if src is None:
-                raise ValueError(f"source must be 'schedule', 'estimate', 'repaired' or an [H, T] array, not {source!r}")
+                raise ValueError("source must be 'schedule', 'estimate', 'repaired', 'central' or an [H, T] array, "
+                                 f"not {source!r}")
         else:
             src, Pp = REVS_NET_HOST, _f64(source, (self.H, T))
         sc = None if scale is None else _f64(scale, (N,))
@@ -409,6 +426,24 @@ class Solver:
                                              None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W,
                                              Z.ctypes.data_as(C.POINTER(C.c_int32))))
         return repair_totals(dict(P_sch=P, mask=M, zone_info=Z))
+
+    def central_bracket(self, vset=1.0, vhigh=1.05, row_tol=1e-9, iters=100, schedule=True, mask=False):
+        """Bracket of the centralized optimum zone by zone on the device (include/revs_admm.h: revs_central_bracket):
+        a voltage-feasible binary schedule (UB) and a Lagrangian lower bound (LB) per zone, from the homes, tariff and
+        trees alone.  Returns dict(P_sch=[H, T] kept schedule or None, mask=[H, ceil(T/64)] uint64 charging bits or
+        None, zone_bounds=[zones, 2] {LB, UB}, zone_info=[zones, 3] int32 {status 0 optimal / 1 bracketed / 2 no
+        feasible schedule found / 3 certified infeasible, ascent steps, repair moves + drops of the kept start}) and
+        the totals of central_totals.  Nothing of an ADMM run is read or changed."""
+        H, T = self.H, self.T
+        W = (T + 63) // 64
+        P = np.empty((H, T)) if schedule else None
+        M = np.empty((H, W), dtype=np.uint64) if mask else None
+        B = np.zeros((self.nf, 2))
+        Z = np.zeros((self.nf, 3), dtype=np.int32)
+        _check(self.lib.revs_central_bracket(self._h, vset, vhigh, row_tol, int(iters), _dp(P),
+                                             None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W, _dp(B),
+                                             Z.ctypes.data_as(C.POINTER(C.c_int32))))
+        return central_totals(dict(P_sch=P, mask=M, zone_bounds=B, zone_info=Z))
 
     # ---- the same check with the rows partitioned over the GPUs of the box; the all-gather of the result is fused
     # into the epilogue of the contraction kernel (peer-memory stores, include/revs_admm.h: revs_gather_*)

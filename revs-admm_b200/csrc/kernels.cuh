@@ -365,4 +365,49 @@ struct RepairParams {
 size_t repair_ws_bytes(int n_res, int T);     // bytes of a zone's state
 cudaError_t launch_repair(const RepairParams& P, int n_zones, size_t smem, cudaStream_t s);
 
+// ---- central.cu: bracket of the centralized optimum per zone (priced selections, Lagrangian ascent, two repairs)
+struct CenSelectParams {          // one warp per home: e*(y), or the most expensive SOC-feasible hours
+    const NetZone* zones;
+    const int* hzone;             // [Hp] zone of every home (EV homes only are read)
+    const double* ry;             // zone blocks [T][n]: R y at the residences (NetParams::drop), or null (y = 0)
+    const double *load, *rating, *cost;
+    const uint8_t* has_ev;
+    const int *start, *end, *n_min, *n_max;
+    double* P;                    // [Hp][T] out: load + rating e
+    double* p_ev;                 // [Hp][T] out: rating e
+    int* infeasible;              // set when a home's n_min exceeds its window or n_max
+    int64_t Hp;
+    int T;
+    int most_expensive;           // 1: reduced cost -rating c (ry ignored)
+};
+struct CenZone { double lb, ub, theta; int stall, done, steps, pad_; };
+struct CenAscentParams {
+    const NetZone* zones;
+    const double* cost;           // [T]
+    const double* P;              // [Hp][T] e*(y) of this evaluation
+    const double* D;              // zone blocks [T][n]: R P
+    double *y, *ybest;            // [Hp][T]
+    const double *cost1, *cmax;   // [zones] cost of the repaired e*(0), C_max
+    const int32_t* info1;         // [zones][3] repair of e*(0)
+    CenZone* state;               // [zones]
+    int k, iters, T;
+    double u;
+};
+struct CenFinalParams {
+    const NetZone* zones;
+    const CenZone* state;
+    const double *cost1, *cost2, *cmax;
+    const int32_t *info1, *info2;
+    double *P1, *p_ev1;           // [Hp][T] repaired e*(0); out: the kept schedule
+    const double *P2, *p_ev2;     // [Hp][T] repaired e*(y_best)
+    double* bounds;               // [zones][2] LB, UB
+    int32_t* info;                // [zones][3] status, ascent steps, moves + drops of the kept start
+    int T;
+};
+cudaError_t launch_central_select(const CenSelectParams& P, cudaStream_t s);
+cudaError_t launch_central_ascent(const CenAscentParams& P, int n_zones, cudaStream_t s);
+cudaError_t launch_central_cost(const NetZone* zones, int n_zones, const double* cost, const double* P, int T,
+                                double* out, cudaStream_t s);
+cudaError_t launch_central_final(const CenFinalParams& P, int n_zones, cudaStream_t s);
+
 }  // namespace revs

@@ -204,6 +204,18 @@ struct revs_solver {
     int64_t* d_rep_wsoff = nullptr;
     int32_t* d_rep_info = nullptr;
     size_t rep_smem = 0;
+    // bracket of the centralized optimum (revs_central_bracket, central.cu): its kept schedule, valid until the homes,
+    // tariff or trees change, and its own scratch (never the repair's above)
+    bool cen_valid = false;
+    double *d_cen_y = nullptr, *d_cen_yb = nullptr, *d_cen_P = nullptr, *d_cen_pev = nullptr, *d_cen_D = nullptr,
+           *d_cen_Drep = nullptr, *d_cen_P1 = nullptr, *d_cen_pev1 = nullptr, *d_cen_P2 = nullptr, *d_cen_pev2 = nullptr;
+    double *d_cen_sums = nullptr, *d_cen_bounds = nullptr;    // [3][zones] cost1, cost2, C_max; [zones][2]
+    int32_t *d_cen_info = nullptr;                            // [3][zones][3] repair of start 1, of start 2, result
+    CenZone* d_cen_state = nullptr;
+    int *d_cen_hzone = nullptr, *d_cen_flag = nullptr;
+    char* d_cen_gws = nullptr;
+    int64_t* d_cen_wsoff = nullptr;
+    size_t cen_smem = 0;
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -907,7 +919,10 @@ void free_all(revs_solver* s) {
                     s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2, s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists,
                     s->d_net_zone_cta, s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_P,
                     s->d_net_scale, s->d_net_volt, s->d_net_load, s->d_net_cumr, s->d_rep_P, s->d_rep_pev, s->d_rep_D,
-                    s->d_rep_gws, s->d_rep_wsoff, s->d_rep_info};
+                    s->d_rep_gws, s->d_rep_wsoff, s->d_rep_info, s->d_cen_y, s->d_cen_yb, s->d_cen_P, s->d_cen_pev,
+                    s->d_cen_D, s->d_cen_Drep, s->d_cen_P1, s->d_cen_pev1, s->d_cen_P2, s->d_cen_pev2, s->d_cen_sums,
+                    s->d_cen_bounds, s->d_cen_info, s->d_cen_state, s->d_cen_hzone, s->d_cen_flag, s->d_cen_gws,
+                    s->d_cen_wsoff};
     for (int r = 0; r < kMaxPeers; ++r)
         if (s->peer_box[r] && s->peer_box[r] != s->d_mailbox) cudaIpcCloseMemHandle(s->peer_box[r]);
     for (int r = 0; r < kGatherMaxPeers; ++r)
@@ -1155,6 +1170,7 @@ int revs_set_feeder_tree(revs_solver* s, int feeder, int n_nodes, const int32_t*
     if (t.d_parent && !t.pooled) { cudaFree(t.d_parent); cudaFree(t.d_cumr); cudaFree(t.d_res_node); }
     t = Tree();
     s->net_valid = false;
+    s->cen_valid = false;
     t.n_nodes = n_nodes;
     CU(dalloc(&t.d_parent, (size_t)n_nodes));
     CU(dalloc(&t.d_cumr, (size_t)n_nodes));
@@ -1205,6 +1221,7 @@ int revs_set_feeder_trees(revs_solver* s, const int64_t* node_off, const int32_t
         }
     }
     s->net_valid = false;
+    s->cen_valid = false;
     if (s->pool_nodes < (size_t)total) {
         if (s->d_pool_parent) { cudaFree(s->d_pool_parent); cudaFree(s->d_pool_cumr); s->d_pool_parent = nullptr; s->d_pool_cumr = nullptr; }
         CU(dalloc(&s->d_pool_parent, (size_t)total));
@@ -1319,6 +1336,7 @@ int revs_set_homes(revs_solver* s, const double* load, const uint8_t* has_ev, co
     if (s->debug_host)
         fprintf(stderr, "[revs host] set_homes: staging %.3f ms, waiting for the link %.3f ms, copies %.3f ms\n", th1 - th0, th2 - th1, now_ms() - th2);
     s->homes_set = true;
+    s->cen_valid = false;
     return REVS_OK;
 }
 
@@ -1327,6 +1345,7 @@ int revs_set_tariff(revs_solver* s, const double* cost) {
     CU(cudaSetDevice(s->device));
     CU(cudaMemcpy(s->d_cost, cost, sizeof(double) * s->T, cudaMemcpyHostToDevice));
     s->tariff_set = true;
+    s->cen_valid = false;
     return REVS_OK;
 }
 
@@ -2073,6 +2092,55 @@ int net_run(revs_solver* s, const double* P, double v2, double u, double low, do
     return REVS_OK;
 }
 
+// The repair kernel's per-zone state: shared memory up to kRepairSmemMaxN residences, else a block of a global
+// scratch (*gws, offsets *wsoff); *smem = the largest shared block.
+int repair_scratch(revs_solver* s, int64_t** wsoff, char** gws, size_t* smem) {
+    std::vector<int64_t> off(s->nf);
+    int64_t g = 0;
+    for (int f = 0; f < s->nf; ++f) {
+        const size_t b = repair_ws_bytes(s->feeders[f].n, s->T);
+        if (s->feeders[f].n > kRepairSmemMaxN) {
+            off[f] = g;
+            g += (int64_t)b;
+        } else {
+            off[f] = -1;
+            *smem = std::max(*smem, b);
+        }
+    }
+    CU(dalloc(wsoff, (size_t)s->nf));
+    CU(cudaMemcpy(*wsoff, off.data(), sizeof(int64_t) * s->nf, cudaMemcpyHostToDevice));
+    CU(dalloc(gws, (size_t)g));
+    return REVS_OK;
+}
+
+// The repair kernel on the schedule P / p_ev (in place) with the drops D of net_run(P), whose zone_worst it reads.
+int run_repair(revs_solver* s, double u, double row_tol, double* D, double* P, double* p_ev, char* gws,
+               const int64_t* wsoff, size_t smem, int32_t* info) {
+    RepairParams rp{};
+    rp.zones = s->d_net_zones;
+    rp.nodes = s->d_net_nodes;
+    rp.res = s->d_net_res;
+    rp.cumr = s->d_net_cumr;
+    rp.zone_worst = s->d_net_zw;
+    rp.load = s->d_load;
+    rp.rating = s->d_rating;
+    rp.cost = s->d_cost;
+    rp.start = s->d_start;
+    rp.end = s->d_end;
+    rp.n_min = s->d_nmin;
+    rp.D = D;
+    rp.P = P;
+    rp.p_ev = p_ev;
+    rp.gws = gws;
+    rp.ws_off = wsoff;
+    rp.info = info;
+    rp.T = s->T;
+    rp.u = u;
+    rp.row_tol = row_tol;
+    CU(launch_repair(rp, s->nf, smem, s->sU));
+    return REVS_OK;
+}
+
 void net_location(const NetArg& a, int T, int32_t* zone, int32_t* index, int32_t* step) {
     const bool none = a.loc == INT64_MAX;      // no candidate (no residence at all)
     *zone = none ? -1 : a.zone;
@@ -2087,11 +2155,14 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
                        const double* scale, double* voltage, double* loading, double* zone_worst,
                        revs_network_summary* summary) {
     if (!s) return fail(REVS_ERR_ARG, "null solver");
-    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST && source != REVS_NET_REPAIRED)
-        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST or REVS_NET_REPAIRED)",
-                    source);
+    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST && source != REVS_NET_REPAIRED &&
+        source != REVS_NET_CENTRAL)
+        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED "
+                    "or REVS_NET_CENTRAL)", source);
     if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
-    if (source != REVS_NET_HOST && s->k == 0)
+    if (source == REVS_NET_CENTRAL && !s->cen_valid)
+        return fail(REVS_ERR_ARG, "REVS_NET_CENTRAL: revs_central_bracket has not run since the homes, tariff or trees were set");
+    if (source != REVS_NET_HOST && source != REVS_NET_CENTRAL && s->k == 0)
         return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check",
                     source == REVS_NET_SCHEDULE ? "schedule" : source == REVS_NET_ESTIMATE ? "estimate" : "repaired schedule");
     if (source == REVS_NET_REPAIRED && !s->rep_valid)
@@ -2105,7 +2176,8 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
     const int T = s->T;
     const size_t out_elems = (size_t)h.total_nodes * T;
     int64_t launches = 0;
-    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->d_rep_P : s->d_pest;
+    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->d_rep_P
+                        : source == REVS_NET_CENTRAL ? s->d_cen_P1 : s->d_pest;
     if (source == REVS_NET_HOST) {
         if (!s->d_net_P) CU(dalloc(&s->d_net_P, (size_t)s->Hp * T));
         if ((rc = h2d_homes(s, s->d_net_P, P, T))) return rc;
@@ -2159,22 +2231,7 @@ int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_t
     const int T = s->T;
     const size_t HT = (size_t)s->Hp * T;
     if (!s->d_rep_P) {
-        // the zones' state: shared memory up to kRepairSmemMaxN residences, else a block of the global scratch
-        std::vector<int64_t> off(s->nf);
-        int64_t g = 0;
-        for (int f = 0; f < s->nf; ++f) {
-            const size_t b = repair_ws_bytes(s->feeders[f].n, T);
-            if (s->feeders[f].n > kRepairSmemMaxN) {
-                off[f] = g;
-                g += (int64_t)b;
-            } else {
-                off[f] = -1;
-                s->rep_smem = std::max(s->rep_smem, b);
-            }
-        }
-        CU(dalloc(&s->d_rep_wsoff, (size_t)s->nf));
-        CU(cudaMemcpy(s->d_rep_wsoff, off.data(), sizeof(int64_t) * s->nf, cudaMemcpyHostToDevice));
-        CU(dalloc(&s->d_rep_gws, (size_t)g));
+        if ((rc = repair_scratch(s, &s->d_rep_wsoff, &s->d_rep_gws, &s->rep_smem))) return rc;
         CU(dalloc(&s->d_rep_info, (size_t)3 * s->nf));
         CU(dalloc(&s->d_rep_D, HT));
         CU(dalloc(&s->d_rep_pev, HT));
@@ -2187,28 +2244,9 @@ int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_t
     CU(cudaMemcpyAsync(s->d_rep_pev, s->d_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
     // the drops of the schedule at every residence, and which zones violate a row
     if ((rc = net_run(s, s->d_psch[s->cur], v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_rep_D, &launches))) return rc;
-    RepairParams rp{};
-    rp.zones = s->d_net_zones;
-    rp.nodes = s->d_net_nodes;
-    rp.res = s->d_net_res;
-    rp.cumr = s->d_net_cumr;
-    rp.zone_worst = s->d_net_zw;
-    rp.load = s->d_load;
-    rp.rating = s->d_rating;
-    rp.cost = s->d_cost;
-    rp.start = s->d_start;
-    rp.end = s->d_end;
-    rp.n_min = s->d_nmin;
-    rp.D = s->d_rep_D;
-    rp.P = s->d_rep_P;
-    rp.p_ev = s->d_rep_pev;
-    rp.gws = s->d_rep_gws;
-    rp.ws_off = s->d_rep_wsoff;
-    rp.info = s->d_rep_info;
-    rp.T = T;
-    rp.u = u;
-    rp.row_tol = row_tol;
-    CU(launch_repair(rp, s->nf, s->rep_smem, s->sU));
+    if ((rc = run_repair(s, u, row_tol, s->d_rep_D, s->d_rep_P, s->d_rep_pev, s->d_rep_gws, s->d_rep_wsoff, s->rep_smem,
+                         s->d_rep_info)))
+        return rc;
     launches += s->nf > 0;
     if (hour_mask && s->H > 0) {
         unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
@@ -2225,6 +2263,153 @@ int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_t
     CU(cudaStreamSynchronize(s->sU));
     s->stats.kernel_launches += launches;
     s->rep_valid = true;
+    return REVS_OK;
+}
+
+int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_tol, int iters, double* P_out,
+                         uint64_t* hour_mask, int mask_words, double* zone_bounds, int32_t* zone_info) {
+    if (!s) return fail(REVS_ERR_ARG, "null solver");
+    if (!s->homes_set) return fail(REVS_ERR_ARG, "revs_set_homes has not been called");
+    if (!s->tariff_set) return fail(REVS_ERR_ARG, "revs_set_tariff has not been called");
+    if (iters < 0) return fail(REVS_ERR_ARG, "iters must be >= 0");
+    if (hour_mask && mask_words != (s->T + 63) / 64) return fail(REVS_ERR_ARG, "mask_words must be ceil(T / 64) = %d", (s->T + 63) / 64);
+    const double v2 = vset * vset, u = vhigh * vhigh - v2;
+    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
+    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
+    CU(cudaSetDevice(s->device));
+    int rc = net_prepare(s);
+    if (rc) return rc;
+    const int T = s->T, nf = s->nf;
+    const size_t HT = (size_t)s->Hp * T;
+    if (!s->d_cen_y) {
+        if ((rc = repair_scratch(s, &s->d_cen_wsoff, &s->d_cen_gws, &s->cen_smem))) return rc;
+        double** hts[] = {&s->d_cen_y, &s->d_cen_yb, &s->d_cen_P, &s->d_cen_pev, &s->d_cen_D, &s->d_cen_Drep,
+                          &s->d_cen_P1, &s->d_cen_pev1, &s->d_cen_P2, &s->d_cen_pev2};
+        for (double** b : hts) CU(dalloc(b, HT));
+        CU(dalloc(&s->d_cen_sums, (size_t)3 * nf));
+        CU(dalloc(&s->d_cen_bounds, (size_t)2 * nf));
+        CU(dalloc(&s->d_cen_info, (size_t)9 * nf));
+        CU(dalloc(&s->d_cen_state, (size_t)nf));
+        CU(dalloc(&s->d_cen_flag, (size_t)1));
+        std::vector<int> hz((size_t)s->Hp, 0);
+        for (int f = 0; f < nf; ++f)
+            for (int j = 0; j < s->feeders[f].n; ++j) hz[(size_t)s->feeders[f].off + j] = f;
+        CU(dalloc(&s->d_cen_hzone, hz.size()));
+        CU(cudaMemcpy(s->d_cen_hzone, hz.data(), sizeof(int) * hz.size(), cudaMemcpyHostToDevice));
+        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
+    }
+    s->cen_valid = false;
+    int64_t launches = 0;
+    double *cost1 = s->d_cen_sums, *cost2 = cost1 + nf, *cmax = cost2 + nf;
+    int32_t *info1 = s->d_cen_info, *info2 = info1 + 3 * nf, *info = info2 + 3 * nf;
+    CU(cudaMemsetAsync(s->d_cen_y, 0, HT * sizeof(double), s->sU));
+    CU(cudaMemsetAsync(s->d_cen_yb, 0, HT * sizeof(double), s->sU));
+    CU(cudaMemsetAsync(s->d_cen_flag, 0, sizeof(int), s->sU));
+    CenSelectParams sp{};
+    sp.zones = s->d_net_zones;
+    sp.hzone = s->d_cen_hzone;
+    sp.load = s->d_load;
+    sp.rating = s->d_rating;
+    sp.cost = s->d_cost;
+    sp.has_ev = s->d_has_ev;
+    sp.start = s->d_start;
+    sp.end = s->d_end;
+    sp.n_min = s->d_nmin;
+    sp.n_max = s->d_nmax;
+    sp.P = s->d_cen_P;
+    sp.p_ev = s->d_cen_pev;
+    sp.infeasible = s->d_cen_flag;
+    sp.Hp = s->Hp;
+    sp.T = T;
+    // C_max: the most expensive SOC-feasible schedule
+    sp.most_expensive = 1;
+    CU(launch_central_select(sp, s->sU));
+    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P, T, cmax, s->sU));
+    // first start: the repair of e*(0)
+    sp.most_expensive = 0;
+    CU(launch_central_select(sp, s->sU));
+    if ((rc = net_run(s, s->d_cen_P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+    CU(cudaMemcpyAsync(s->d_cen_Drep, s->d_cen_D, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(s->d_cen_P1, s->d_cen_P, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(s->d_cen_pev1, s->d_cen_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    if ((rc = run_repair(s, u, row_tol, s->d_cen_Drep, s->d_cen_P1, s->d_cen_pev1, s->d_cen_gws, s->d_cen_wsoff,
+                         s->cen_smem, info1)))
+        return rc;
+    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P1, T, cost1, s->sU));
+    // the ascent (a host loop: every evaluation is two network checks, the selection and the ascent kernel)
+    CenAscentParams ap{};
+    ap.zones = s->d_net_zones;
+    ap.cost = s->d_cost;
+    ap.P = s->d_cen_P;
+    ap.D = s->d_cen_D;
+    ap.y = s->d_cen_y;
+    ap.ybest = s->d_cen_yb;
+    ap.cost1 = cost1;
+    ap.cmax = cmax;
+    ap.info1 = info1;
+    ap.state = s->d_cen_state;
+    ap.iters = iters;
+    ap.T = T;
+    ap.u = u;
+    sp.ry = s->d_cen_D;
+    for (int k = 0; k <= iters; ++k) {
+        if (k > 0) {
+            if ((rc = net_run(s, s->d_cen_y, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+            CU(launch_central_select(sp, s->sU));
+            if ((rc = net_run(s, s->d_cen_P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+            launches += 1;
+        }
+        ap.k = k;
+        CU(launch_central_ascent(ap, nf, s->sU));
+        launches += nf > 0;
+    }
+    // second start: the repair of e*(y_best)
+    if ((rc = net_run(s, s->d_cen_yb, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+    sp.P = s->d_cen_P2;
+    sp.p_ev = s->d_cen_pev2;
+    CU(launch_central_select(sp, s->sU));
+    if ((rc = net_run(s, s->d_cen_P2, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_Drep, &launches))) return rc;
+    if ((rc = run_repair(s, u, row_tol, s->d_cen_Drep, s->d_cen_P2, s->d_cen_pev2, s->d_cen_gws, s->d_cen_wsoff,
+                         s->cen_smem, info2)))
+        return rc;
+    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P2, T, cost2, s->sU));
+    CenFinalParams fp{};
+    fp.zones = s->d_net_zones;
+    fp.state = s->d_cen_state;
+    fp.cost1 = cost1;
+    fp.cost2 = cost2;
+    fp.cmax = cmax;
+    fp.info1 = info1;
+    fp.info2 = info2;
+    fp.P1 = s->d_cen_P1;
+    fp.p_ev1 = s->d_cen_pev1;
+    fp.P2 = s->d_cen_P2;
+    fp.p_ev2 = s->d_cen_pev2;
+    fp.bounds = s->d_cen_bounds;
+    fp.info = info;
+    fp.T = T;
+    CU(launch_central_final(fp, nf, s->sU));
+    launches += (s->H > 0 ? 3 : 0) + (nf > 0 ? 6 : 0);     // selections; costs, repairs, final
+    int infeasible = 0;
+    CU(cudaMemcpyAsync(&infeasible, s->d_cen_flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->stats.kernel_launches += launches;
+    if (infeasible) return fail(REVS_ERR_INFEASIBLE, "a home's SOC target needs more hours than its plug-in window has");
+    if (hour_mask && s->H > 0) {
+        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
+        CU(launch_hour_mask(s->d_cen_pev1, s->d_hmap, s->H, T, d_mask, s->sU));
+        ++s->stats.kernel_launches;
+        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
+    }
+    if (P_out && s->H > 0) {
+        if ((rc = d2h_homes(s, P_out, s->d_cen_P1, T))) return rc;
+        ++s->stats.kernel_launches;
+    }
+    if (zone_bounds && nf > 0)
+        CU(cudaMemcpyAsync(zone_bounds, s->d_cen_bounds, sizeof(double) * 2 * nf, cudaMemcpyDeviceToHost, s->sU));
+    if (zone_info && nf > 0) CU(cudaMemcpyAsync(zone_info, info, sizeof(int32_t) * 3 * nf, cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->cen_valid = true;
     return REVS_OK;
 }
 

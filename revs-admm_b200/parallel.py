@@ -398,6 +398,16 @@ class PipelinedSolver:
                                   mask=np.concatenate([r["mask"] for r in res]) if mask else None,
                                   zone_info=np.concatenate([r["zone_info"] for r in res])))
 
+    def central_bracket(self, schedule=True, mask=False, **kw):
+        """Solver.central_bracket over all pipelines at once: schedules, masks, zone_bounds and zone_info concatenated in
+        zone order, totals recomputed -- the bytes of a single solver over the same zones."""
+        from ._cabi import central_totals
+        res = self._each(lambda k: self.parts[k].central_bracket(schedule=schedule, mask=mask, **kw))
+        return central_totals(dict(P_sch=np.concatenate([r["P_sch"] for r in res]) if schedule else None,
+                                   mask=np.concatenate([r["mask"] for r in res]) if mask else None,
+                                   zone_bounds=np.concatenate([r["zone_bounds"] for r in res]),
+                                   zone_info=np.concatenate([r["zone_info"] for r in res])))
+
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
         pipeline (they run side by side), residuals are recombined from the per-pipeline norms."""
