@@ -24,6 +24,7 @@
  *   revs_network_check                            drawing.py:29-78    the same for every zone at once
  *   revs_repair_schedule                          no reference counterpart (a voltage-feasible binary schedule)
  *   revs_central_bracket                          lpsolver.py:463-502 solve_central(), bracketed per zone
+ *   revs_certify_infeasible                       lpsolver.py:463-502 solve_central(), zones proved infeasible
  *   revs_get_results / revs_get_schedule(_ld)     lpsolver.py:289-290 return diff,P_sch,S,C
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
@@ -272,6 +273,36 @@ int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_t
 int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_tol, int iters, double* P_out,
                          uint64_t* hour_mask, int mask_words, double* zone_bounds, int32_t* zone_info);
 #define REVS_NET_CENTRAL 4    /* the kept schedule of the last revs_central_bracket                    */
+
+/* Certificate of voltage infeasibility, zone by zone on the device: a proof that no binary schedule keeps every home's
+ * SOC window (n_min charging hours at least) and plug-in window and the voltage rows (R P)_i,t - u <= row_tol, or "no
+ * proof found".  It covers the zones the Lagrangian bound of revs_central_bracket cannot: that bound equals the LP
+ * relaxation's, and a zone whose LP relaxation meets the rows can still have no binary schedule, because a home draws
+ * its full rating in every hour it charges.  Needs the homes and the tree of every zone; no tariff or ADMM run.
+ *
+ * The rule, with u = vhigh^2 - vset^2, D0 = R load at the residences (the network check's drops of the base load),
+ * a_h(i) = rating_h R[i,h] (R[i,h] = 2 cumr at the lowest common ancestor of the two residences' nodes), the homes
+ * that count = the EV homes with n_min > 0, and a set of charges fitting row (i,t) when (D0[i,t] + s) - u <=
+ * row_tol + 1e-12, s the sum of their coefficients (round-to-nearest; the 1e-12 pu^2 margin resolves every rounding
+ * in favour of "fits", so no certificate comes from rounding):
+ *   kind 1: some row has D0[i,t] - u > row_tol + 1e-12 (the base load alone violates it); witness: the worst such row,
+ *           ties to the lowest residence, then the lowest step;
+ *   kind 2: for a residence i, S_k = the k homes of largest a_h(i) (ties to the lowest home), k = 1..K,
+ *           K = min(32, homes that count); m_t(k) = the largest j such that the j smallest coefficients of the members
+ *           of S_k whose window contains t fit row (i,t), added in ascending order; cap_k = sum_t m_t(k),
+ *           need_k = sum of n_min over S_k.  cap_k < need_k proves the zone infeasible (R >= 0 and rating >= 0: charges
+ *           outside S_k and at other rows only use up slack).  Witness: the (i, k) of the largest need_k - cap_k, ties
+ *           to the lowest residence, then the lowest k.
+ * A zone of kind 1 reports kind 1.  zone_cert [n_feeders, 4] int32 {kind 0 (no proof) / 1 / 2, residence (local index
+ * in the zone, -1 for kind 0), step (kind 1) or k (kind 2) (-1 for kind 0), need_k - cap_k (kind 2, else 0)} and
+ * n_certified (zones of kind 1 or 2) may each be NULL.  Every reduction is an integer or total-order maximum: two calls
+ * give the same bytes, and a zone's result does not depend on the other zones.
+ * REVS_ERR_ARG: homes not set, a zone without tree (named), not vset < vhigh, row_tol < 0 or NaN, an EV home with a
+ * negative or non-finite rating.  REVS_ERR_INFEASIBLE: a home whose n_min exceeds its plug-in window (or n_max), as in
+ * revs_central_bracket.  Synchronous on the utility stream; adds its launches to revs_stats.kernel_launches and
+ * changes no other state (the schedules of revs_repair_schedule and revs_central_bracket stay checkable). */
+int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double row_tol, int32_t* zone_cert,
+                            int* n_certified);
 
 /* The same check with the ROWS PARTITIONED over the GPUs of one box (one process per GPU, every process holds the
  * feeder's tree; BASELINE north_star: "the sensitivity contraction is row-partitioned"): every rank builds and

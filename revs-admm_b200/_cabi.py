@@ -93,6 +93,8 @@ SIGNATURES = {
                               C.POINTER(C.c_int32)], C.c_int),
     "revs_central_bracket": ([_P, C.c_double, C.c_double, C.c_double, C.c_int, _D, C.POINTER(C.c_uint64), C.c_int, _D,
                               C.POINTER(C.c_int32)], C.c_int),
+    "revs_certify_infeasible": ([_P, C.c_double, C.c_double, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int)],
+                                C.c_int),
 }
 
 _lib = None
@@ -194,6 +196,27 @@ def central_totals(r):
     r.update(lb=float(b[:, 0].sum()), lb_bracketed=lbb, ub=ub, gap=(ub - lbb) / abs(lbb) if lbb else 0.0,
              zones_status=[int((st == k).sum()) for k in range(4)])
     return r
+
+
+def certify_totals(r):
+    """Add the counts of zone_cert to a certify_infeasible result: zones_kind (zones of kind 0, 1, 2) and certified
+    (zones of kind 1 or 2)."""
+    kind = r["zone_cert"][:, 0]
+    r.update(zones_kind=[int((kind == k).sum()) for k in range(3)], certified=int((kind > 0).sum()))
+    return r
+
+
+def central_status(zone_info, zone_cert):
+    """The status of central_bracket's zone_info with the zones that certify_infeasible proves infeasible: 2 (no feasible
+    schedule found) becomes 3 (certified infeasible) where zone_cert has a certificate.  Raises ValueError when a zone
+    of status 0 or 1 (a voltage-feasible schedule is known) is certified: one of the two results would be wrong."""
+    st = np.array(np.asarray(zone_info)[:, 0], dtype=np.int32)
+    cert = np.asarray(zone_cert)[:, 0] > 0
+    bad = np.nonzero(cert & (st <= 1))[0]
+    if bad.size:
+        raise ValueError(f"zones {bad.tolist()} have a voltage-feasible schedule and a certificate of infeasibility")
+    st[cert] = 3
+    return st
 
 
 class Solver:
@@ -444,6 +467,17 @@ class Solver:
                                              None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W, _dp(B),
                                              Z.ctypes.data_as(C.POINTER(C.c_int32))))
         return central_totals(dict(P_sch=P, mask=M, zone_bounds=B, zone_info=Z))
+
+    def certify_infeasible(self, vset, vhigh, row_tol=1e-9):
+        """Certificate of voltage infeasibility zone by zone on the device (include/revs_admm.h:
+        revs_certify_infeasible): a proof that no binary schedule keeps the SOC windows, plug-in windows and voltage
+        rows, from the homes and trees alone.  Returns dict(zone_cert=[zones, 4] int32 {kind 0 no proof / 1 base load /
+        2 counting, residence (local), step (kind 1) or k (kind 2), need - cap (kind 2)}) with the counts of
+        certify_totals.  Nothing of an ADMM run or of central_bracket is read or changed."""
+        Z = np.zeros((self.nf, 4), dtype=np.int32)
+        _check(self.lib.revs_certify_infeasible(self._h, vset, vhigh, row_tol, Z.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                None))
+        return certify_totals(dict(zone_cert=Z))
 
     # ---- the same check with the rows partitioned over the GPUs of the box; the all-gather of the result is fused
     # into the epilogue of the contraction kernel (peer-memory stores, include/revs_admm.h: revs_gather_*)

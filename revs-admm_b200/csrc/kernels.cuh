@@ -324,6 +324,17 @@ struct NetParams {
     int T;
     double v2, u, low, row_tol;   // vset^2, vhigh^2 - vset^2, vset^2 - vlow^2, tolerance of the row count
 };
+// R[i,h] of two residences on the breadth-first positions a, b of their nodes: 2 cumr at the lowest common ancestor
+// (0 when they hang on different roots).  A larger position is never above a smaller one, so moving the larger one up
+// never passes the ancestor.
+__device__ __forceinline__ double lca_r(const NetNode* __restrict__ nd, const double* __restrict__ cumr, int a, int b) {
+    while (a != b) {
+        if (a > b) a = nd[a].parent;
+        else b = nd[b].parent;
+        if (a < 0 || b < 0) return 0.0;
+    }
+    return 2.0 * cumr[nd[a].node];
+}
 struct NetHost {                  // host side of the arrays above, built once per set of trees
     std::vector<NetZone> zones;
     std::vector<NetNode> nodes;
@@ -409,5 +420,27 @@ cudaError_t launch_central_ascent(const CenAscentParams& P, int n_zones, cudaStr
 cudaError_t launch_central_cost(const NetZone* zones, int n_zones, const double* cost, const double* P, int T,
                                 double* out, cudaStream_t s);
 cudaError_t launch_central_final(const CenFinalParams& P, int n_zones, cudaStream_t s);
+
+// ---- certify.cu: certificate of voltage infeasibility per zone (base load, counting over the top-K homes of a row)
+constexpr int kCertTopK = 32;     // homes of largest coefficient per residence row that the counting rule looks at
+struct CertParams {
+    const NetZone* zones;         // the network check's breadth-first arrays
+    const NetNode* nodes;
+    const int* res;
+    const double* cumr;           // [total nodes], zone z at zones[z].out_row
+    const int* hzone;             // [Hp] zone of every padded home row, -1: padding
+    const double* D;              // zone blocks [T][n]: R load at the residences (NetParams::drop)
+    const double* rating;
+    const uint8_t* has_ev;
+    const int *start, *end, *n_min, *n_max;
+    int* hpos;                    // [Hp] out: breadth-first position of every residence's node
+    unsigned long long* key;      // [zones] packed witness of kind 2 (atomicMax)
+    int32_t* cert;                // [zones][4] out: kind, residence, k or step, need - cap
+    int* flag;                    // out: |1 a home's n_min exceeds its window or n_max, |2 a non-finite or negative rating
+    int64_t Hp;
+    int T;
+    double u, thr;                // vhigh^2 - vset^2, row_tol + 1e-12
+};
+cudaError_t launch_certify(const CertParams& P, int n_zones, cudaStream_t s);
 
 }  // namespace revs

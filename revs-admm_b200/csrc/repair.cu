@@ -62,17 +62,6 @@ __device__ __forceinline__ RepArg rep_argmax(double v, int i, RepArg* slot) {
     return r;
 }
 
-// 2 cumr at the lowest common ancestor of two breadth-first positions (0 when they hang on different roots).  A
-// larger position is never above a smaller one, so moving the larger one up never passes the ancestor.
-__device__ __forceinline__ double rep_r(const NetNode* __restrict__ nd, const double* __restrict__ cumr, int a, int b) {
-    while (a != b) {
-        if (a > b) a = nd[a].parent;
-        else b = nd[b].parent;
-        if (a < 0 || b < 0) return 0.0;
-    }
-    return 2.0 * cumr[nd[a].node];
-}
-
 // The zone's state, in shared memory or in the global scratch (layout of repair_ws_bytes).
 struct RepWs {
     double *wv, *rel, *col;   // [T] worst excess of every step, [n] relief of the candidates, [n] R column * rating
@@ -187,7 +176,7 @@ __global__ void __launch_bounds__(kRepThreads, 2) repair_kernel(RepairParams p) 
         const int qi = w.hpos[is];
         for (int h = threadIdx.x; h < n; h += blockDim.x)
             w.rel[h] = (w.bits[h * W + (ts >> 6)] >> (ts & 63)) & 1ull
-                           ? __dmul_rn(p.rating[h0 + h], rep_r(nd, cumr, qi, w.hpos[h])) : -INFINITY;
+                           ? __dmul_rn(p.rating[h0 + h], lca_r(nd, cumr, qi, w.hpos[h])) : -INFINITY;
         __syncthreads();
         // 3. candidates in order of relief: the first that can drop or move
         int act = 0, tp = -1, hc = -1;
@@ -201,7 +190,7 @@ __global__ void __launch_bounds__(kRepThreads, 2) repair_kernel(RepairParams p) 
             hc = c.i;
             const double rt = p.rating[h0 + hc];
             const int qh = w.hpos[hc];
-            for (int i = threadIdx.x; i < n; i += blockDim.x) w.col[i] = __dmul_rn(rt, rep_r(nd, cumr, w.hpos[i], qh));
+            for (int i = threadIdx.x; i < n; i += blockDim.x) w.col[i] = __dmul_rn(rt, lca_r(nd, cumr, w.hpos[i], qh));
             int cnt = 0;
             for (int k = 0; k < W; ++k) cnt += __popcll(w.bits[hc * W + k]);
             if (cnt > p.n_min[h0 + hc]) {

@@ -216,6 +216,11 @@ struct revs_solver {
     char* d_cen_gws = nullptr;
     int64_t* d_cen_wsoff = nullptr;
     size_t cen_smem = 0;
+    // certificate of voltage infeasibility (revs_certify_infeasible, certify.cu): scratch only, no result is kept
+    double* d_crt_D = nullptr;                                // [Hp * T] R load at the residences
+    int *d_crt_hzone = nullptr, *d_crt_hpos = nullptr, *d_crt_flag = nullptr;
+    int32_t* d_crt_cert = nullptr;                            // [zones][4]
+    unsigned long long* d_crt_key = nullptr;                  // [zones]
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -922,7 +927,8 @@ void free_all(revs_solver* s) {
                     s->d_rep_gws, s->d_rep_wsoff, s->d_rep_info, s->d_cen_y, s->d_cen_yb, s->d_cen_P, s->d_cen_pev,
                     s->d_cen_D, s->d_cen_Drep, s->d_cen_P1, s->d_cen_pev1, s->d_cen_P2, s->d_cen_pev2, s->d_cen_sums,
                     s->d_cen_bounds, s->d_cen_info, s->d_cen_state, s->d_cen_hzone, s->d_cen_flag, s->d_cen_gws,
-                    s->d_cen_wsoff};
+                    s->d_cen_wsoff, s->d_crt_D, s->d_crt_hzone, s->d_crt_hpos, s->d_crt_flag, s->d_crt_cert,
+                    s->d_crt_key};
     for (int r = 0; r < kMaxPeers; ++r)
         if (s->peer_box[r] && s->peer_box[r] != s->d_mailbox) cudaIpcCloseMemHandle(s->peer_box[r]);
     for (int r = 0; r < kGatherMaxPeers; ++r)
@@ -2410,6 +2416,74 @@ int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_t
     if (zone_info && nf > 0) CU(cudaMemcpyAsync(zone_info, info, sizeof(int32_t) * 3 * nf, cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->cen_valid = true;
+    return REVS_OK;
+}
+
+int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double row_tol, int32_t* zone_cert,
+                            int* n_certified) {
+    if (!s) return fail(REVS_ERR_ARG, "null solver");
+    if (!s->homes_set) return fail(REVS_ERR_ARG, "revs_set_homes has not been called");
+    const double v2 = vset * vset, u = vhigh * vhigh - v2;
+    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
+    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
+    CU(cudaSetDevice(s->device));
+    int rc = net_prepare(s);
+    if (rc) return rc;
+    const int T = s->T, nf = s->nf;
+    if (!s->d_crt_D) {
+        CU(dalloc(&s->d_crt_D, (size_t)s->Hp * T));
+        CU(dalloc(&s->d_crt_hpos, (size_t)s->Hp));
+        CU(dalloc(&s->d_crt_cert, (size_t)4 * nf));
+        CU(dalloc(&s->d_crt_key, (size_t)nf));
+        CU(dalloc(&s->d_crt_flag, (size_t)1));
+        std::vector<int> hz((size_t)s->Hp, -1);
+        for (int f = 0; f < nf; ++f)
+            for (int j = 0; j < s->feeders[f].n; ++j) hz[(size_t)s->feeders[f].off + j] = f;
+        CU(dalloc(&s->d_crt_hzone, hz.size()));
+        CU(cudaMemcpy(s->d_crt_hzone, hz.data(), sizeof(int) * hz.size(), cudaMemcpyHostToDevice));
+        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
+    }
+    int64_t launches = 0;
+    CU(cudaMemsetAsync(s->d_crt_flag, 0, sizeof(int), s->sU));
+    // the drops of the base load at every residence
+    if ((rc = net_run(s, s->d_load, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_crt_D, &launches))) return rc;
+    CertParams cp{};
+    cp.zones = s->d_net_zones;
+    cp.nodes = s->d_net_nodes;
+    cp.res = s->d_net_res;
+    cp.cumr = s->d_net_cumr;
+    cp.hzone = s->d_crt_hzone;
+    cp.D = s->d_crt_D;
+    cp.rating = s->d_rating;
+    cp.has_ev = s->d_has_ev;
+    cp.start = s->d_start;
+    cp.end = s->d_end;
+    cp.n_min = s->d_nmin;
+    cp.n_max = s->d_nmax;
+    cp.hpos = s->d_crt_hpos;
+    cp.key = s->d_crt_key;
+    cp.cert = s->d_crt_cert;
+    cp.flag = s->d_crt_flag;
+    cp.Hp = s->Hp;
+    cp.T = T;
+    cp.u = u;
+    cp.thr = row_tol + 1e-12;
+    CU(launch_certify(cp, nf, s->sU));
+    launches += nf > 0 ? 3 : 0;
+    int flag = 0;
+    std::vector<int32_t> cert((size_t)4 * nf);
+    CU(cudaMemcpyAsync(&flag, s->d_crt_flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
+    if (nf > 0) CU(cudaMemcpyAsync(cert.data(), s->d_crt_cert, sizeof(int32_t) * cert.size(), cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->stats.kernel_launches += launches;
+    if (flag & 2) return fail(REVS_ERR_ARG, "an EV home has a negative or non-finite rating: the certificate needs rating >= 0");
+    if (flag & 1) return fail(REVS_ERR_INFEASIBLE, "a home's SOC target needs more hours than its plug-in window has");
+    if (zone_cert && nf > 0) memcpy(zone_cert, cert.data(), sizeof(int32_t) * cert.size());
+    if (n_certified) {
+        int c = 0;
+        for (int f = 0; f < nf; ++f) c += cert[4 * (size_t)f] != 0;
+        *n_certified = c;
+    }
     return REVS_OK;
 }
 

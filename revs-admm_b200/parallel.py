@@ -408,6 +408,13 @@ class PipelinedSolver:
                                    zone_bounds=np.concatenate([r["zone_bounds"] for r in res]),
                                    zone_info=np.concatenate([r["zone_info"] for r in res])))
 
+    def certify_infeasible(self, *args, **kw):
+        """Solver.certify_infeasible over all pipelines at once: zone_cert concatenated in zone order, counts
+        recomputed -- the bytes of a single solver over the same zones."""
+        from ._cabi import certify_totals
+        res = self._each(lambda k: self.parts[k].certify_infeasible(*args, **kw))
+        return certify_totals(dict(zone_cert=np.concatenate([r["zone_cert"] for r in res])))
+
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
         pipeline (they run side by side), residuals are recombined from the per-pipeline norms."""
