@@ -433,6 +433,14 @@ class Solver:
                                            _dp(Z), C.byref(summ)))
         return dict(summary=summ.as_dict(), voltage=V, loading=L, zone_worst=Z)
 
+    def _schedule_out(self, schedule, mask):
+        """The host buffers of a tool's schedule, each None unless asked for: P_sch [H, T] and the charging bits
+        [H, ceil(T/64)] uint64, with the (P_out, hour_mask, mask_words) arguments of the library call."""
+        W = (self.T + 63) // 64
+        P = np.empty((self.H, self.T)) if schedule else None
+        M = np.empty((self.H, W), dtype=np.uint64) if mask else None
+        return P, M, (_dp(P), None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W)
+
     def repair_schedule(self, vset=1.0, vhigh=1.05, row_tol=1e-9, schedule=True, mask=False):
         """Greedy voltage repair of the last ADMM run's charging decisions, zone by zone on the device
         (include/revs_admm.h: revs_repair_schedule; a heuristic, a zone may be left with violated rows).  Returns
@@ -440,13 +448,9 @@ class Solver:
         zone_info=[zones, 3] int32 {status 0 untouched / 1 repaired / 2 violations left, hours moved, hours dropped},
         moves, drops, zones_violated, zones_repaired, zones_left).  P_sch, P_est and the results of the run stay as
         they are; expand_schedule(mask, ...) gives the repaired P_ev and SOC."""
-        H, T = self.H, self.T
-        W = (T + 63) // 64
-        P = np.empty((H, T)) if schedule else None
-        M = np.empty((H, W), dtype=np.uint64) if mask else None
+        P, M, args = self._schedule_out(schedule, mask)
         Z = np.zeros((self.nf, 3), dtype=np.int32)
-        _check(self.lib.revs_repair_schedule(self._h, vset, vhigh, row_tol, _dp(P),
-                                             None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W,
+        _check(self.lib.revs_repair_schedule(self._h, vset, vhigh, row_tol, *args,
                                              Z.ctypes.data_as(C.POINTER(C.c_int32))))
         return repair_totals(dict(P_sch=P, mask=M, zone_info=Z))
 
@@ -457,14 +461,10 @@ class Solver:
         None, zone_bounds=[zones, 2] {LB, UB}, zone_info=[zones, 3] int32 {status 0 optimal / 1 bracketed / 2 no
         feasible schedule found / 3 certified infeasible, ascent steps, repair moves + drops of the kept start}) and
         the totals of central_totals.  Nothing of an ADMM run is read or changed."""
-        H, T = self.H, self.T
-        W = (T + 63) // 64
-        P = np.empty((H, T)) if schedule else None
-        M = np.empty((H, W), dtype=np.uint64) if mask else None
+        P, M, args = self._schedule_out(schedule, mask)
         B = np.zeros((self.nf, 2))
         Z = np.zeros((self.nf, 3), dtype=np.int32)
-        _check(self.lib.revs_central_bracket(self._h, vset, vhigh, row_tol, int(iters), _dp(P),
-                                             None if M is None else M.ctypes.data_as(C.POINTER(C.c_uint64)), W, _dp(B),
+        _check(self.lib.revs_central_bracket(self._h, vset, vhigh, row_tol, int(iters), *args, _dp(B),
                                              Z.ctypes.data_as(C.POINTER(C.c_int32))))
         return central_totals(dict(P_sch=P, mask=M, zone_bounds=B, zone_info=Z))
 

@@ -379,7 +379,7 @@ cudaError_t launch_repair(const RepairParams& P, int n_zones, size_t smem, cudaS
 // ---- central.cu: bracket of the centralized optimum per zone (priced selections, Lagrangian ascent, two repairs)
 struct CenSelectParams {          // one warp per home: e*(y), or the most expensive SOC-feasible hours
     const NetZone* zones;
-    const int* hzone;             // [Hp] zone of every home (EV homes only are read)
+    const int* hzone;             // [Hp] zone of every home, -1: padding (EV homes only are read)
     const double* ry;             // zone blocks [T][n]: R y at the residences (NetParams::drop), or null (y = 0)
     const double *load, *rating, *cost;
     const uint8_t* has_ev;

@@ -87,6 +87,79 @@ struct Tree {
     bool pooled = false;     // sub-range of the solver's tree pool (revs_set_feeder_trees)
 };
 
+template <class Tp>
+cudaError_t dalloc(Tp** p, size_t n) {
+    cudaError_t e = cudaMalloc((void**)p, (n ? n : 1) * sizeof(Tp));
+    if (e == cudaSuccess) e = cudaMemset(*p, 0, (n ? n : 1) * sizeof(Tp));
+    return e;
+}
+
+// One device array with one owner (move-only): freed when it is reallocated, replaced or destroyed.
+template <class Tp>
+struct DevArray {
+    Tp* p = nullptr;
+    DevArray& operator=(DevArray&& o) noexcept {
+        std::swap(p, o.p);    // o frees the previous array
+        return *this;
+    }
+    ~DevArray() { if (p) cudaFree(p); }
+    cudaError_t alloc(size_t n) {    // n elements, zeroed when it returns
+        *this = DevArray();
+        cudaError_t e = dalloc(&p, n);
+        // dalloc zeroes on the legacy stream, which does not order with the non-blocking streams of the kernels
+        return e == cudaSuccess ? cudaStreamSynchronize(cudaStreamLegacy) : e;
+    }
+    cudaError_t upload(const std::vector<Tp>& v) {    // alloc(v.size()) holding v
+        cudaError_t e = alloc(v.size());
+        if (e == cudaSuccess && !v.empty()) e = cudaMemcpy(p, v.data(), sizeof(Tp) * v.size(), cudaMemcpyHostToDevice);
+        return e;
+    }
+    operator Tp*() const { return p; }
+};
+
+// The breadth-first zone arrays of the network tools (network_check.cu) and revs_network_check's arrays sized by the
+// total node count: built by net_prepare from the trees, replaced as a whole when the trees change.
+struct NetArrays {
+    NetHost h;
+    DevArray<NetZone> zones;
+    DevArray<NetNode> nodes;
+    DevArray<int> levels, res, lists, zone_cta;
+    DevArray<NetCta> ctas;
+    DevArray<NetPartial> part, sum;
+    DevArray<double> zw, gstate;             // [zones][3] zone_worst; state of the zones above kNetSmemMax
+    DevArray<double> cumr;                   // [total nodes] cumulative resistances in the zones' order
+    DevArray<double> scale, volt, load;      // revs_network_check's scale, voltage and loading, on first use
+};
+
+enum NetTool { kNetHostCheck, kNetRepair, kNetCentral, kNetCertify, kNetTools };
+
+// State of the network tools (revs_network_check, revs_repair_schedule, revs_central_bracket, revs_certify_infeasible).
+// Everything but the zone arrays is allocated on a tool's first call by net_alloc and kept until revs_destroy.
+struct NetTools {
+    bool valid = false;                      // bf matches the trees
+    bool ready[kNetTools] = {};              // net_alloc has run for the tool
+    NetArrays bf;
+    // [Hp][T] scratch, as many as the bracket uses: no call reads a word of it that the same call did not write
+    DevArray<double> scratch[9];
+    // the kept schedules, never scratch: REVS_NET_REPAIRED until the next ADMM run begins, REVS_NET_CENTRAL until the
+    // homes, tariff or trees change
+    DevArray<double> repaired, central;      // [Hp][T]
+    bool repaired_valid = false, central_valid = false;
+    // built once from the feeder sizes and T, which revs_create fixes
+    DevArray<int> hzone;                     // [Hp] zone of every padded home row, -1: padding
+    DevArray<int64_t> rep_wsoff;             // [zones] the repair kernel's state: shared memory (-1, at most rep_smem
+    DevArray<char> rep_gws;                  // bytes) up to kRepairSmemMaxN residences, else at this offset of rep_gws
+    size_t rep_smem = 0;
+    // per-zone results and flags, read by no later call
+    DevArray<int32_t> info;                  // [3][zones][3] the repair's zone_info; the bracket's two repairs and result
+    DevArray<int> flag;                      // [1] the bracket's and the certificate's error flags
+    DevArray<double> cen_sums, cen_bounds;   // [3][zones] cost1, cost2, C_max; [zones][2]
+    DevArray<CenZone> cen_state;
+    DevArray<int> crt_hpos;                  // [Hp]
+    DevArray<int32_t> crt_cert;              // [zones][4]
+    DevArray<unsigned long long> crt_key;    // [zones]
+};
+
 struct TimedSpan { cudaEvent_t a, b; int cat; };
 
 inline double now_ms() {
@@ -183,44 +256,7 @@ struct revs_solver {
     double* d_pool_cumr = nullptr;
     int64_t* d_pool_off = nullptr;
     size_t pool_nodes = 0;
-    // population network check (revs_network_check, network_check.cu): breadth-first zone arrays, built on its first
-    // call after the trees were set, and its scratch, kept until revs_destroy
-    bool net_valid = false;
-    NetHost net;
-    NetZone* d_net_zones = nullptr;
-    NetNode* d_net_nodes = nullptr;
-    int *d_net_levels = nullptr, *d_net_res = nullptr, *d_net_lists = nullptr, *d_net_zone_cta = nullptr;
-    NetCta* d_net_ctas = nullptr;
-    NetPartial *d_net_part = nullptr, *d_net_sum = nullptr;
-    double *d_net_zw = nullptr, *d_net_gstate = nullptr, *d_net_P = nullptr, *d_net_scale = nullptr, *d_net_volt = nullptr,
-           *d_net_load = nullptr;
-    size_t net_cap[6] = {0, 0, 0, 0, 0, 0};    // elements allocated: nodes, levels, residences, CTAs, zones, global state
-    bool net_scale_ok = false, net_out_ok = false;
-    double* d_net_cumr = nullptr;              // [total nodes] cumulative resistances in the network check's zone order
-    // greedy voltage repair (revs_repair_schedule, repair.cu): the repaired schedule of the current ADMM run and scratch
-    bool rep_valid = false;
-    double *d_rep_P = nullptr, *d_rep_pev = nullptr, *d_rep_D = nullptr;
-    char* d_rep_gws = nullptr;
-    int64_t* d_rep_wsoff = nullptr;
-    int32_t* d_rep_info = nullptr;
-    size_t rep_smem = 0;
-    // bracket of the centralized optimum (revs_central_bracket, central.cu): its kept schedule, valid until the homes,
-    // tariff or trees change, and its own scratch (never the repair's above)
-    bool cen_valid = false;
-    double *d_cen_y = nullptr, *d_cen_yb = nullptr, *d_cen_P = nullptr, *d_cen_pev = nullptr, *d_cen_D = nullptr,
-           *d_cen_Drep = nullptr, *d_cen_P1 = nullptr, *d_cen_pev1 = nullptr, *d_cen_P2 = nullptr, *d_cen_pev2 = nullptr;
-    double *d_cen_sums = nullptr, *d_cen_bounds = nullptr;    // [3][zones] cost1, cost2, C_max; [zones][2]
-    int32_t *d_cen_info = nullptr;                            // [3][zones][3] repair of start 1, of start 2, result
-    CenZone* d_cen_state = nullptr;
-    int *d_cen_hzone = nullptr, *d_cen_flag = nullptr;
-    char* d_cen_gws = nullptr;
-    int64_t* d_cen_wsoff = nullptr;
-    size_t cen_smem = 0;
-    // certificate of voltage infeasibility (revs_certify_infeasible, certify.cu): scratch only, no result is kept
-    double* d_crt_D = nullptr;                                // [Hp * T] R load at the residences
-    int *d_crt_hzone = nullptr, *d_crt_hpos = nullptr, *d_crt_flag = nullptr;
-    int32_t* d_crt_cert = nullptr;                            // [zones][4]
-    unsigned long long* d_crt_key = nullptr;                  // [zones]
+    NetTools net;                              // network check, repair, bracket and certificate
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -262,13 +298,6 @@ struct revs_solver {
 };
 
 namespace {
-
-template <class Tp>
-cudaError_t dalloc(Tp** p, size_t n) {
-    cudaError_t e = cudaMalloc((void**)p, (n ? n : 1) * sizeof(Tp));
-    if (e == cudaSuccess) e = cudaMemset(*p, 0, (n ? n : 1) * sizeof(Tp));
-    return e;
-}
 
 int use_device(int device) {
     int n = 0;
@@ -341,6 +370,24 @@ int d2h_homes(const revs_solver* s, double* dst, const double* src, int w) {
     if (s->H == 0) return REVS_OK;
     CU(launch_pack_rows(src, s->d_stage, s->d_hmap, s->H, w, 0, s->sU));
     CU(cudaMemcpyAsync(dst, s->d_stage, (size_t)s->H * w * sizeof(double), cudaMemcpyDeviceToHost, s->sU));
+    return REVS_OK;
+}
+
+// A schedule on the device (P, p_ev: [Hp][T]) to the caller in the compact home order: hour_mask [H][mask_words]
+// charging bits and P_out [H][T], each when given; *launches counts both kernels.
+int schedule_d2h(const revs_solver* s, const double* P, const double* p_ev, double* P_out, uint64_t* hour_mask,
+                 int mask_words, int64_t* launches) {
+    if (hour_mask && s->H > 0) {
+        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
+        CU(launch_hour_mask(p_ev, s->d_hmap, s->H, s->T, d_mask, s->sU));
+        ++*launches;
+        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
+    }
+    if (P_out && s->H > 0) {
+        int rc = d2h_homes(s, P_out, P, s->T);
+        if (rc) return rc;
+        ++*launches;
+    }
     return REVS_OK;
 }
 
@@ -921,14 +968,7 @@ void free_all(revs_solver* s) {
                     s->d_gt, s->d_vt, s->d_wcount, s->d_widx, s->d_status, s->d_innerok, s->d_cls, s->d_order, s->d_order4, s->d_order_count, s->d_cnt, s->d_diff,
                     s->d_cprob, s->d_ctiles, s->d_respart, s->d_dsum,
                     s->d_nt_zones, s->d_nt_lvl, s->d_nt_parent, s->d_nt_home, s->d_nt_hnode, s->d_nt_wsi, s->d_nt_child, s->d_nt_homes, s->d_nt_rho,
-                    s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2, s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists,
-                    s->d_net_zone_cta, s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_P,
-                    s->d_net_scale, s->d_net_volt, s->d_net_load, s->d_net_cumr, s->d_rep_P, s->d_rep_pev, s->d_rep_D,
-                    s->d_rep_gws, s->d_rep_wsoff, s->d_rep_info, s->d_cen_y, s->d_cen_yb, s->d_cen_P, s->d_cen_pev,
-                    s->d_cen_D, s->d_cen_Drep, s->d_cen_P1, s->d_cen_pev1, s->d_cen_P2, s->d_cen_pev2, s->d_cen_sums,
-                    s->d_cen_bounds, s->d_cen_info, s->d_cen_state, s->d_cen_hzone, s->d_cen_flag, s->d_cen_gws,
-                    s->d_cen_wsoff, s->d_crt_D, s->d_crt_hzone, s->d_crt_hpos, s->d_crt_flag, s->d_crt_cert,
-                    s->d_crt_key};
+                    s->d_nt_ws, s->d_nt_ws4, s->d_nt_ws2};
     for (int r = 0; r < kMaxPeers; ++r)
         if (s->peer_box[r] && s->peer_box[r] != s->d_mailbox) cudaIpcCloseMemHandle(s->peer_box[r]);
     for (int r = 0; r < kGatherMaxPeers; ++r)
@@ -1175,8 +1215,8 @@ int revs_set_feeder_tree(revs_solver* s, int feeder, int n_nodes, const int32_t*
     Tree& t = s->trees[feeder];
     if (t.d_parent && !t.pooled) { cudaFree(t.d_parent); cudaFree(t.d_cumr); cudaFree(t.d_res_node); }
     t = Tree();
-    s->net_valid = false;
-    s->cen_valid = false;
+    s->net.valid = false;
+    s->net.central_valid = false;
     t.n_nodes = n_nodes;
     CU(dalloc(&t.d_parent, (size_t)n_nodes));
     CU(dalloc(&t.d_cumr, (size_t)n_nodes));
@@ -1226,8 +1266,8 @@ int revs_set_feeder_trees(revs_solver* s, const int64_t* node_off, const int32_t
             res_p[s->feeders[f].off + (j - s->off[f])] = res_node[j];
         }
     }
-    s->net_valid = false;
-    s->cen_valid = false;
+    s->net.valid = false;
+    s->net.central_valid = false;
     if (s->pool_nodes < (size_t)total) {
         if (s->d_pool_parent) { cudaFree(s->d_pool_parent); cudaFree(s->d_pool_cumr); s->d_pool_parent = nullptr; s->d_pool_cumr = nullptr; }
         CU(dalloc(&s->d_pool_parent, (size_t)total));
@@ -1342,7 +1382,7 @@ int revs_set_homes(revs_solver* s, const double* load, const uint8_t* has_ev, co
     if (s->debug_host)
         fprintf(stderr, "[revs host] set_homes: staging %.3f ms, waiting for the link %.3f ms, copies %.3f ms\n", th1 - th0, th2 - th1, now_ms() - th2);
     s->homes_set = true;
-    s->cen_valid = false;
+    s->net.central_valid = false;
     return REVS_OK;
 }
 
@@ -1351,7 +1391,7 @@ int revs_set_tariff(revs_solver* s, const double* cost) {
     CU(cudaSetDevice(s->device));
     CU(cudaMemcpy(s->d_cost, cost, sizeof(double) * s->T, cudaMemcpyHostToDevice));
     s->tariff_set = true;
-    s->cen_valid = false;
+    s->net.central_valid = false;
     return REVS_OK;
 }
 
@@ -1365,7 +1405,7 @@ int revs_admm_begin(revs_solver* s, double kappa, int iter_max, double vset, dou
     CU(cudaSetDevice(s->device));
     s->kappa = kappa; s->iter_max = iter_max; s->vset = vset; s->vlow = vlow; s->vhigh = vhigh;
     s->k = 0; s->cur = 0; s->running = true;
-    s->rep_valid = false;            // the repaired schedule belongs to the previous run
+    s->net.repaired_valid = false;   // the repaired schedule belongs to the previous run
     s->warm_cls = 0;                 // multipliers start at zero
     s->ws_bound = 0;
     memset(&s->stats, 0, sizeof s->stats);
@@ -1738,13 +1778,10 @@ int revs_get_schedule_ld(const revs_solver* s, double* P_sch, uint64_t* hour_mas
     if (s->k == 0) return fail(REVS_ERR_ARG, "no ADMM iteration has run");
     if (hour_mask && mask_words != (s->T + 63) / 64) return fail(REVS_ERR_ARG, "mask_words must be ceil(T / 64) = %d", (s->T + 63) / 64);
     CU(cudaSetDevice(s->device));
-    if (hour_mask && s->H > 0) {
-        // the staging buffer holds H (T + 1) doubles >= H ceil(T / 64) words
-        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);
-        CU(launch_hour_mask(s->d_pev, s->d_hmap, s->H, s->T, d_mask, s->sU));
-        const_cast<revs_solver*>(s)->stats.kernel_launches++;
-        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
-    }
+    // P_sch goes with the other results: their gathers are not counted as launches
+    int rc = schedule_d2h(s, s->d_psch[s->cur], s->d_pev, nullptr, hour_mask, mask_words,
+                          &const_cast<revs_solver*>(s)->stats.kernel_launches);
+    if (rc) return rc;
     return get_results_impl(s, P_sch, nullptr, nullptr, diff, diff_rows, diff_ld);
 }
 
@@ -2007,7 +2044,7 @@ namespace {
 // The breadth-first arrays of revs_network_check, from the trees on the device (nothing of this runs in
 // revs_set_feeder_tree(s), which the schedule path times end to end).
 int net_prepare(revs_solver* s) {
-    if (s->net_valid) return REVS_OK;
+    if (s->net.valid) return REVS_OK;
     for (int f = 0; f < s->nf; ++f)
         if (!s->trees[f].d_parent)
             return fail(REVS_ERR_ARG, "zone %d has no tree (given as a sensitivity block): the network check needs "
@@ -2028,60 +2065,44 @@ int net_prepare(revs_solver* s) {
         all_cumr.insert(all_cumr.end(), cumr.begin(), cumr.end());
     }
     net_finish(h, s->T);
-    // the arrays below depend on the trees; the host-input staging d_net_P does not
-    void* old[] = {s->d_net_zones, s->d_net_nodes, s->d_net_levels, s->d_net_res, s->d_net_lists, s->d_net_zone_cta,
-                   s->d_net_ctas, s->d_net_part, s->d_net_sum, s->d_net_zw, s->d_net_gstate, s->d_net_scale, s->d_net_volt,
-                   s->d_net_load, s->d_net_cumr};
-    for (void* p : old)
-        if (p) cudaFree(p);
-    s->d_net_zones = nullptr; s->d_net_nodes = nullptr; s->d_net_levels = nullptr; s->d_net_res = nullptr;
-    s->d_net_lists = nullptr; s->d_net_zone_cta = nullptr; s->d_net_ctas = nullptr; s->d_net_part = nullptr;
-    s->d_net_sum = nullptr; s->d_net_zw = nullptr; s->d_net_gstate = nullptr; s->d_net_scale = nullptr;
-    s->d_net_volt = nullptr; s->d_net_load = nullptr; s->d_net_cumr = nullptr;
-    CU(dalloc(&s->d_net_zones, h.zones.size()));
-    CU(dalloc(&s->d_net_cumr, all_cumr.size()));
-    if (!all_cumr.empty())
-        CU(cudaMemcpy(s->d_net_cumr, all_cumr.data(), sizeof(double) * all_cumr.size(), cudaMemcpyHostToDevice));
-    CU(dalloc(&s->d_net_nodes, h.nodes.size()));
-    CU(dalloc(&s->d_net_levels, h.levels.size()));
-    CU(dalloc(&s->d_net_res, h.res.size()));
-    CU(dalloc(&s->d_net_lists, h.lists.size()));
-    CU(dalloc(&s->d_net_zone_cta, h.zone_cta.size()));
-    CU(dalloc(&s->d_net_ctas, h.ctas.size()));
-    CU(dalloc(&s->d_net_part, h.ctas.size()));
-    CU(dalloc(&s->d_net_sum, (size_t)1));
-    CU(dalloc(&s->d_net_zw, (size_t)3 * s->nf));
-    CU(dalloc(&s->d_net_gstate, (size_t)h.gstate_doubles));
-    CU(cudaMemcpy(s->d_net_zones, h.zones.data(), sizeof(NetZone) * h.zones.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_net_nodes, h.nodes.data(), sizeof(NetNode) * h.nodes.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_net_levels, h.levels.data(), sizeof(int) * h.levels.size(), cudaMemcpyHostToDevice));
-    if (!h.res.empty()) CU(cudaMemcpy(s->d_net_res, h.res.data(), sizeof(int) * h.res.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_net_lists, h.lists.data(), sizeof(int) * h.lists.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_net_zone_cta, h.zone_cta.data(), sizeof(int) * h.zone_cta.size(), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(s->d_net_ctas, h.ctas.data(), sizeof(NetCta) * h.ctas.size(), cudaMemcpyHostToDevice));
-    s->net = std::move(h);
-    s->net_valid = true;
+    s->net.bf = NetArrays();     // frees the arrays of the previous trees
+    NetArrays& b = s->net.bf;
+    CU(b.part.alloc(h.ctas.size()));
+    CU(b.sum.alloc((size_t)1));
+    CU(b.zw.alloc((size_t)3 * s->nf));
+    CU(b.gstate.alloc((size_t)h.gstate_doubles));
+    CU(b.zones.upload(h.zones));
+    CU(b.cumr.upload(all_cumr));
+    CU(b.nodes.upload(h.nodes));
+    CU(b.levels.upload(h.levels));
+    CU(b.res.upload(h.res));
+    CU(b.lists.upload(h.lists));
+    CU(b.zone_cta.upload(h.zone_cta));
+    CU(b.ctas.upload(h.ctas));
+    b.h = std::move(h);
+    s->net.valid = true;
     return REVS_OK;
 }
 
-// The network check kernels on the schedule P (device, [Hp][T]): per-CTA partials, d_net_zw and d_net_sum, and
+// The network check kernels on the schedule P (device, [Hp][T]): per-CTA partials, zone_worst and the summary, and
 // optionally the voltages, loadings and residence drops.
 int net_run(revs_solver* s, const double* P, double v2, double u, double low, double row_tol, const double* scale,
             double* voltage, double* loading, double* drop, int64_t* launches) {
-    const NetHost& h = s->net;
+    const NetArrays& b = s->net.bf;
+    const NetHost& h = b.h;
     NetParams prm{};
-    prm.zones = s->d_net_zones;
-    prm.nodes = s->d_net_nodes;
-    prm.levels = s->d_net_levels;
-    prm.res = s->d_net_res;
-    prm.ctas = s->d_net_ctas;
+    prm.zones = b.zones;
+    prm.nodes = b.nodes;
+    prm.levels = b.levels;
+    prm.res = b.res;
+    prm.ctas = b.ctas;
     prm.P = P;
     prm.scale = scale;
     prm.voltage = voltage;
     prm.loading = loading;
     prm.drop = drop;
-    prm.gstate = s->d_net_gstate;
-    prm.part = s->d_net_part;
+    prm.gstate = b.gstate;
+    prm.part = b.part;
     prm.T = s->T;
     prm.v2 = v2;
     prm.u = u;
@@ -2090,44 +2111,81 @@ int net_run(revs_solver* s, const double* P, double v2, double u, double low, do
     for (int c = 0; c < 3; ++c) {
         const int n = h.class_off[c + 1] - h.class_off[c];
         if (n == 0) continue;
-        CU(launch_network_check(prm, s->d_net_lists + h.class_off[c], n, c == 2 ? 0 : h.class_smem[c], s->sU));
+        CU(launch_network_check(prm, b.lists + h.class_off[c], n, c == 2 ? 0 : h.class_smem[c], s->sU));
         ++*launches;
     }
-    CU(launch_network_reduce(s->d_net_part, s->d_net_zone_cta, s->nf, s->d_net_zw, s->d_net_sum, s->sU));
+    CU(launch_network_reduce(b.part, b.zone_cta, s->nf, b.zw, b.sum, s->sU));
     ++*launches;
     return REVS_OK;
 }
 
-// The repair kernel's per-zone state: shared memory up to kRepairSmemMaxN residences, else a block of a global
-// scratch (*gws, offsets *wsoff); *smem = the largest shared block.
-int repair_scratch(revs_solver* s, int64_t** wsoff, char** gws, size_t* smem) {
-    std::vector<int64_t> off(s->nf);
-    int64_t g = 0;
-    for (int f = 0; f < s->nf; ++f) {
-        const size_t b = repair_ws_bytes(s->feeders[f].n, s->T);
-        if (s->feeders[f].n > kRepairSmemMaxN) {
-            off[f] = g;
-            g += (int64_t)b;
-        } else {
-            off[f] = -1;
-            *smem = std::max(*smem, b);
-        }
+// A tool's state besides the zone arrays: [Hp][T] scratch up to the number the tool uses, its kept schedule and per-zone
+// buffers, the repair kernel's per-zone state (repair, bracket) and the home -> zone map (bracket, certificate).
+int net_alloc(revs_solver* s, NetTool tool) {
+    static const int n_scratch[] = {1, 2, 9, 1};
+    NetTools& t = s->net;
+    if (t.ready[tool]) return REVS_OK;
+    const size_t HT = (size_t)s->Hp * s->T, nf = (size_t)s->nf;
+    for (int i = 0; i < n_scratch[tool]; ++i)
+        if (!t.scratch[i]) CU(t.scratch[i].alloc(HT));
+    if (tool == kNetRepair) CU(t.repaired.alloc(HT));
+    if (tool == kNetCentral) {
+        CU(t.central.alloc(HT));
+        CU(t.cen_sums.alloc(3 * nf));
+        CU(t.cen_bounds.alloc(2 * nf));
+        CU(t.cen_state.alloc(nf));
     }
-    CU(dalloc(wsoff, (size_t)s->nf));
-    CU(cudaMemcpy(*wsoff, off.data(), sizeof(int64_t) * s->nf, cudaMemcpyHostToDevice));
-    CU(dalloc(gws, (size_t)g));
+    if (tool == kNetCertify) {
+        CU(t.crt_hpos.alloc((size_t)s->Hp));
+        CU(t.crt_cert.alloc(4 * nf));
+        CU(t.crt_key.alloc(nf));
+    }
+    if ((tool == kNetRepair || tool == kNetCentral) && !t.rep_gws) {
+        std::vector<int64_t> off(nf);
+        int64_t g = 0;
+        for (size_t f = 0; f < nf; ++f) {
+            const size_t b = repair_ws_bytes(s->feeders[f].n, s->T);
+            if (s->feeders[f].n > kRepairSmemMaxN) {
+                off[f] = g;
+                g += (int64_t)b;
+            } else {
+                off[f] = -1;
+                t.rep_smem = std::max(t.rep_smem, b);
+            }
+        }
+        CU(t.info.alloc(9 * nf));
+        CU(t.rep_wsoff.upload(off));
+        CU(t.rep_gws.alloc((size_t)g));
+    }
+    if ((tool == kNetCentral || tool == kNetCertify) && !t.hzone) {
+        std::vector<int> hz((size_t)s->Hp, -1);
+        for (size_t f = 0; f < nf; ++f)
+            for (int j = 0; j < s->feeders[f].n; ++j) hz[(size_t)s->feeders[f].off + j] = (int)f;
+        CU(t.flag.alloc(1));
+        CU(t.hzone.upload(hz));
+    }
+    t.ready[tool] = true;
+    return REVS_OK;
+}
+
+// The voltage limits of the repair, the bracket and the certificate: v2 = vset^2, u = vhigh^2 - vset^2.
+int tool_limits(double vset, double vhigh, double row_tol, double* v2, double* u) {
+    *v2 = vset * vset;
+    *u = vhigh * vhigh - *v2;
+    if (!(vset < vhigh) || !(*u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
+    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
     return REVS_OK;
 }
 
 // The repair kernel on the schedule P / p_ev (in place) with the drops D of net_run(P), whose zone_worst it reads.
-int run_repair(revs_solver* s, double u, double row_tol, double* D, double* P, double* p_ev, char* gws,
-               const int64_t* wsoff, size_t smem, int32_t* info) {
+int run_repair(revs_solver* s, double u, double row_tol, double* D, double* P, double* p_ev, int32_t* info) {
+    const NetArrays& b = s->net.bf;
     RepairParams rp{};
-    rp.zones = s->d_net_zones;
-    rp.nodes = s->d_net_nodes;
-    rp.res = s->d_net_res;
-    rp.cumr = s->d_net_cumr;
-    rp.zone_worst = s->d_net_zw;
+    rp.zones = b.zones;
+    rp.nodes = b.nodes;
+    rp.res = b.res;
+    rp.cumr = b.cumr;
+    rp.zone_worst = b.zw;
     rp.load = s->d_load;
     rp.rating = s->d_rating;
     rp.cost = s->d_cost;
@@ -2137,13 +2195,13 @@ int run_repair(revs_solver* s, double u, double row_tol, double* D, double* P, d
     rp.D = D;
     rp.P = P;
     rp.p_ev = p_ev;
-    rp.gws = gws;
-    rp.ws_off = wsoff;
+    rp.gws = s->net.rep_gws;
+    rp.ws_off = s->net.rep_wsoff;
     rp.info = info;
     rp.T = s->T;
     rp.u = u;
     rp.row_tol = row_tol;
-    CU(launch_repair(rp, s->nf, smem, s->sU));
+    CU(launch_repair(rp, s->nf, s->net.rep_smem, s->sU));
     return REVS_OK;
 }
 
@@ -2166,44 +2224,43 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
         return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED "
                     "or REVS_NET_CENTRAL)", source);
     if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
-    if (source == REVS_NET_CENTRAL && !s->cen_valid)
+    if (source == REVS_NET_CENTRAL && !s->net.central_valid)
         return fail(REVS_ERR_ARG, "REVS_NET_CENTRAL: revs_central_bracket has not run since the homes, tariff or trees were set");
     if (source != REVS_NET_HOST && source != REVS_NET_CENTRAL && s->k == 0)
         return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check",
                     source == REVS_NET_SCHEDULE ? "schedule" : source == REVS_NET_ESTIMATE ? "estimate" : "repaired schedule");
-    if (source == REVS_NET_REPAIRED && !s->rep_valid)
+    if (source == REVS_NET_REPAIRED && !s->net.repaired_valid)
         return fail(REVS_ERR_ARG, "REVS_NET_REPAIRED: revs_repair_schedule has not run since the last ADMM run began");
     const double v2 = vset * vset, u = vhigh * vhigh - v2, lo = vlow * vlow - v2;
     if (!(u > 0.0) || !(lo <= 0.0)) return fail(REVS_ERR_ARG, "need vlow <= vset < vhigh");
     CU(cudaSetDevice(s->device));
     int rc = net_prepare(s);
     if (rc) return rc;
-    const NetHost& h = s->net;
+    NetArrays& b = s->net.bf;
     const int T = s->T;
-    const size_t out_elems = (size_t)h.total_nodes * T;
+    const size_t out_elems = (size_t)b.h.total_nodes * T;
     int64_t launches = 0;
-    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->d_rep_P
-                        : source == REVS_NET_CENTRAL ? s->d_cen_P1 : s->d_pest;
+    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->net.repaired
+                        : source == REVS_NET_CENTRAL ? s->net.central : s->d_pest;
     if (source == REVS_NET_HOST) {
-        if (!s->d_net_P) CU(dalloc(&s->d_net_P, (size_t)s->Hp * T));
-        if ((rc = h2d_homes(s, s->d_net_P, P, T))) return rc;
+        if ((rc = net_alloc(s, kNetHostCheck)) || (rc = h2d_homes(s, s->net.scratch[0], P, T))) return rc;
         launches += s->H > 0;
-        src = s->d_net_P;
+        src = s->net.scratch[0];
     }
     if (scale) {
-        if (!s->d_net_scale) CU(dalloc(&s->d_net_scale, (size_t)h.total_nodes));
-        CU(cudaMemcpyAsync(s->d_net_scale, scale, sizeof(double) * h.total_nodes, cudaMemcpyHostToDevice, s->sU));
+        if (!b.scale) CU(b.scale.alloc((size_t)b.h.total_nodes));
+        CU(cudaMemcpyAsync(b.scale, scale, sizeof(double) * b.h.total_nodes, cudaMemcpyHostToDevice, s->sU));
     }
-    if (voltage && !s->d_net_volt) CU(dalloc(&s->d_net_volt, out_elems));
-    if (loading && !s->d_net_load) CU(dalloc(&s->d_net_load, out_elems));
-    if ((rc = net_run(s, src, v2, u, -lo, row_tol, scale ? s->d_net_scale : nullptr, voltage ? s->d_net_volt : nullptr,
-                      loading ? s->d_net_load : nullptr, nullptr, &launches)))
+    if (voltage && !b.volt) CU(b.volt.alloc(out_elems));
+    if (loading && !b.load) CU(b.load.alloc(out_elems));
+    if ((rc = net_run(s, src, v2, u, -lo, row_tol, scale ? b.scale.p : nullptr, voltage ? b.volt.p : nullptr,
+                      loading ? b.load.p : nullptr, nullptr, &launches)))
         return rc;
     NetPartial m;
-    CU(cudaMemcpyAsync(&m, s->d_net_sum, sizeof m, cudaMemcpyDeviceToHost, s->sU));
-    if (zone_worst) CU(cudaMemcpyAsync(zone_worst, s->d_net_zw, sizeof(double) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
-    if (voltage) CU(cudaMemcpyAsync(voltage, s->d_net_volt, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
-    if (loading) CU(cudaMemcpyAsync(loading, s->d_net_load, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaMemcpyAsync(&m, b.sum, sizeof m, cudaMemcpyDeviceToHost, s->sU));
+    if (zone_worst) CU(cudaMemcpyAsync(zone_worst, b.zw, sizeof(double) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
+    if (voltage) CU(cudaMemcpyAsync(voltage, b.volt, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
+    if (loading) CU(cudaMemcpyAsync(loading, b.load, sizeof(double) * out_elems, cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->stats.kernel_launches += launches;
     if (summary) {
@@ -2228,47 +2285,28 @@ int revs_repair_schedule(revs_solver* s, double vset, double vhigh, double row_t
     if (!s) return fail(REVS_ERR_ARG, "null solver");
     if (s->k == 0) return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no schedule to repair");
     if (hour_mask && mask_words != (s->T + 63) / 64) return fail(REVS_ERR_ARG, "mask_words must be ceil(T / 64) = %d", (s->T + 63) / 64);
-    const double v2 = vset * vset, u = vhigh * vhigh - v2;
-    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
-    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
-    CU(cudaSetDevice(s->device));
-    int rc = net_prepare(s);
+    double v2, u;
+    int rc = tool_limits(vset, vhigh, row_tol, &v2, &u);
     if (rc) return rc;
-    const int T = s->T;
-    const size_t HT = (size_t)s->Hp * T;
-    if (!s->d_rep_P) {
-        if ((rc = repair_scratch(s, &s->d_rep_wsoff, &s->d_rep_gws, &s->rep_smem))) return rc;
-        CU(dalloc(&s->d_rep_info, (size_t)3 * s->nf));
-        CU(dalloc(&s->d_rep_D, HT));
-        CU(dalloc(&s->d_rep_pev, HT));
-        CU(dalloc(&s->d_rep_P, HT));
-        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
-    }
-    s->rep_valid = false;
+    CU(cudaSetDevice(s->device));
+    if ((rc = net_prepare(s)) || (rc = net_alloc(s, kNetRepair))) return rc;
+    NetTools& t = s->net;
+    const size_t HT = (size_t)s->Hp * s->T;
+    double *D = t.scratch[0], *pev = t.scratch[1];
+    t.repaired_valid = false;
     int64_t launches = 0;
-    CU(cudaMemcpyAsync(s->d_rep_P, s->d_psch[s->cur], HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
-    CU(cudaMemcpyAsync(s->d_rep_pev, s->d_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(t.repaired, s->d_psch[s->cur], HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(pev, s->d_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
     // the drops of the schedule at every residence, and which zones violate a row
-    if ((rc = net_run(s, s->d_psch[s->cur], v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_rep_D, &launches))) return rc;
-    if ((rc = run_repair(s, u, row_tol, s->d_rep_D, s->d_rep_P, s->d_rep_pev, s->d_rep_gws, s->d_rep_wsoff, s->rep_smem,
-                         s->d_rep_info)))
-        return rc;
+    if ((rc = net_run(s, s->d_psch[s->cur], v2, u, v2, row_tol, nullptr, nullptr, nullptr, D, &launches))) return rc;
+    if ((rc = run_repair(s, u, row_tol, D, t.repaired, pev, t.info))) return rc;
     launches += s->nf > 0;
-    if (hour_mask && s->H > 0) {
-        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
-        CU(launch_hour_mask(s->d_rep_pev, s->d_hmap, s->H, T, d_mask, s->sU));
-        ++launches;
-        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
-    }
-    if (P_out && s->H > 0) {
-        if ((rc = d2h_homes(s, P_out, s->d_rep_P, T))) return rc;
-        ++launches;
-    }
+    if ((rc = schedule_d2h(s, t.repaired, pev, P_out, hour_mask, mask_words, &launches))) return rc;
     if (zone_info && s->nf > 0)
-        CU(cudaMemcpyAsync(zone_info, s->d_rep_info, sizeof(int32_t) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
+        CU(cudaMemcpyAsync(zone_info, t.info, sizeof(int32_t) * 3 * s->nf, cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->stats.kernel_launches += launches;
-    s->rep_valid = true;
+    t.repaired_valid = true;
     return REVS_OK;
 }
 
@@ -2279,41 +2317,26 @@ int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_t
     if (!s->tariff_set) return fail(REVS_ERR_ARG, "revs_set_tariff has not been called");
     if (iters < 0) return fail(REVS_ERR_ARG, "iters must be >= 0");
     if (hour_mask && mask_words != (s->T + 63) / 64) return fail(REVS_ERR_ARG, "mask_words must be ceil(T / 64) = %d", (s->T + 63) / 64);
-    const double v2 = vset * vset, u = vhigh * vhigh - v2;
-    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
-    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
-    CU(cudaSetDevice(s->device));
-    int rc = net_prepare(s);
+    double v2, u;
+    int rc = tool_limits(vset, vhigh, row_tol, &v2, &u);
     if (rc) return rc;
+    CU(cudaSetDevice(s->device));
+    if ((rc = net_prepare(s)) || (rc = net_alloc(s, kNetCentral))) return rc;
+    NetTools& t = s->net;
     const int T = s->T, nf = s->nf;
     const size_t HT = (size_t)s->Hp * T;
-    if (!s->d_cen_y) {
-        if ((rc = repair_scratch(s, &s->d_cen_wsoff, &s->d_cen_gws, &s->cen_smem))) return rc;
-        double** hts[] = {&s->d_cen_y, &s->d_cen_yb, &s->d_cen_P, &s->d_cen_pev, &s->d_cen_D, &s->d_cen_Drep,
-                          &s->d_cen_P1, &s->d_cen_pev1, &s->d_cen_P2, &s->d_cen_pev2};
-        for (double** b : hts) CU(dalloc(b, HT));
-        CU(dalloc(&s->d_cen_sums, (size_t)3 * nf));
-        CU(dalloc(&s->d_cen_bounds, (size_t)2 * nf));
-        CU(dalloc(&s->d_cen_info, (size_t)9 * nf));
-        CU(dalloc(&s->d_cen_state, (size_t)nf));
-        CU(dalloc(&s->d_cen_flag, (size_t)1));
-        std::vector<int> hz((size_t)s->Hp, 0);
-        for (int f = 0; f < nf; ++f)
-            for (int j = 0; j < s->feeders[f].n; ++j) hz[(size_t)s->feeders[f].off + j] = f;
-        CU(dalloc(&s->d_cen_hzone, hz.size()));
-        CU(cudaMemcpy(s->d_cen_hzone, hz.data(), sizeof(int) * hz.size(), cudaMemcpyHostToDevice));
-        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
-    }
-    s->cen_valid = false;
+    double *y = t.scratch[0], *yb = t.scratch[1], *P = t.scratch[2], *pev = t.scratch[3], *D = t.scratch[4],
+           *Drep = t.scratch[5], *pev1 = t.scratch[6], *P2 = t.scratch[7], *pev2 = t.scratch[8], *P1 = t.central;
+    t.central_valid = false;
     int64_t launches = 0;
-    double *cost1 = s->d_cen_sums, *cost2 = cost1 + nf, *cmax = cost2 + nf;
-    int32_t *info1 = s->d_cen_info, *info2 = info1 + 3 * nf, *info = info2 + 3 * nf;
-    CU(cudaMemsetAsync(s->d_cen_y, 0, HT * sizeof(double), s->sU));
-    CU(cudaMemsetAsync(s->d_cen_yb, 0, HT * sizeof(double), s->sU));
-    CU(cudaMemsetAsync(s->d_cen_flag, 0, sizeof(int), s->sU));
+    double *cost1 = t.cen_sums, *cost2 = cost1 + nf, *cmax = cost2 + nf;
+    int32_t *info1 = t.info, *info2 = info1 + 3 * nf, *info = info2 + 3 * nf;
+    CU(cudaMemsetAsync(y, 0, HT * sizeof(double), s->sU));
+    CU(cudaMemsetAsync(yb, 0, HT * sizeof(double), s->sU));
+    CU(cudaMemsetAsync(t.flag, 0, sizeof(int), s->sU));
     CenSelectParams sp{};
-    sp.zones = s->d_net_zones;
-    sp.hzone = s->d_cen_hzone;
+    sp.zones = t.bf.zones;
+    sp.hzone = t.hzone;
     sp.load = s->d_load;
     sp.rating = s->d_rating;
     sp.cost = s->d_cost;
@@ -2322,47 +2345,45 @@ int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_t
     sp.end = s->d_end;
     sp.n_min = s->d_nmin;
     sp.n_max = s->d_nmax;
-    sp.P = s->d_cen_P;
-    sp.p_ev = s->d_cen_pev;
-    sp.infeasible = s->d_cen_flag;
+    sp.P = P;
+    sp.p_ev = pev;
+    sp.infeasible = t.flag;
     sp.Hp = s->Hp;
     sp.T = T;
     // C_max: the most expensive SOC-feasible schedule
     sp.most_expensive = 1;
     CU(launch_central_select(sp, s->sU));
-    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P, T, cmax, s->sU));
+    CU(launch_central_cost(t.bf.zones, nf, s->d_cost, P, T, cmax, s->sU));
     // first start: the repair of e*(0)
     sp.most_expensive = 0;
     CU(launch_central_select(sp, s->sU));
-    if ((rc = net_run(s, s->d_cen_P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
-    CU(cudaMemcpyAsync(s->d_cen_Drep, s->d_cen_D, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
-    CU(cudaMemcpyAsync(s->d_cen_P1, s->d_cen_P, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
-    CU(cudaMemcpyAsync(s->d_cen_pev1, s->d_cen_pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
-    if ((rc = run_repair(s, u, row_tol, s->d_cen_Drep, s->d_cen_P1, s->d_cen_pev1, s->d_cen_gws, s->d_cen_wsoff,
-                         s->cen_smem, info1)))
-        return rc;
-    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P1, T, cost1, s->sU));
+    if ((rc = net_run(s, P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, D, &launches))) return rc;
+    CU(cudaMemcpyAsync(Drep, D, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(P1, P, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    CU(cudaMemcpyAsync(pev1, pev, HT * sizeof(double), cudaMemcpyDeviceToDevice, s->sU));
+    if ((rc = run_repair(s, u, row_tol, Drep, P1, pev1, info1))) return rc;
+    CU(launch_central_cost(t.bf.zones, nf, s->d_cost, P1, T, cost1, s->sU));
     // the ascent (a host loop: every evaluation is two network checks, the selection and the ascent kernel)
     CenAscentParams ap{};
-    ap.zones = s->d_net_zones;
+    ap.zones = t.bf.zones;
     ap.cost = s->d_cost;
-    ap.P = s->d_cen_P;
-    ap.D = s->d_cen_D;
-    ap.y = s->d_cen_y;
-    ap.ybest = s->d_cen_yb;
+    ap.P = P;
+    ap.D = D;
+    ap.y = y;
+    ap.ybest = yb;
     ap.cost1 = cost1;
     ap.cmax = cmax;
     ap.info1 = info1;
-    ap.state = s->d_cen_state;
+    ap.state = t.cen_state;
     ap.iters = iters;
     ap.T = T;
     ap.u = u;
-    sp.ry = s->d_cen_D;
+    sp.ry = D;
     for (int k = 0; k <= iters; ++k) {
         if (k > 0) {
-            if ((rc = net_run(s, s->d_cen_y, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+            if ((rc = net_run(s, y, v2, u, v2, row_tol, nullptr, nullptr, nullptr, D, &launches))) return rc;
             CU(launch_central_select(sp, s->sU));
-            if ((rc = net_run(s, s->d_cen_P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
+            if ((rc = net_run(s, P, v2, u, v2, row_tol, nullptr, nullptr, nullptr, D, &launches))) return rc;
             launches += 1;
         }
         ap.k = k;
@@ -2370,52 +2391,41 @@ int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_t
         launches += nf > 0;
     }
     // second start: the repair of e*(y_best)
-    if ((rc = net_run(s, s->d_cen_yb, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_D, &launches))) return rc;
-    sp.P = s->d_cen_P2;
-    sp.p_ev = s->d_cen_pev2;
+    if ((rc = net_run(s, yb, v2, u, v2, row_tol, nullptr, nullptr, nullptr, D, &launches))) return rc;
+    sp.P = P2;
+    sp.p_ev = pev2;
     CU(launch_central_select(sp, s->sU));
-    if ((rc = net_run(s, s->d_cen_P2, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_cen_Drep, &launches))) return rc;
-    if ((rc = run_repair(s, u, row_tol, s->d_cen_Drep, s->d_cen_P2, s->d_cen_pev2, s->d_cen_gws, s->d_cen_wsoff,
-                         s->cen_smem, info2)))
-        return rc;
-    CU(launch_central_cost(s->d_net_zones, nf, s->d_cost, s->d_cen_P2, T, cost2, s->sU));
+    if ((rc = net_run(s, P2, v2, u, v2, row_tol, nullptr, nullptr, nullptr, Drep, &launches))) return rc;
+    if ((rc = run_repair(s, u, row_tol, Drep, P2, pev2, info2))) return rc;
+    CU(launch_central_cost(t.bf.zones, nf, s->d_cost, P2, T, cost2, s->sU));
     CenFinalParams fp{};
-    fp.zones = s->d_net_zones;
-    fp.state = s->d_cen_state;
+    fp.zones = t.bf.zones;
+    fp.state = t.cen_state;
     fp.cost1 = cost1;
     fp.cost2 = cost2;
     fp.cmax = cmax;
     fp.info1 = info1;
     fp.info2 = info2;
-    fp.P1 = s->d_cen_P1;
-    fp.p_ev1 = s->d_cen_pev1;
-    fp.P2 = s->d_cen_P2;
-    fp.p_ev2 = s->d_cen_pev2;
-    fp.bounds = s->d_cen_bounds;
+    fp.P1 = P1;
+    fp.p_ev1 = pev1;
+    fp.P2 = P2;
+    fp.p_ev2 = pev2;
+    fp.bounds = t.cen_bounds;
     fp.info = info;
     fp.T = T;
     CU(launch_central_final(fp, nf, s->sU));
     launches += (s->H > 0 ? 3 : 0) + (nf > 0 ? 6 : 0);     // selections; costs, repairs, final
     int infeasible = 0;
-    CU(cudaMemcpyAsync(&infeasible, s->d_cen_flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaMemcpyAsync(&infeasible, t.flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->stats.kernel_launches += launches;
     if (infeasible) return fail(REVS_ERR_INFEASIBLE, "a home's SOC target needs more hours than its plug-in window has");
-    if (hour_mask && s->H > 0) {
-        unsigned long long* d_mask = reinterpret_cast<unsigned long long*>(s->d_stage);     // H (T + 1) doubles >= H W words
-        CU(launch_hour_mask(s->d_cen_pev1, s->d_hmap, s->H, T, d_mask, s->sU));
-        ++s->stats.kernel_launches;
-        CU(cudaMemcpyAsync(hour_mask, d_mask, (size_t)s->H * mask_words * sizeof(uint64_t), cudaMemcpyDeviceToHost, s->sU));
-    }
-    if (P_out && s->H > 0) {
-        if ((rc = d2h_homes(s, P_out, s->d_cen_P1, T))) return rc;
-        ++s->stats.kernel_launches;
-    }
+    if ((rc = schedule_d2h(s, P1, pev1, P_out, hour_mask, mask_words, &s->stats.kernel_launches))) return rc;
     if (zone_bounds && nf > 0)
-        CU(cudaMemcpyAsync(zone_bounds, s->d_cen_bounds, sizeof(double) * 2 * nf, cudaMemcpyDeviceToHost, s->sU));
+        CU(cudaMemcpyAsync(zone_bounds, t.cen_bounds, sizeof(double) * 2 * nf, cudaMemcpyDeviceToHost, s->sU));
     if (zone_info && nf > 0) CU(cudaMemcpyAsync(zone_info, info, sizeof(int32_t) * 3 * nf, cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
-    s->cen_valid = true;
+    t.central_valid = true;
     return REVS_OK;
 }
 
@@ -2423,47 +2433,34 @@ int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double ro
                             int* n_certified) {
     if (!s) return fail(REVS_ERR_ARG, "null solver");
     if (!s->homes_set) return fail(REVS_ERR_ARG, "revs_set_homes has not been called");
-    const double v2 = vset * vset, u = vhigh * vhigh - v2;
-    if (!(vset < vhigh) || !(u > 0.0)) return fail(REVS_ERR_ARG, "need vset < vhigh");
-    if (!(row_tol >= 0.0)) return fail(REVS_ERR_ARG, "row_tol must be >= 0");
-    CU(cudaSetDevice(s->device));
-    int rc = net_prepare(s);
+    double v2, u;
+    int rc = tool_limits(vset, vhigh, row_tol, &v2, &u);
     if (rc) return rc;
+    CU(cudaSetDevice(s->device));
+    if ((rc = net_prepare(s)) || (rc = net_alloc(s, kNetCertify))) return rc;
+    const NetTools& t = s->net;
     const int T = s->T, nf = s->nf;
-    if (!s->d_crt_D) {
-        CU(dalloc(&s->d_crt_D, (size_t)s->Hp * T));
-        CU(dalloc(&s->d_crt_hpos, (size_t)s->Hp));
-        CU(dalloc(&s->d_crt_cert, (size_t)4 * nf));
-        CU(dalloc(&s->d_crt_key, (size_t)nf));
-        CU(dalloc(&s->d_crt_flag, (size_t)1));
-        std::vector<int> hz((size_t)s->Hp, -1);
-        for (int f = 0; f < nf; ++f)
-            for (int j = 0; j < s->feeders[f].n; ++j) hz[(size_t)s->feeders[f].off + j] = f;
-        CU(dalloc(&s->d_crt_hzone, hz.size()));
-        CU(cudaMemcpy(s->d_crt_hzone, hz.data(), sizeof(int) * hz.size(), cudaMemcpyHostToDevice));
-        CU(cudaDeviceSynchronize());    // dalloc zeroes on the legacy stream, which does not order with the non-blocking sU
-    }
     int64_t launches = 0;
-    CU(cudaMemsetAsync(s->d_crt_flag, 0, sizeof(int), s->sU));
+    CU(cudaMemsetAsync(t.flag, 0, sizeof(int), s->sU));
     // the drops of the base load at every residence
-    if ((rc = net_run(s, s->d_load, v2, u, v2, row_tol, nullptr, nullptr, nullptr, s->d_crt_D, &launches))) return rc;
+    if ((rc = net_run(s, s->d_load, v2, u, v2, row_tol, nullptr, nullptr, nullptr, t.scratch[0], &launches))) return rc;
     CertParams cp{};
-    cp.zones = s->d_net_zones;
-    cp.nodes = s->d_net_nodes;
-    cp.res = s->d_net_res;
-    cp.cumr = s->d_net_cumr;
-    cp.hzone = s->d_crt_hzone;
-    cp.D = s->d_crt_D;
+    cp.zones = t.bf.zones;
+    cp.nodes = t.bf.nodes;
+    cp.res = t.bf.res;
+    cp.cumr = t.bf.cumr;
+    cp.hzone = t.hzone;
+    cp.D = t.scratch[0];
     cp.rating = s->d_rating;
     cp.has_ev = s->d_has_ev;
     cp.start = s->d_start;
     cp.end = s->d_end;
     cp.n_min = s->d_nmin;
     cp.n_max = s->d_nmax;
-    cp.hpos = s->d_crt_hpos;
-    cp.key = s->d_crt_key;
-    cp.cert = s->d_crt_cert;
-    cp.flag = s->d_crt_flag;
+    cp.hpos = t.crt_hpos;
+    cp.key = t.crt_key;
+    cp.cert = t.crt_cert;
+    cp.flag = t.flag;
     cp.Hp = s->Hp;
     cp.T = T;
     cp.u = u;
@@ -2472,8 +2469,8 @@ int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double ro
     launches += nf > 0 ? 3 : 0;
     int flag = 0;
     std::vector<int32_t> cert((size_t)4 * nf);
-    CU(cudaMemcpyAsync(&flag, s->d_crt_flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
-    if (nf > 0) CU(cudaMemcpyAsync(cert.data(), s->d_crt_cert, sizeof(int32_t) * cert.size(), cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaMemcpyAsync(&flag, t.flag, sizeof(int), cudaMemcpyDeviceToHost, s->sU));
+    if (nf > 0) CU(cudaMemcpyAsync(cert.data(), t.crt_cert, sizeof(int32_t) * cert.size(), cudaMemcpyDeviceToHost, s->sU));
     CU(cudaStreamSynchronize(s->sU));
     s->stats.kernel_launches += launches;
     if (flag & 2) return fail(REVS_ERR_ARG, "an EV home has a negative or non-finite rating: the certificate needs rating >= 0");

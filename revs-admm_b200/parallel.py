@@ -389,31 +389,27 @@ class PipelinedSolver:
                     voltage=None if out is None else out["voltage"], loading=None if out is None else out["loading"],
                     zone_worst=np.concatenate([r["zone_worst"] for r in res]) if zones else None)
 
+    def _zone_order(self, method, totals, *args, **kw):
+        """Solver.<method> on every pipeline at once: each array of the results concatenated in zone order (None where
+        not asked for) and the totals recomputed by `totals` -- the bytes of a single solver over the same zones."""
+        res = self._each(lambda k: getattr(self.parts[k], method)(*args, **kw))
+        return totals({n: None if v is None else np.concatenate([r[n] for r in res])
+                       for n, v in res[0].items() if v is None or isinstance(v, np.ndarray)})
+
     def repair_schedule(self, schedule=True, mask=False, **kw):
-        """Solver.repair_schedule over all pipelines at once: the schedules, masks and zone_info are concatenated in
-        zone order and the totals summed -- the bytes of a single solver over the same zones."""
+        """Solver.repair_schedule over all pipelines at once (_zone_order)."""
         from ._cabi import repair_totals
-        res = self._each(lambda k: self.parts[k].repair_schedule(schedule=schedule, mask=mask, **kw))
-        return repair_totals(dict(P_sch=np.concatenate([r["P_sch"] for r in res]) if schedule else None,
-                                  mask=np.concatenate([r["mask"] for r in res]) if mask else None,
-                                  zone_info=np.concatenate([r["zone_info"] for r in res])))
+        return self._zone_order("repair_schedule", repair_totals, schedule=schedule, mask=mask, **kw)
 
     def central_bracket(self, schedule=True, mask=False, **kw):
-        """Solver.central_bracket over all pipelines at once: schedules, masks, zone_bounds and zone_info concatenated in
-        zone order, totals recomputed -- the bytes of a single solver over the same zones."""
+        """Solver.central_bracket over all pipelines at once (_zone_order)."""
         from ._cabi import central_totals
-        res = self._each(lambda k: self.parts[k].central_bracket(schedule=schedule, mask=mask, **kw))
-        return central_totals(dict(P_sch=np.concatenate([r["P_sch"] for r in res]) if schedule else None,
-                                   mask=np.concatenate([r["mask"] for r in res]) if mask else None,
-                                   zone_bounds=np.concatenate([r["zone_bounds"] for r in res]),
-                                   zone_info=np.concatenate([r["zone_info"] for r in res])))
+        return self._zone_order("central_bracket", central_totals, schedule=schedule, mask=mask, **kw)
 
     def certify_infeasible(self, *args, **kw):
-        """Solver.certify_infeasible over all pipelines at once: zone_cert concatenated in zone order, counts
-        recomputed -- the bytes of a single solver over the same zones."""
+        """Solver.certify_infeasible over all pipelines at once (_zone_order)."""
         from ._cabi import certify_totals
-        res = self._each(lambda k: self.parts[k].certify_infeasible(*args, **kw))
-        return certify_totals(dict(zone_cert=np.concatenate([r["zone_cert"] for r in res])))
+        return self._zone_order("certify_infeasible", certify_totals, *args, **kw)
 
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
