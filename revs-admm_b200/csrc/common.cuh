@@ -71,7 +71,8 @@ struct ScreenProblem {
 };
 
 constexpr double kScreenMargin = 0.01;   // rows with v~ <= (1-margin) u are proven feasible (see screen_bf16.cu)
-constexpr double kScreenUp = 1.005;      // v <= kScreenUp * v~ for the BF16/FP32 product of non-negative terms, K <= 16384
+constexpr double kScreenUp = 1.0099;     // v <= kScreenUp * v~ for the BF16/FP32 product of non-negative terms, K <= kScreenMaxN
+constexpr int kScreenMaxN = 16384;       // largest zone (K of the screening product) the bound above holds for
 constexpr int kVerifyMaxN = 512;         // zones up to this size verify all voltage rows inside the QP kernels
 constexpr int kQpBuckets = 4;            // work lists of the warp kernel: |W| >= 3, 2, 1, 0 (hardest first)
 

@@ -416,7 +416,7 @@ int build_tables(revs_solver* s) {
         else if (n <= 256) { ++s->zg.n_mid; s->zg.mid_max = std::max(s->zg.mid_max, n); }
         else ++s->zg.n_big;
     }
-    if (s->zg.max_n > 16384) s->screen = false;    // the error bound of the BF16 screening pass (kScreenUp) holds up to 16384 terms
+    if (s->zg.max_n > kScreenMaxN) s->screen = false;    // the error bound of the BF16 screening pass (kScreenUp) holds up to kScreenMaxN terms
     void* old[] = {s->d_sprob, s->d_stiles, s->d_maps_a, s->d_bcol0, s->d_cprob, s->d_ctiles};
     for (void* q : old) if (q) cudaFree(q);
     s->d_sprob = nullptr; s->d_stiles = nullptr; s->d_maps_a = nullptr; s->d_bcol0 = nullptr; s->d_cprob = nullptr; s->d_ctiles = nullptr;
@@ -2687,9 +2687,10 @@ int revs_set_option(revs_solver* s, const char* name, double value) {
     if (!s || !name) return fail(REVS_ERR_ARG, "bad arguments");
     const bool mid_run = s->running && s->k > 0 && s->k < s->iter_max;
     if (!strcmp(name, "screen")) {
-        // the error bound of the BF16 screening pass (kScreenUp) holds up to 16384 residences per zone, and the
+        // the error bound of the BF16 screening pass (kScreenUp) holds up to kScreenMaxN residences per zone, and the
         // bf16 copy of the iterate is only maintained while screening is on
-        if (value != 0.0 && s->zg.max_n > 16384) return fail(REVS_ERR_ARG, "screening is limited to zones of at most 16384 residences");
+        if (value != 0.0 && s->zg.max_n > kScreenMaxN)
+            return fail(REVS_ERR_ARG, "screening is limited to zones of at most %d residences", kScreenMaxN);
         if (mid_run) return fail(REVS_ERR_ARG, "'screen' cannot change between revs_admm_step calls of one run");
         s->screen = value != 0.0;
         return REVS_OK;

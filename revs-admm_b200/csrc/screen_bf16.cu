@@ -3,10 +3,14 @@
 // Inside the ADMM loop the operator's LinDistFlow check (R_res @ g of Utility.network,
 // lpsolver.py:183-194) only has to answer "which rows can violate v <= u?".  All terms of
 // R g are non-negative, so a low-precision product has a rigorous RELATIVE error bound:
-//     |R~ - R| <= 2^-9 R,  |g~ - g| <= 2^-9 g   (round to nearest BF16, via FP32)
-//     FP32 accumulation of K <= 65536 exact BF16xBF16 products: <= K 2^-24 relative
-//  => v <= v~ (1 + 0.0045) for K <= 16384.
-// Rows with v~ <= (1 - kScreenMargin) u are therefore PROVEN feasible; only the remaining
+//     R <= R~ / (1 - 2^-8),  g <= g~ / (1 - 2^-8)   (BF16 keeps 8 significant bits: round to nearest loses up
+//                                                   to 2^-8, the FP64 -> FP32 -> BF16 double rounding included)
+//     FP32 accumulation of K exact BF16xBF16 products: v~ >= (1 - 2 K 2^-24) * exact sum (truncating
+//     accumulator; measured on the B200 for both screening kernels: tests/test_gpu_screening.py)
+//  => v <= v~ / ((1 - 2^-8)^2 (1 - 2^-9)) = 1.00983 v~ for K <= kScreenMaxN = 16384  (kScreenUp = 1.0099).
+// Operands just below a rounding midpoint reach v = 1.0078 v~ at every K.
+// Rows with v~ <= (1 - kScreenMargin) u are therefore PROVEN feasible ((1 - kScreenMargin) kScreenUp < 1);
+// only the remaining
 // candidates are re-evaluated exactly in FP64 (utility_qp.cu: exact_voltages), so the KKT
 // test and the results are those of the FP64 path -- "BF16 with refinement".  The screening
 // pass reads the sensitivity blocks at 2 bytes per entry instead of 8 and runs at the BF16

@@ -299,7 +299,7 @@ def test_admm_early_stop_and_step_api(gpu_lib):
 @pytest.mark.parametrize("impl", [0, 1])
 @pytest.mark.parametrize("M,K,T", [(128, 64, 96), (1008, 1008, 96), (130, 100, 24), (77, 333, 5), (300, 48, 96)])
 def test_screen_contract_bound(gpu_lib, impl, M, K, T):
-    """BF16 screening product: rigorous one-sided bound v <= 1.0045 v~ on non-negative data,
+    """BF16 screening product: rigorous one-sided bound v <= 1.0099 v~ on non-negative data,
     for the mma.sync kernel (impl 0) and the tcgen05/TMEM/TMA kernel (impl 1)."""
     rng = np.random.default_rng(M + K + T)
     A = rng.uniform(0, 2e-2, (M, K)) * (rng.random((M, K)) < 0.7)
@@ -308,8 +308,8 @@ def test_screen_contract_bound(gpu_lib, impl, M, K, T):
     ref = A @ B
     assert C.shape == ref.shape
     rel = np.abs(C - ref) / np.maximum(ref, 1e-300)
-    assert rel[ref > 0].max() <= 4.5e-3
-    assert (ref <= 1.0045 * C + 1e-30).all()
+    assert rel[ref > 0].max() <= 9.9e-3
+    assert (ref <= 1.0099 * C + 1e-30).all()
 
 
 def test_screen_impls_agree_in_the_loop(gpu_lib):
