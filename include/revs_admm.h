@@ -25,6 +25,7 @@
  *   revs_repair_schedule                          no reference counterpart (a voltage-feasible binary schedule)
  *   revs_central_bracket                          lpsolver.py:463-502 solve_central(), bracketed per zone
  *   revs_certify_infeasible                       lpsolver.py:463-502 solve_central(), zones proved infeasible
+ *   revs_hosting_capacity                         no reference counterpart (the extra load every home can take)
  *   revs_get_results / revs_get_schedule(_ld)     lpsolver.py:289-290 return diff,P_sch,S,C
  *   revs_set_option / revs_get_stats / revs_version / revs_last_error / revs_device_count /
  *   revs_reliability_sharded / revs_gather_export / revs_gather_attach
@@ -303,6 +304,41 @@ int revs_central_bracket(revs_solver* s, double vset, double vhigh, double row_t
  * changes no other state (the schedules of revs_repair_schedule and revs_central_bracket stay checkable). */
 int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double row_tol, int32_t* zone_cert,
                             int* n_certified);
+
+/* Hosting capacity of a schedule, zone by zone on the device: for every residence and step, how many more kW its home
+ * can draw, with everything else unchanged, before a voltage row or a rated line binds; for every zone and step, how
+ * many more kW every residence of the zone can draw at once.  Needs the tree of every zone; no homes, tariff or ADMM
+ * run (the counts below read the homes' windows and ratings when they are set, else they are 0).
+ *
+ * Per zone and step, with u = vhigh^2 - vset^2 and D = R P at the nodes (as in revs_network_check), the residence rows
+ * (R P)_i - u <= row_tol of the repair, bracket and certificate, d_a = 2 cumr[a] (R[i,h] = d at the lowest common
+ * ancestor of the two residences' nodes), F_a the flow on the edge above node a and s_a the caller's signed 1/rating of
+ * that edge (s_a = 0 or scale = NULL: unrated):
+ *   sigma_i = (u + row_tol) - D_i, the slack of residence i (u + row_tol formed once, then the subtraction);
+ *   home_cap[h,t] = max(0, min(V_h, L_h)), +inf when nothing limits, where
+ *     V_h = min over the ancestors a of h's node (the node included) with d_a > 0 of M_a / d_a, M_a = min sigma_i over
+ *           the residences below a, and
+ *     L_h = min over the rated edges a on h's path of (1 - |s_a| F_a) / |s_a|.
+ *   V_h equals min_i sigma_i / R[i,h] over R[i,h] > 0 bit for bit: a correctly rounded division is monotone in both
+ *   operands and min sigma / d = min (sigma / d); an ancestor above the true lowest common ancestor has a smaller d, so
+ *   its term is never the smaller one while sigma >= 0; a negative slack makes both forms negative, and both clamp to 0.
+ *   L_h is exact while no edge is overloaded against its flow (adding load at h raises F on every edge of h's path).
+ *   zone_uniform[z,t] = max(0, min(min_i sigma_i / W_i over W_i > 0, min over rated edges a with N_a > 0 of
+ *     (1 - |s_a| F_a) / (|s_a| N_a))), W = R 1 the drop of 1 kW at every residence (the network check's recurrences on
+ *     P = 1), N_a the residences below edge a: the extra load every residence of the zone can draw at once.
+ *   zone_counts[z] = {window_steps: (EV home, step of its plug-in window) pairs; window_steps_open: of those, the pairs
+ *     with home_cap >= rating (one more charger fits with nothing else changed); thermal_bound: (home, step) pairs with
+ *     L_h < V_h, 0 without scale} (int64).
+ * The lower voltage limit vlow is not a row here, nor are non-residence nodes.  home_cap [H,T] (compact home order),
+ * zone_uniform [n_feeders, T] and zone_counts [n_feeders, 3] may each be NULL; scale [total nodes] as in
+ * revs_network_check.  Every output is a minimum or an integer count: two calls give the same bytes, and a zone's
+ * result does not depend on the other zones.
+ * source: the five REVS_NET_* sources, with the preconditions of revs_network_check.  REVS_ERR_ARG: those of the
+ * source, a zone without tree (named), not vset < vhigh, row_tol < 0 or NaN, a non-finite scale entry.  Synchronous on
+ * the utility stream; adds its launches to revs_stats.kernel_launches and changes no other state (the schedules of
+ * revs_repair_schedule and revs_central_bracket stay checkable). */
+int revs_hosting_capacity(revs_solver* s, int source, const double* P, double vset, double vhigh, double row_tol,
+                          const double* scale, double* home_cap, double* zone_uniform, int64_t* zone_counts);
 
 /* The same check with the ROWS PARTITIONED over the GPUs of one box (one process per GPU, every process holds the
  * feeder's tree; BASELINE north_star: "the sensitivity contraction is row-partitioned"): every rank builds and

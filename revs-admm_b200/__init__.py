@@ -7,7 +7,7 @@ path is hand-written CUDA for sm_100a behind the C ABI of include/revs_admm.h
 from . import _cabi, extract, feeder, lpsolver, revs_fixture  # noqa: F401
 from ._cabi import (REVS_NET_CENTRAL, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED, REVS_NET_SCHEDULE,  # noqa: F401
                     REVS_REL_DROP, REVS_REL_FLOW, REVS_REL_VOLTAGE, NetworkSummary, RevsError, Solver, contract, device_count,
-                    central_status, expand_schedule, screen_contract)
+                    central_status, expand_schedule, hosting_totals, screen_contract)
 from .parallel import PipelinedSolver  # noqa: F401
 from .revs_fixture import REVS  # noqa: F401
 

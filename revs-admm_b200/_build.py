@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librevs_admm.so")
 SOURCES = ["contract_f64.cu", "home_solve.cu", "dual_update.cu", "utility_qp.cu", "utility_qp_warp.cu", "tree_newton.cu",
-           "feeder_build.cu", "network_check.cu", "repair.cu", "central.cu", "certify.cu", "screen_bf16.cu", "screen_tc5.cu",
+           "feeder_build.cu", "network_check.cu", "repair.cu", "central.cu", "certify.cu", "hosting.cu", "screen_bf16.cu", "screen_tc5.cu",
            "revs_capi.cu"]
 HEADERS = ["common.cuh", "kernels.cuh", os.path.join("..", "..", "include", "revs_admm.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--threads", "0",

@@ -95,6 +95,8 @@ SIGNATURES = {
                               C.POINTER(C.c_int32)], C.c_int),
     "revs_certify_infeasible": ([_P, C.c_double, C.c_double, C.c_double, C.POINTER(C.c_int32), C.POINTER(C.c_int)],
                                 C.c_int),
+    "revs_hosting_capacity": ([_P, C.c_int, _D, C.c_double, C.c_double, C.c_double, _D, _D, _D, C.POINTER(C.c_int64)],
+                              C.c_int),
 }
 
 _lib = None
@@ -203,6 +205,27 @@ def certify_totals(r):
     (zones of kind 1 or 2)."""
     kind = r["zone_cert"][:, 0]
     r.update(zones_kind=[int((kind == k).sum()) for k in range(3)], certified=int((kind > 0).sum()))
+    return r
+
+
+def hosting_totals(r, zone_off):
+    """Add the totals of a hosting_capacity result: window_steps, window_steps_open and thermal_bound (zone_counts summed
+    over the zones), home_cap_min = dict(value, zone, index, step) of the smallest home capacity (index local to the
+    zone; zone_off = the [zones + 1] home offsets) and uniform_min = dict(value, zone, step) of the smallest uniform
+    headroom.  Ties go to the lowest zone, index, step; a minimum is None when its array was not asked for."""
+    c = r["zone_counts"]
+    r.update(window_steps=int(c[:, 0].sum()), window_steps_open=int(c[:, 1].sum()), thermal_bound=int(c[:, 2].sum()),
+             home_cap_min=None, uniform_min=None)
+    cap, uni = r["home_cap"], r["zone_uniform"]
+    if cap is not None and cap.size:
+        k = int(np.argmin(cap))
+        h, t = divmod(k, cap.shape[1])
+        z = int(np.searchsorted(zone_off, h, side="right")) - 1
+        r["home_cap_min"] = dict(value=float(cap.flat[k]), zone=z, index=h - int(zone_off[z]), step=t)
+    if uni is not None and uni.size:
+        k = int(np.argmin(uni))
+        z, t = divmod(k, uni.shape[1])
+        r["uniform_min"] = dict(value=float(uni.flat[k]), zone=z, step=t)
     return r
 
 
@@ -478,6 +501,33 @@ class Solver:
         _check(self.lib.revs_certify_infeasible(self._h, vset, vhigh, row_tol, Z.ctypes.data_as(C.POINTER(C.c_int32)),
                                                 None))
         return certify_totals(dict(zone_cert=Z))
+
+    def hosting_capacity(self, source="schedule", vset=1.0, vhigh=1.05, row_tol=1e-9, scale=None, homes=True,
+                         uniform=True):
+        """Hosting capacity of a schedule zone by zone on the device (include/revs_admm.h: revs_hosting_capacity): how
+        many more kW every home can draw at every step, with everything else unchanged, before a voltage row
+        (R P)_i - (vhigh^2 - vset^2) <= row_tol or a rated line binds.  source as in network_check; scale: [total_nodes]
+        signed 1/rating per edge, 0 = unrated (None: no edge is rated).  Returns dict(home_cap=[H, T] kW or None,
+        zone_uniform=[zones, T] kW every residence of the zone can add at once, or None, zone_counts=[zones, 3] int64
+        {window steps, window steps where one more charger fits, thermally bound (home, step) pairs}) with the totals of
+        hosting_totals.  Nothing else is read or changed."""
+        T = self.T
+        Pp = None
+        if isinstance(source, str):
+            src = {"schedule": REVS_NET_SCHEDULE, "estimate": REVS_NET_ESTIMATE, "repaired": REVS_NET_REPAIRED,
+                   "central": REVS_NET_CENTRAL}.get(source)
+            if src is None:
+                raise ValueError("source must be 'schedule', 'estimate', 'repaired', 'central' or an [H, T] array, "
+                                 f"not {source!r}")
+        else:
+            src, Pp = REVS_NET_HOST, _f64(source, (self.H, T))
+        sc = None if scale is None else _f64(scale, (self.total_nodes,))
+        cap = np.empty((self.H, T)) if homes else None
+        uni = np.empty((self.nf, T)) if uniform else None
+        cnt = np.zeros((self.nf, 3), dtype=np.int64)
+        _check(self.lib.revs_hosting_capacity(self._h, src, _dp(Pp), vset, vhigh, row_tol, _dp(sc), _dp(cap), _dp(uni),
+                                              cnt.ctypes.data_as(C.POINTER(C.c_int64))))
+        return hosting_totals(dict(home_cap=cap, zone_uniform=uni, zone_counts=cnt), self.off)
 
     # ---- the same check with the rows partitioned over the GPUs of the box; the all-gather of the result is fused
     # into the epilogue of the contraction kernel (peer-memory stores, include/revs_admm.h: revs_gather_*)

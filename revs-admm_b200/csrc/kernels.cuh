@@ -347,6 +347,8 @@ struct NetHost {                  // host side of the arrays above, built once p
 void net_add_zone(NetHost& h, int n_nodes, const int* parent, const double* cumr, int n_res, const int* res_node,
                   int64_t home_row);
 void net_finish(NetHost& h, int T);
+// log2 of the steps per CTA of a zone whose state is `one` bytes per step, and the class of its CTAs (NetHost::class_off)
+int net_zone_lg(size_t one, int T, int* cls);
 cudaError_t launch_network_check(const NetParams& P, const int* d_list, int n_ctas, size_t smem, cudaStream_t s);
 cudaError_t launch_network_reduce(const NetPartial* part, const int* zone_cta, int n_zones, double* zone_worst,
                                   NetPartial* out, cudaStream_t s);
@@ -442,5 +444,40 @@ struct CertParams {
     double u, thr;                // vhigh^2 - vset^2, row_tol + 1e-12
 };
 cudaError_t launch_certify(const CertParams& P, int n_zones, cudaStream_t s);
+
+// ---- hosting.cu: hosting capacity of a schedule, per residence and step and per zone and step
+struct HcCta { int zone, t0, lg, pad_; int64_t gstate; };  // lg: log2 of the steps; gstate: global scratch offset, -1: shared
+struct HcParams {
+    const NetZone* zones;         // the network check's breadth-first arrays
+    const NetNode* nodes;
+    const int* levels;
+    const int* res;
+    const HcCta* ctas;
+    const double* cumr;           // [total nodes], zone z at zones[z].out_row
+    const double2* wn;            // [nodes pool] per breadth-first position: {W, N}, the drop and flow of 1 kW everywhere
+    const double* P;              // [Hp][T]
+    const double* scale;          // [total nodes] signed 1/rating per edge (0 = unrated), or null: no edge is rated
+    const uint8_t* has_ev;        // [Hp]
+    const double* rating;
+    const int *start, *end;
+    double* cap;                  // [Hp][T] out, or null
+    double* uniform;              // [zones][T] out, or null
+    double* gstate;               // global scratch of the zones above kNetSmemMax (two doubles per node)
+    unsigned long long* part;     // [CTAs][3] window steps, open window steps, thermally bound pairs
+    int T;
+    double ur;                    // u + row_tol
+};
+struct HcHost {                   // host side of the hosting CTAs, built once per set of trees
+    std::vector<HcCta> ctas;
+    std::vector<int> lists, zone_cta;
+    std::vector<double2> wn;
+    int class_off[4] = {0, 0, 0, 0};
+    size_t class_smem[3] = {0, 0, 0};        // dynamic shared memory of each class, at least the final reduction's
+    int64_t gstate_doubles = 0;
+};
+void hc_prepare(const NetHost& h, int T, HcHost& out);
+cudaError_t launch_hosting(const HcParams& P, const int* d_list, int n_ctas, size_t smem, cudaStream_t s);
+cudaError_t launch_hosting_reduce(const unsigned long long* part, const int* zone_cta, int n_zones, int64_t* counts,
+                                  cudaStream_t s);
 
 }  // namespace revs

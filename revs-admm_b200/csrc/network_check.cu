@@ -233,9 +233,18 @@ void net_add_zone(NetHost& h, int n_nodes, const int* parent, const double* cumr
     h.total_nodes += n_nodes;
 }
 
+int net_zone_lg(size_t one, int T, int* cls) {
+    int G = 1;
+    while (G < T && G < kNetMaxSteps) G <<= 1;
+    *cls = 0;
+    while (G > 1 && one * G > kNetSmemSmall) G >>= 1;
+    if (one * G > kNetSmemSmall) *cls = one <= kNetSmemMax ? 1 : 2;
+    int lg = 0;
+    while ((1 << lg) < G) ++lg;
+    return lg;
+}
+
 void net_finish(NetHost& h, int T) {
-    int gmax = 1;
-    while (gmax < T && gmax < kNetMaxSteps) gmax <<= 1;
     std::vector<int> lists[3];
     h.zone_cta.assign(1, 0);
     h.ctas.clear();
@@ -244,11 +253,9 @@ void net_finish(NetHost& h, int T) {
     for (size_t zi = 0; zi < h.zones.size(); ++zi) {
         NetZone& z = h.zones[zi];
         const size_t one = (size_t)z.n_nodes * sizeof(double);
-        int G = gmax, cls = 0;
-        while (G > 1 && one * G > kNetSmemSmall) G >>= 1;
-        if (one * G > kNetSmemSmall) cls = one <= kNetSmemMax ? 1 : 2;
-        z.lg = 0;
-        while ((1 << z.lg) < G) ++z.lg;
+        int cls = 0;
+        z.lg = net_zone_lg(one, T, &cls);
+        const int G = 1 << z.lg;
         for (int t0 = 0; t0 < T; t0 += G) {
             NetCta c{(int)zi, t0, -1};
             if (cls == 2) {

@@ -129,11 +129,21 @@ struct NetArrays {
     DevArray<double> zw, gstate;             // [zones][3] zone_worst; state of the zones above kNetSmemMax
     DevArray<double> cumr;                   // [total nodes] cumulative resistances in the zones' order
     DevArray<double> scale, volt, load;      // revs_network_check's scale, voltage and loading, on first use
+    // revs_hosting_capacity's CTAs (two doubles of state per node and step: their own step grouping) and per-node
+    // {W, N}, on its first call
+    HcHost hc;
+    bool hc_ready = false;
+    DevArray<HcCta> hc_ctas;
+    DevArray<int> hc_lists, hc_zone_cta;
+    DevArray<double2> hc_wn;
+    DevArray<double> hc_gstate;
+    DevArray<unsigned long long> hc_part;    // [hosting CTAs][3]
 };
 
-enum NetTool { kNetHostCheck, kNetRepair, kNetCentral, kNetCertify, kNetTools };
+enum NetTool { kNetHostCheck, kNetRepair, kNetCentral, kNetCertify, kNetHosting, kNetTools };
 
-// State of the network tools (revs_network_check, revs_repair_schedule, revs_central_bracket, revs_certify_infeasible).
+// State of the network tools (revs_network_check, revs_repair_schedule, revs_central_bracket, revs_certify_infeasible,
+// revs_hosting_capacity).
 // Everything but the zone arrays is allocated on a tool's first call by net_alloc and kept until revs_destroy.
 struct NetTools {
     bool valid = false;                      // bf matches the trees
@@ -158,6 +168,8 @@ struct NetTools {
     DevArray<int> crt_hpos;                  // [Hp]
     DevArray<int32_t> crt_cert;              // [zones][4]
     DevArray<unsigned long long> crt_key;    // [zones]
+    DevArray<double> hc_cap, hc_uni;         // [Hp][T] home_cap (on first use); [zones][T] zone_uniform
+    DevArray<int64_t> hc_counts;             // [zones][3]
 };
 
 struct TimedSpan { cudaEvent_t a, b; int cat; };
@@ -256,7 +268,7 @@ struct revs_solver {
     double* d_pool_cumr = nullptr;
     int64_t* d_pool_off = nullptr;
     size_t pool_nodes = 0;
-    NetTools net;                              // network check, repair, bracket and certificate
+    NetTools net;                              // network check, repair, bracket, certificate and hosting capacity
     size_t Rpool_elems = 0;
     bool rn2_valid = false;
     // home-major [Hp][T]
@@ -2122,7 +2134,7 @@ int net_run(revs_solver* s, const double* P, double v2, double u, double low, do
 // A tool's state besides the zone arrays: [Hp][T] scratch up to the number the tool uses, its kept schedule and per-zone
 // buffers, the repair kernel's per-zone state (repair, bracket) and the home -> zone map (bracket, certificate).
 int net_alloc(revs_solver* s, NetTool tool) {
-    static const int n_scratch[] = {1, 2, 9, 1};
+    static const int n_scratch[] = {1, 2, 9, 1, 0};
     NetTools& t = s->net;
     if (t.ready[tool]) return REVS_OK;
     const size_t HT = (size_t)s->Hp * s->T, nf = (size_t)s->nf;
@@ -2139,6 +2151,10 @@ int net_alloc(revs_solver* s, NetTool tool) {
         CU(t.crt_hpos.alloc((size_t)s->Hp));
         CU(t.crt_cert.alloc(4 * nf));
         CU(t.crt_key.alloc(nf));
+    }
+    if (tool == kNetHosting) {
+        CU(t.hc_uni.alloc(nf * s->T));
+        CU(t.hc_counts.alloc(3 * nf));
     }
     if ((tool == kNetRepair || tool == kNetCentral) && !t.rep_gws) {
         std::vector<int64_t> off(nf);
@@ -2205,6 +2221,51 @@ int run_repair(revs_solver* s, double u, double row_tol, double* D, double* P, d
     return REVS_OK;
 }
 
+// The checks of a schedule source (REVS_NET_*) of revs_network_check and revs_hosting_capacity.
+int net_source_check(const revs_solver* s, int source, const double* P) {
+    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST && source != REVS_NET_REPAIRED &&
+        source != REVS_NET_CENTRAL)
+        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED "
+                    "or REVS_NET_CENTRAL)", source);
+    if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
+    if (source == REVS_NET_CENTRAL && !s->net.central_valid)
+        return fail(REVS_ERR_ARG, "REVS_NET_CENTRAL: revs_central_bracket has not run since the homes, tariff or trees were set");
+    if (source != REVS_NET_HOST && source != REVS_NET_CENTRAL && s->k == 0)
+        return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check",
+                    source == REVS_NET_SCHEDULE ? "schedule" : source == REVS_NET_ESTIMATE ? "estimate" : "repaired schedule");
+    if (source == REVS_NET_REPAIRED && !s->net.repaired_valid)
+        return fail(REVS_ERR_ARG, "REVS_NET_REPAIRED: revs_repair_schedule has not run since the last ADMM run began");
+    return REVS_OK;
+}
+
+// The device schedule of a checked source; a host schedule P goes to scratch 0 (one launch).
+int net_source(revs_solver* s, int source, const double* P, const double** src, int64_t* launches) {
+    *src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->net.repaired
+           : source == REVS_NET_CENTRAL ? s->net.central : s->d_pest;
+    if (source == REVS_NET_HOST) {
+        int rc = net_alloc(s, kNetHostCheck);
+        if (rc || (rc = h2d_homes(s, s->net.scratch[0], P, s->T))) return rc;
+        *launches += s->H > 0;
+        *src = s->net.scratch[0];
+    }
+    return REVS_OK;
+}
+
+// revs_hosting_capacity's CTAs and per-node {W, N}, once per set of trees (after net_prepare).
+int hc_ready(revs_solver* s) {
+    NetArrays& b = s->net.bf;
+    if (b.hc_ready) return REVS_OK;
+    hc_prepare(b.h, s->T, b.hc);
+    CU(b.hc_ctas.upload(b.hc.ctas));
+    CU(b.hc_lists.upload(b.hc.lists));
+    CU(b.hc_zone_cta.upload(b.hc.zone_cta));
+    CU(b.hc_wn.upload(b.hc.wn));
+    CU(b.hc_gstate.alloc((size_t)b.hc.gstate_doubles));
+    CU(b.hc_part.alloc(3 * b.hc.ctas.size()));
+    b.hc_ready = true;
+    return REVS_OK;
+}
+
 void net_location(const NetArg& a, int T, int32_t* zone, int32_t* index, int32_t* step) {
     const bool none = a.loc == INT64_MAX;      // no candidate (no residence at all)
     *zone = none ? -1 : a.zone;
@@ -2219,34 +2280,18 @@ int revs_network_check(revs_solver* s, int source, const double* P, double vset,
                        const double* scale, double* voltage, double* loading, double* zone_worst,
                        revs_network_summary* summary) {
     if (!s) return fail(REVS_ERR_ARG, "null solver");
-    if (source != REVS_NET_SCHEDULE && source != REVS_NET_ESTIMATE && source != REVS_NET_HOST && source != REVS_NET_REPAIRED &&
-        source != REVS_NET_CENTRAL)
-        return fail(REVS_ERR_ARG, "unknown source %d (REVS_NET_SCHEDULE, REVS_NET_ESTIMATE, REVS_NET_HOST, REVS_NET_REPAIRED "
-                    "or REVS_NET_CENTRAL)", source);
-    if (source == REVS_NET_HOST && !P) return fail(REVS_ERR_ARG, "REVS_NET_HOST needs the schedule P");
-    if (source == REVS_NET_CENTRAL && !s->net.central_valid)
-        return fail(REVS_ERR_ARG, "REVS_NET_CENTRAL: revs_central_bracket has not run since the homes, tariff or trees were set");
-    if (source != REVS_NET_HOST && source != REVS_NET_CENTRAL && s->k == 0)
-        return fail(REVS_ERR_ARG, "no ADMM iteration has run: there is no %s to check",
-                    source == REVS_NET_SCHEDULE ? "schedule" : source == REVS_NET_ESTIMATE ? "estimate" : "repaired schedule");
-    if (source == REVS_NET_REPAIRED && !s->net.repaired_valid)
-        return fail(REVS_ERR_ARG, "REVS_NET_REPAIRED: revs_repair_schedule has not run since the last ADMM run began");
+    int rc = net_source_check(s, source, P);
+    if (rc) return rc;
     const double v2 = vset * vset, u = vhigh * vhigh - v2, lo = vlow * vlow - v2;
     if (!(u > 0.0) || !(lo <= 0.0)) return fail(REVS_ERR_ARG, "need vlow <= vset < vhigh");
     CU(cudaSetDevice(s->device));
-    int rc = net_prepare(s);
-    if (rc) return rc;
+    if ((rc = net_prepare(s))) return rc;
     NetArrays& b = s->net.bf;
     const int T = s->T;
     const size_t out_elems = (size_t)b.h.total_nodes * T;
     int64_t launches = 0;
-    const double* src = source == REVS_NET_SCHEDULE ? s->d_psch[s->cur] : source == REVS_NET_REPAIRED ? s->net.repaired
-                        : source == REVS_NET_CENTRAL ? s->net.central : s->d_pest;
-    if (source == REVS_NET_HOST) {
-        if ((rc = net_alloc(s, kNetHostCheck)) || (rc = h2d_homes(s, s->net.scratch[0], P, T))) return rc;
-        launches += s->H > 0;
-        src = s->net.scratch[0];
-    }
+    const double* src = nullptr;
+    if ((rc = net_source(s, source, P, &src, &launches))) return rc;
     if (scale) {
         if (!b.scale) CU(b.scale.alloc((size_t)b.h.total_nodes));
         CU(cudaMemcpyAsync(b.scale, scale, sizeof(double) * b.h.total_nodes, cudaMemcpyHostToDevice, s->sU));
@@ -2481,6 +2526,72 @@ int revs_certify_infeasible(revs_solver* s, double vset, double vhigh, double ro
         for (int f = 0; f < nf; ++f) c += cert[4 * (size_t)f] != 0;
         *n_certified = c;
     }
+    return REVS_OK;
+}
+
+int revs_hosting_capacity(revs_solver* s, int source, const double* P, double vset, double vhigh, double row_tol,
+                          const double* scale, double* home_cap, double* zone_uniform, int64_t* zone_counts) {
+    if (!s) return fail(REVS_ERR_ARG, "null solver");
+    int rc = net_source_check(s, source, P);
+    if (rc) return rc;
+    double v2, u;
+    if ((rc = tool_limits(vset, vhigh, row_tol, &v2, &u))) return rc;
+    CU(cudaSetDevice(s->device));
+    if ((rc = net_prepare(s)) || (rc = net_alloc(s, kNetHosting)) || (rc = hc_ready(s))) return rc;
+    NetTools& t = s->net;
+    NetArrays& b = t.bf;
+    const int T = s->T, nf = s->nf;
+    const int64_t N = b.h.total_nodes;
+    if (scale)
+        for (int64_t i = 0; i < N; ++i)
+            if (!std::isfinite(scale[i])) return fail(REVS_ERR_ARG, "scale[%lld] is not finite", (long long)i);
+    int64_t launches = 0;
+    const double* src = nullptr;
+    if ((rc = net_source(s, source, P, &src, &launches))) return rc;
+    if (scale) {
+        if (!b.scale) CU(b.scale.alloc((size_t)N));
+        CU(cudaMemcpyAsync(b.scale, scale, sizeof(double) * N, cudaMemcpyHostToDevice, s->sU));
+    }
+    if (home_cap && !t.hc_cap) CU(t.hc_cap.alloc((size_t)s->Hp * T));
+    HcParams hp{};
+    hp.zones = b.zones;
+    hp.nodes = b.nodes;
+    hp.levels = b.levels;
+    hp.res = b.res;
+    hp.ctas = b.hc_ctas;
+    hp.cumr = b.cumr;
+    hp.wn = b.hc_wn;
+    hp.P = src;
+    hp.scale = scale ? b.scale.p : nullptr;
+    hp.has_ev = s->d_has_ev;
+    hp.rating = s->d_rating;
+    hp.start = s->d_start;
+    hp.end = s->d_end;
+    hp.cap = home_cap ? t.hc_cap.p : nullptr;
+    hp.uniform = t.hc_uni;
+    hp.gstate = b.hc_gstate;
+    hp.part = b.hc_part;
+    hp.T = T;
+    hp.ur = u + row_tol;
+    const HcHost& h = b.hc;
+    for (int c = 0; c < 3; ++c) {
+        const int n = h.class_off[c + 1] - h.class_off[c];
+        if (n == 0) continue;
+        CU(launch_hosting(hp, b.hc_lists + h.class_off[c], n, h.class_smem[c], s->sU));
+        ++launches;
+    }
+    CU(launch_hosting_reduce(b.hc_part, b.hc_zone_cta, nf, t.hc_counts, s->sU));
+    launches += nf > 0;
+    if (home_cap) {
+        if ((rc = d2h_homes(s, home_cap, t.hc_cap, T))) return rc;
+        launches += s->H > 0;
+    }
+    if (zone_uniform && nf > 0)
+        CU(cudaMemcpyAsync(zone_uniform, t.hc_uni, sizeof(double) * nf * T, cudaMemcpyDeviceToHost, s->sU));
+    if (zone_counts && nf > 0)
+        CU(cudaMemcpyAsync(zone_counts, t.hc_counts, sizeof(int64_t) * 3 * nf, cudaMemcpyDeviceToHost, s->sU));
+    CU(cudaStreamSynchronize(s->sU));
+    s->stats.kernel_launches += launches;
     return REVS_OK;
 }
 

@@ -389,10 +389,11 @@ class PipelinedSolver:
                     voltage=None if out is None else out["voltage"], loading=None if out is None else out["loading"],
                     zone_worst=np.concatenate([r["zone_worst"] for r in res]) if zones else None)
 
-    def _zone_order(self, method, totals, *args, **kw):
+    def _zone_order(self, method, totals, *args, part_kw=None, **kw):
         """Solver.<method> on every pipeline at once: each array of the results concatenated in zone order (None where
-        not asked for) and the totals recomputed by `totals` -- the bytes of a single solver over the same zones."""
-        res = self._each(lambda k: getattr(self.parts[k], method)(*args, **kw))
+        not asked for) and the totals recomputed by `totals` -- the bytes of a single solver over the same zones.
+        part_kw(k): optional further keyword arguments of pipeline k (its share of a per-home or per-node input)."""
+        res = self._each(lambda k: getattr(self.parts[k], method)(*args, **kw, **(part_kw(k) if part_kw else {})))
         return totals({n: None if v is None else np.concatenate([r[n] for r in res])
                        for n, v in res[0].items() if v is None or isinstance(v, np.ndarray)})
 
@@ -410,6 +411,27 @@ class PipelinedSolver:
         """Solver.certify_infeasible over all pipelines at once (_zone_order)."""
         from ._cabi import certify_totals
         return self._zone_order("certify_infeasible", certify_totals, *args, **kw)
+
+    def hosting_capacity(self, source="schedule", scale=None, homes=True, uniform=True, **kw):
+        """Solver.hosting_capacity over all pipelines at once (_zone_order); a host schedule [H, T] and scale
+        [total nodes] are cut into every pipeline's rows of homes and nodes."""
+        from ._cabi import hosting_totals
+        node_off = np.concatenate([[0], np.cumsum([p.total_nodes for p in self.parts])]).astype(np.int64)
+        host = not isinstance(source, str)
+        if host:
+            source = np.ascontiguousarray(source, dtype=np.float64)
+            if source.shape != (self.H, self.T):
+                raise ValueError(f"expected shape {(self.H, self.T)}, got {source.shape}")
+        if scale is not None:
+            scale = np.ascontiguousarray(scale, dtype=np.float64)
+            if scale.shape != (int(node_off[-1]),):
+                raise ValueError(f"expected shape {(int(node_off[-1]),)}, got {scale.shape}")
+
+        def part(k):
+            (lo, hi), a, b = self.rows[k], node_off[k], node_off[k + 1]
+            return dict(source=source[lo:hi] if host else source, scale=None if scale is None else scale[a:b])
+        return self._zone_order("hosting_capacity", lambda r: hosting_totals(r, self.off), part_kw=part, homes=homes,
+                                uniform=uniform, **kw)
 
     def stats(self):
         """Counters and CUDA-event spans summed over the pipelines; total_ms is the longest
