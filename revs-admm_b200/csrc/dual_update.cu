@@ -257,8 +257,13 @@ cudaError_t launch_dual_update(const DualParams& P, cudaStream_t stream) {
     const int slots = (P.T + 31) / 32;
     const dim3 grid((P.Hp + 31) / 32);
     auto go = [&](auto kernel) -> cudaError_t {
-        if (smem > 48 * 1024) {
-            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        // the 48 KB a launch gets without opting in hold the kernel's static shared memory too (s_part, s_fin, s_peer:
+        // 1.7 KB), so the tile needs the opt-in from T = 185 on, not only beyond 48 KB of its own (T >= 192)
+        cudaFuncAttributes fa;
+        cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+        if (e != cudaSuccess) return e;
+        if (smem + fa.sharedSizeBytes > 48 * 1024) {
+            e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
         }
         kernel<<<grid, 256, smem, stream>>>(P);
