@@ -62,6 +62,7 @@ constexpr double kDegTolN = 1e-9;                  // |d(flow of the subtree)/d(
 constexpr double kPdasSlackN = 1e-13;              // a row off the guess re-enters when violated by more than this fraction of u
 constexpr double kContractRelN = 1e-10;            // edges below this fraction of the largest root-to-node resistance are contracted
 constexpr int kOuterMaxN = 200;
+constexpr int kSkylineOuterN = 32;                 // from this outer iteration on, every violated row is a working row
 
 enum : int { kRes = 1, kW = 2, kA = 4, kPin = 8, kEff = 16 };
 
@@ -499,14 +500,16 @@ __global__ void __launch_bounds__(kNtThreads) tree_newton_kernel(NewtonParams P)
         // ---- working rows (= first guess): the multipliers' support and the SKYLINE of the violated rows -- a violated row
         // enters when no row in the subtree of its parent is more violated.  Under a heavy shared drop thousands of rows are
         // violated by similar amounts and a hundred end up binding; holding the skyline repairs most of the others, what is
-        // left is admitted by the next iteration (the KKT test above always runs over all rows).
+        // left is admitted by the next iteration (the KKT test above always runs over all rows).  Siblings share their
+        // parent's subtree, so the skyline admits ONE row per node per iteration: hundreds of binding service drops on
+        // one node would need as many iterations.  After kSkylineOuterN iterations every violated row enters.
         tree_sums<true>(Z, X, C.ln, C.acc);
         for (int k = threadIdx.x; k < nn; k += kNtThreads) {
             int fl = C.fl[k];
             if (fl & kRes) {
                 const double viol = C.ln[k];
                 const int p = Z.parent[k];
-                if (C.lam[k] > 0.0 || (viol > 0.0 && viol >= C.acc[p >= 0 ? p : k])) fl |= kW | kA;
+                if (C.lam[k] > 0.0 || (viol > 0.0 && (its >= kSkylineOuterN || viol >= C.acc[p >= 0 ? p : k]))) fl |= kW | kA;
                 C.fl[k] = fl;
             }
         }

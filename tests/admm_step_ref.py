@@ -53,7 +53,7 @@ def _multipliers_lstsq(RF, r):
 
 
 def _multipliers_lp(RF, r, RZ, zZ, tol):
-    """min s  s.t. |r - R_FA lam| <= s, z_Z - R_ZA lam <= tol, lam >= 0.  The columns of R_FA are scaled to a largest
+    """min s  s.t. |r - R_FA lam| <= s, z_Z - R_ZA lam <= tol / 2, lam >= 0.  The columns of R_FA are scaled to a largest
     entry of 1 so that HiGHS sees coefficients of order one; its tolerances only steer the search, the caller
     checks the multipliers it returns exactly."""
     m = RF.shape[1]
@@ -64,7 +64,7 @@ def _multipliers_lp(RF, r, RZ, zZ, tol):
     A[:nF, :m], A[:nF, m] = MF, -1.0
     A[nF:2 * nF, :m], A[nF:2 * nF, m] = -MF, -1.0
     A[2 * nF:, :m] = -MZ
-    b = np.concatenate([r, -r, tol - zZ])
+    b = np.concatenate([r, -r, 0.5 * tol - zZ])        # half of tol: a vertex ON the bound lands past it after rounding
     obj = np.zeros(m + 1)
     obj[m] = 1.0
     res = linprog(obj, A_ub=A, b_ub=b, bounds=[(0.0, None)] * (m + 1), method="highs",

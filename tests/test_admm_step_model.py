@@ -130,3 +130,24 @@ def test_next_target_and_dual_update_keep_the_kernel_order():
         want = math.sqrt(float(exact)) / T
         assert abs(diff[h] - want) <= 2.3e-16 * want
     assert not np.array_equal(z, (P_est + P_sch) * 0.5 - Gamma * (1.0 / kappa))    # the order does matter
+
+
+def test_certificate_accepts_projections_that_need_the_lp_at_its_bound():
+    """Iteration 3 of the tree-Newton ADMM case with shared nodes and daisy chains (test_gpu_admm_steps, newton_odd):
+    the LP's multipliers for columns with hundreds of candidate rows sit on the bound of the homes at zero, and were
+    rejected by rounding (residual 1.000005e-9) when that bound was the acceptance tolerance itself."""
+    from test_gpu_newton_shapes import odd_wide
+    from revs_admm_b200.feeder import synthetic_homes, synthetic_tariff
+    tr = odd_wide()
+    T = 24
+    hm = synthetic_homes(tr.n_res, T, seed=tr.n_res)
+    kw = dict(kappa=5.0, vset=1.0, vlow=0.95, vhigh=1.02)
+    R = O.rmat_from_tree(tr.parent, tr.r)[np.ix_(tr.res_node, tr.res_node)]
+    u = kw["vhigh"] ** 2 - kw["vset"] ** 2
+    h = O.solve_ADMM_arrays([R], load=hm["load"], cost=synthetic_tariff(T), ev_mask=hm["has_ev"].astype(bool),
+                            rating=hm["rating"], capacity=hm["capacity"], initial=hm["initial"], start=hm["start"],
+                            end=hm["end"], iter_max=2, return_history=True, **kw)["history"]
+    z = AR.next_target(*h[1], kw["kappa"])[:, [21, 22]]           # the two columns of iteration 3 that were rejected
+    g = np.stack([O.project_voltage(z[:, j], R, u)[0] for j in range(2)], axis=1)
+    c = AR.certify_projection(R, z, g, u)
+    assert c["ok"].all() and c["lp"] >= 1, (np.nonzero(~c["ok"])[0], c["resid"].max(), c["lp"])

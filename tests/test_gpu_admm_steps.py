@@ -21,6 +21,7 @@ import admm_step_ref as AR
 import revs_oracle as O
 from revs_admm_b200 import expand_schedule
 from test_gpu_edges import _problem
+from test_gpu_newton_shapes import deep, odd_wide, wide2
 
 pytestmark = pytest.mark.gpu
 
@@ -76,6 +77,7 @@ def _counts(hm):
 
 def _case(name):
     """(sizes, T, trees, homes, tariff, kw, iterations, options)."""
+    from revs_admm_b200.feeder import synthetic_homes, synthetic_tariff
     kw = dict(kappa=5.0, vset=1.0, vlow=0.95, vhigh=1.02)
     classes = {"cls_warp_small": [1, 16, 17, 127, 128, 129, 192], "cls_warp_big": [193, 255, 256, 257, 320],
                "cls_cta": [321, 512, 513, 700]}
@@ -89,6 +91,11 @@ def _case(name):
         sizes, T = [600, 90], 24
         trees, hm, cost = _problem(sizes, T, seed=690)
         return sizes, T, trees, hm, cost, dict(kw, vhigh=1.05), 5, {}
+    if name in ("newton_wide", "newton_deep", "newton_odd"):    # layout branches of the tree-Newton kernel
+        tr, K = {"newton_wide": (wide2(), 5), "newton_deep": (deep(1025), 3), "newton_odd": (odd_wide(), 5)}[name]
+        T = 24
+        hm = synthetic_homes(tr.n_res, T, seed=tr.n_res)
+        return [tr.n_res], T, [tr], hm, synthetic_tariff(T), kw, K, dict(newton_min_n=0)
     if name == "handover":          # every charger free in every step: working sets beyond 16 and 32 rows
         sizes, T = [120, 96], 12
         trees, hm, cost = _problem(sizes, T, seed=77, r_secondary=2e-3, adoption=1.0)
@@ -112,7 +119,7 @@ def _case(name):
 
 
 HORIZONS = [1, 31, 32, 33, 64, 65, 96, 97, 128, 129, 185, 191, 192, 256]      # 185..191: dual_update opts in to > 48 KB of shared memory
-CASES = ["cls_warp_small", "cls_warp_big", "cls_cta", "newton", "handover", "no_warp", "padding"] + \
+CASES = ["cls_warp_small", "cls_warp_big", "cls_cta", "newton", "newton_wide", "newton_deep", "newton_odd", "handover", "no_warp", "padding"] + \
         [f"T{T}" for T in HORIZONS] + ["T96_noscreen", "T97_noscreen"]
 
 

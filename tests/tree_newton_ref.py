@@ -98,6 +98,7 @@ PHI_NOISE = 1e-14
 CONTRACT_REL = 1e-10      # edges below this fraction of the largest root-to-node resistance are contracted
 DEG_TOL = 1e-9           # |d(flow of the subtree)/d(mu)| below this: no home of the piece below an effective row
 PDAS_SLACK = 1e-13        # a row off the guess re-enters when it is violated by more than this fraction of u
+SKYLINE_OUTER = 32        # from this outer iteration on, every violated row is a working row (not only the skyline)
 
 
 def contract_tree(parent, r, res_node, rel=CONTRACT_REL):
@@ -325,7 +326,8 @@ class LevelTree:
             # working rows: the multipliers' support and the SKYLINE of the violated rows -- a violated row enters when no row
             # in the subtree of its parent is more violated.  Under a heavy shared drop thousands of rows are violated by
             # similar amounts, a hundred end up binding; holding the skyline repairs most of the others, the rest is admitted
-            # by the next iteration (the KKT test always runs over all rows).
+            # by the next iteration (the KKT test always runs over all rows).  Siblings share their parent's subtree, so the
+            # skyline admits one row per node per iteration; after SKYLINE_OUTER iterations every violated row enters.
             viol = np.where(isres, np.maximum(-grad, 0.0), 0.0)
             sub = viol.copy()
             for lo, hi in self.levels_up():
@@ -334,7 +336,7 @@ class LevelTree:
                     m = nc > j
                     sub[lo:hi][m] = np.maximum(sub[lo:hi][m], sub[c0[m] + j])
             ref = np.where(self.parent >= 0, sub[np.maximum(self.parent, 0)], sub)
-            W = isres & ((lam > 0) | ((viol > 0) & (viol >= ref)))
+            W = isres & ((lam > 0) | ((viol > 0) & ((viol >= ref) | (it >= SKYLINE_OUTER))))
             Fh = g > 0
             nF = node_sum(Fh.astype(float))
             zF = node_sum(np.where(Fh, z, 0.0))
