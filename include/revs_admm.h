@@ -132,7 +132,9 @@ int revs_admm_step(revs_solver* s, double sums[3]);
  *   P_sch_new = g_opt [H,T], P_ev = p_opt [H,T] (either may be NULL).
  * revs_utility_step == Utility(graph, P_est, P_sch, Gamma, kappa, vset, vlow, vhigh).solve():
  *   P_est_new = g_opt [H,T]; lam0 (may be NULL) warm-starts the voltage-row multipliers,
- *   lam_out (may be NULL) returns them, both [H,T]. */
+ *   lam_out (may be NULL) returns them, both [H,T].  Only the positive entries of lam0 are
+ *   used; zero, negative and NaN entries count as 0, and lam_out is 0 on every row that does
+ *   not bind, whatever lam0 held there. */
 int revs_home_step(revs_solver* s, double kappa, const double* p_est, const double* p_sch,
                    const double* gamma, double* P_sch_new, double* P_ev);
 int revs_utility_step(revs_solver* s, double kappa, double vset, double vlow, double vhigh,

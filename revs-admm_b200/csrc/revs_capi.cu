@@ -1878,7 +1878,9 @@ int revs_utility_step(revs_solver* s, double kappa, double vset, double vlow, do
             for (int t = 0; t < T; ++t) {
                 const size_t src = (size_t)i * T + t;
                 zt[(size_t)t * s->Hp + hp] = (p_est[src] + p_sch[src]) / 2.0 - gamma[src] / kappa;
-                if (lam0) lt[(size_t)t * s->Hp + hp] = lam0[src];
+                // only positive multipliers start a working set (qp_init_kernel): zero, negative and NaN entries are
+                // stored as 0, so that no row outside the solution comes back with the caller's value
+                if (lam0) lt[(size_t)t * s->Hp + hp] = lam0[src] > 0.0 ? lam0[src] : 0.0;
             }
         }
     CU(cudaMemcpyAsync(s->d_zt, zt.data(), HT * sizeof(double), cudaMemcpyHostToDevice, s->sU));

@@ -224,7 +224,7 @@ __device__ void hessian(const double* __restrict__ R, int ld, int n, const doubl
 // with shuffles once at the end -- every thread does useful work and each accumulator is its
 // own dependency chain.  Same contract as hessian<>.
 constexpr int kPairM = 8;
-constexpr int kPairMax = kPairM * (kPairM + 1) / 2;     // 78
+constexpr int kPairMax = kPairM * (kPairM + 1) / 2;     // 36
 
 template <int WMAX, int THREADS, bool INCR, class S>
 __device__ void hessian_pairs(const double* __restrict__ R, int ld, int n, const double* g, int m, int nchg, S& sm) {
@@ -703,7 +703,9 @@ __device__ void qp_column(const QpParams& P, const int c, S& sm) {
                 handed = true;
                 break;
             }
-            if (added == 0) {
+            // a full working set overflows only once it has been solved: rows of a warm start that was never solved
+            // on W may leave it with a zero multiplier (solve first, admit in the next pass)
+            if (added == 0 && inner_prev == 1) {
                 if (tid == 0) { P.status[c] = 2; atomicAdd(P.n_failed, 1); }
                 finished = true;
                 break;
